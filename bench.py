@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Headline benchmark: 1080p preprocessing-chain frames/s on N B200s (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A step is one pass of the hot path (CLAHEDehaze -> MedianDerain) over one batch of fogged + rained frames.  Workload at
 every N: BASELINE.json configs[1] -- 1920x1080, batch 64 per GPU, YCrCb, clip 2.0, tile grid 8, median k5 (frames /
@@ -357,6 +357,28 @@ def load_ncu_constants(rvb200):
     return j, info
 
 
+DUMP_ROWS, DUMP_SEED = 2048, 0
+
+
+def sample_output_rows(d_out):
+    """A fixed sample of an output batch (BATCH, H, W, 3) uint8 for comparing two builds: DUMP_ROWS whole rows, gathered on the
+    device (so that later steps cannot overwrite them), and their (frame, row) index."""
+    import numpy as np
+    import torch
+    pick = np.sort(np.random.default_rng(DUMP_SEED).choice(BATCH * H, DUMP_ROWS, replace=False))
+    frame, row = pick // H, pick % H
+    rows = d_out[torch.from_numpy(frame).to(d_out.device), torch.from_numpy(row).to(d_out.device)]
+    return rows, np.stack([frame, row], axis=1)
+
+
+def dump_outputs(out_dir, rows, index):
+    """chain_out_rows.npy: the sampled rows as float32 (47 MB); chain_out_rows_index.npy: their (frame, row) as float64."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "chain_out_rows.npy"), rows.cpu().numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, "chain_out_rows_index.npy"), index.astype(np.float64))
+
+
 def run_gpu(args, rank, world, local_rank):
     import numpy as np
     import torch
@@ -414,6 +436,7 @@ def run_gpu(args, rank, world, local_rank):
     torch.cuda.synchronize(); barrier()
     ms = e0.elapsed_time(e1)
     launches = ctx.launch_count - l0
+    dump = sample_output_rows(d_out) if args.dump_outputs and rank == 0 else None
     ms_max = max_over_ranks(ms)
     frames_total = sum_over_ranks(BATCH * args.steps)
     value = frames_total / (ms_max * 1e-3)
@@ -430,6 +453,9 @@ def run_gpu(args, rank, world, local_rank):
     sustained = {"steps": n_sus, "seconds": ms_sus * 1e-3, "value": sum_over_ranks(BATCH * n_sus) / (ms_sus * 1e-3), "unit": UNIT}
     t1 = time.time()
     clocks = sampler.stop(t0, t1) if rank == 0 else None
+    if dump is not None:                        # written outside the sampled clock window
+        dump_outputs(args.dump_outputs, *dump)
+        del dump
     if clocks is not None:
         clocks["window"] = "the K timed steps + the sustained loop (%d steps), %.2f s" % (n_sus, t1 - t0)
 
@@ -562,7 +588,8 @@ def run_gpu(args, rank, world, local_rank):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=1200, help="timed steps (default sized so that the timed region spans > 1 s)")
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default 1200 for the GPU arm, sized so that the timed region spans > 1 s; 20 for the reference arm)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--group", type=int, default=0, help="frames per hist->lut->chain group (0 = library default)")
@@ -573,7 +600,15 @@ def main():
     ap.add_argument("--no-e2e", action="store_true", help="skip the end-to-end legs (profiling runs)")
     ap.add_argument("--stream-seconds", type=float, default=32.0, help="length of the paced-stream leg (0 = skip)")
     ap.add_argument("--cpu-seconds", type=float, default=10.0, help="time budget of the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a seeded sample of the last step's output (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 20 if args.impl == "reference" else 1200
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the GPU arm's outputs")
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -585,8 +620,6 @@ def main():
         raise SystemExit(subprocess.call(cmd))
 
     if args.impl == "reference":
-        if args.steps > 200:
-            args.steps = 20                     # the CPU arm's default: 20 x 64 frames (a few seconds)
         run_reference(args, rank, world)
         return
     if world > 1:

@@ -1,10 +1,9 @@
 """The reference's six OpenCV calls, restated -- TEST INFRASTRUCTURE ONLY.
 
 The reference's CPU implementation of the path *is* this sequence of cv2 calls
-(/root/reference/src/preprocess/ops/clahe_dehaze.py:13-32 and ops/median_derain.py:10-14);
-/root/reference does not travel to the GPU box, so the sequence is restated here and
-tests/test_oracle_reference.py asserts it equals the reference's own classes whenever
-/root/reference is importable.  Used as the live ground truth in tests and as the
+(src/preprocess/ops/clahe_dehaze.py:13-32 and ops/median_derain.py:10-14); the reference is
+not part of this repository, so the sequence is restated here and tests/test_oracle.py and
+tests/test_reference_equivalence.py check it against outputs and coercions recorded from the reference's own classes.  Used as the live ground truth in tests and as the
 `--impl reference` / cpu_baseline arm of bench.py.
 """
 import cv2

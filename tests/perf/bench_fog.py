@@ -1,6 +1,6 @@
 #!/usr/bin/env python3
-"""Fog synthesis throughput: this package on the GPU next to the reference's EnhancedFogSynthesizer on the host (oracle/_ref or
-/root/reference), 1080p frames, fog_batch.py's parameters.  One JSON line."""
+"""Fog synthesis throughput: this package on the GPU next to the reference's EnhancedFogSynthesizer on the host (where
+oracle/install_ref.py has installed it under oracle/_ref), 1080p frames, fog_batch.py's parameters.  One JSON line."""
 import json
 import os
 import sys
@@ -12,7 +12,22 @@ sys.path.insert(1, os.path.join(ROOT, "tests"))
 import rvb200  # noqa: E402
 from rvb200 import synth  # noqa: E402
 from rvb200.augment import EnhancedFogSynthesizer  # noqa: E402
-from test_fog import KW, reference_fog_class  # noqa: E402
+from test_fog import KW  # noqa: E402
+from oracle import install_ref  # noqa: E402
+
+
+def reference_fog_class():
+    """The reference's class from oracle/_ref, or None."""
+    if not install_ref.available():
+        return None
+    sys.path.insert(0, install_ref.ref_root())
+    try:
+        sys.dont_write_bytecode = True
+        from src.augment.fog import EnhancedFogSynthesizer as Ref
+        return Ref
+    finally:
+        sys.path.remove(install_ref.ref_root())
+
 
 clean = [synth.clean_scene(1080, 1920, 950 + i) for i in range(4)]
 ctx = rvb200.default_context()

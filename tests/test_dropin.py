@@ -1,6 +1,6 @@
-"""The drop-in claim: the reference's own config loader + configs/default.yaml + `from src.preprocess import
-PreprocessPipeline` (main_preview.py:6,58,94) drive the B200 ops unchanged when this package is mounted as `src/preprocess`
-(INTEGRATION.md §2).  Needs /root/reference (this container); the GPU half also needs a B200."""
+"""The drop-in claim: `from src.preprocess import PreprocessPipeline` (main_preview.py:6,58,94) and the `preprocess:` block of
+the reference's configs/default.yaml drive the B200 ops unchanged when this package is mounted as `src/preprocess`
+(INTEGRATION.md section 2); the GPU half also needs a B200."""
 import os
 import subprocess
 import sys
@@ -9,21 +9,22 @@ import textwrap
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
 PKG = os.path.join(ROOT, "road-vision-system_b200")
 
-needs_ref = pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "configs", "default.yaml")), reason="reference not mounted")
+# what the reference's load_config() returns under "preprocess" for its stock configs/default.yaml:21-34
+STOCK_PREPROCESS = {"enabled": True,
+                    "chain": [{"name": "CLAHEDehaze", "params": {"space": "YCrCb", "clip_limit": 2.0, "tile_grid": 8}},
+                              {"name": "MedianDerain", "params": {"ksize": 3}}],
+                    "auto_gate": {"enable_low_contrast_gate": False, "contrast_thresh": 20.0}}
 
 
 def make_tree(tmp_path):
-    """<tmp>/src/{preprocess,io_video,_native.py,csrc} -> this repo; config.py, configs/ -> the reference."""
+    """<tmp>/src/{preprocess,io_video,_native.py,csrc,synth.py} -> this package."""
     src = tmp_path / "src"
     src.mkdir()
     (src / "__init__.py").write_text("")
     for name in ("preprocess", "io_video", "_native.py", "csrc", "synth.py"):
         os.symlink(os.path.join(PKG, name), src / name)
-    os.symlink(os.path.join(REF, "src", "config.py"), src / "config.py")
-    os.symlink(os.path.join(REF, "configs"), tmp_path / "configs")
     return tmp_path
 
 
@@ -33,15 +34,12 @@ def run(tmp, body):
     return subprocess.run([sys.executable, "-c", code], cwd=str(tmp), capture_output=True, text=True, timeout=600)
 
 
-@needs_ref
 def test_stock_yaml_builds_the_pipeline(tmp_path):
     tmp = make_tree(tmp_path)
     r = run(tmp, """
-        from src.config import load_config                    # the reference's loader, unchanged
         from src.preprocess import PreprocessPipeline         # main_preview.py:6
         from src.preprocess.registry import REGISTRY
-        cfg = load_config()
-        pp = cfg.get("preprocess", {})
+        pp = %r
         pipe = PreprocessPipeline(pp)                         # main_preview.py:58
         assert pipe.enabled and [type(o).__name__ for o in pipe.ops] == ["CLAHEDehaze", "MedianDerain"], pipe.ops
         seg = pipe._segments()
@@ -51,29 +49,20 @@ def test_stock_yaml_builds_the_pipeline(tmp_path):
         img = np.zeros((4, 4, 3), np.uint8)
         assert PreprocessPipeline({"enabled": False})(img) is img
         print("ok")
-    """)
+    """ % (STOCK_PREPROCESS,))
     assert r.returncode == 0 and "ok" in r.stdout, r.stderr[-2000:]
 
 
 @pytest.mark.gpu
 def test_stock_chain_runs_on_gpu_as_src_preprocess(tmp_path):
-    """GPU half (the GPU box has no /root/reference): same mount as `src/preprocess`, config = the `preprocess:` block of
-    configs/default.yaml:21-34 spelled out; the loader + YAML themselves are covered by the CPU test above."""
-    src = tmp_path / "src"
-    src.mkdir()
-    (src / "__init__.py").write_text("")
-    for name in ("preprocess", "io_video", "_native.py", "csrc", "synth.py"):
-        os.symlink(os.path.join(PKG, name), src / name)
-    r = run(tmp_path, """
+    """GPU half: the same mount as `src/preprocess` and the same stock `preprocess:` block, one camera-sized frame."""
+    tmp = make_tree(tmp_path)
+    r = run(tmp, """
         import numpy as np
         from src.preprocess import PreprocessPipeline         # main_preview.py:6
         from src import synth
         from oracle import rv_oracle as O
-        pp = {"enabled": True,
-              "chain": [{"name": "CLAHEDehaze", "params": {"space": "YCrCb", "clip_limit": 2.0, "tile_grid": 8}},
-                        {"name": "MedianDerain", "params": {"ksize": 3}}],
-              "auto_gate": {"enable_low_contrast_gate": False, "contrast_thresh": 20.0}}
-        pipe = PreprocessPipeline(pp)                         # main_preview.py:58
+        pipe = PreprocessPipeline(%r)                         # main_preview.py:58
         raw = synth.road_frame(480, 640, 1)                   # default.yaml:3-4 camera size
         keep = raw.copy()
         proc = pipe(raw, ts=0.0)                              # main_preview.py:94
@@ -82,5 +71,5 @@ def test_stock_chain_runs_on_gpu_as_src_preprocess(tmp_path):
         assert np.array_equal(proc, O.chain(raw, O.SPACE_YCRCB, 2.0, 8, 3))
         proc[:] = 0                                           # draw_detections writes into it (main_preview.py:114)
         print("ok")
-    """)
+    """ % (STOCK_PREPROCESS,))
     assert r.returncode == 0 and "ok" in r.stdout, r.stderr[-2000:]

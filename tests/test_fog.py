@@ -1,4 +1,4 @@
-"""Fog synthesis on the GPU (SURVEY.md 8 f4) against the reference's EnhancedFogSynthesizer (/root/reference/src/augment/fog.py:84-299).
+"""Fog synthesis on the GPU (SURVEY.md 8 f4) against the reference's EnhancedFogSynthesizer (src/augment/fog.py:84-299).
 
 Parity is statistical by nature (float pipeline; library exp / pow; OpenCV's SIMD summation order; the reference's own output
 moves by an LSB between OpenCV builds), so the bar is written here as tolerances:
@@ -6,17 +6,15 @@ moves by an LSB between OpenCV builds), so the bar is written here as tolerances
   * per-pixel: mean absolute difference <= 0.002 LSB, at most 0.01 % of the values off by more than 2 LSB, none by more than 6
     (measured on B200: 5e-6 .. 4e-5 LSB mean, at most 3 LSB on a handful of pixels);
   * per-channel mean and standard deviation within 0.02 LSB of the reference frame's (measured: <= 4e-5);
-  * transmission map RMS error <= 4e-4 against the fixtures (which store it as float16; measured 1.4e-4, all of it storage) and
-    <= 1e-6 against the live reference (measured 6e-8);
+  * transmission map RMS error <= 4e-4 against the fixtures (which store it as float16; measured 1.4e-4, all of it storage);
   * with the sensor-noise field generated on the device instead of drawn from the reference's stream: statistics only
     (mean / std within 0.02 LSB; measured 0.005).
 
-Fixtures (tests/golden/fog_small.npz) were produced by the reference itself (tests/golden/make_fog_golden.py); on a box where the
-reference tree is available (here: /root/reference, GPU box: oracle/_ref) a second test runs the reference live with fresh seeds.
+Fixtures (tests/golden/fog_small.npz) were produced by the reference itself (tests/golden/make_fog_golden.py); at full size, the
+benchmark's frame pool (tests/golden/pool_1080p, tests/golden/make_bench_pool.py) holds eight 1080p frames the reference fogged.
 """
 import ctypes as C
 import os
-import sys
 
 import numpy as np
 import pytest
@@ -24,24 +22,6 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLDEN = os.path.join(ROOT, "tests", "golden", "fog_small.npz")
 KW = dict(y_h_ratio=0.42, perlin_scale_ratio=0.18, perlin_octaves=2, horizon_softness=0.07, global_veil=0.5, depth_blur_max=4.0)
-
-
-def reference_fog_class():
-    """The reference's class from /root/reference or oracle/_ref, or None."""
-    for cand in ("/root/reference", os.path.join(ROOT, "oracle", "_ref", "road-vision-system")):
-        if os.path.isfile(os.path.join(cand, "src", "augment", "fog.py")):
-            saved = {k: sys.modules.pop(k) for k in [k for k in sys.modules if k == "src" or k.startswith("src.")]}
-            sys.path.insert(0, cand)
-            try:
-                sys.dont_write_bytecode = True
-                from src.augment.fog import EnhancedFogSynthesizer as Ref
-                return Ref
-            finally:
-                sys.path.remove(cand)
-                for k in [k for k in sys.modules if k == "src" or k.startswith("src.")]:
-                    del sys.modules[k]
-                sys.modules.update(saved)
-    return None
 
 
 def cases():
@@ -99,33 +79,36 @@ def value_noise(fr, lattice, h, w):
 
 
 def test_host_side_matches_the_reference_draw_for_draw():
-    """Depth prior, horizon, noise lattices / beta map and the branch decisions of every fixture case equal the reference's."""
-    Ref = reference_fog_class()
-    if Ref is None:
-        pytest.skip("reference tree not available")
-    import rvb200
+    """Depth prior, horizon, noise lattices / beta map and the branch decisions of every fixture case against what the reference
+    recorded with it.  The host's depth prior and beta map give the transmission map t = clip(exp(-beta d), 0.05, 1), edge-guided
+    by cv2.bilateralFilter (radius 8, both sigmas 12; fog.py:55-67, 179-185); every pixel must equal the reference's own t, which the
+    fixture stores as float16, to within that storage's rounding.  The beta map's mean must equal the recorded one (8 decimals)."""
+    import cv2
     from rvb200 import synth
     from rvb200.augment import EnhancedFogSynthesizer
     from rvb200 import _native
     for c in cases():
         clean = synth.clean_scene(c["h"], c["w"], c["scene"])
-        _, meta = Ref(level=c["level"], seed=c["seed"], **KW).synthesize(clean)
         cap = Capture()
         fake = _native.Context.__new__(_native.Context)
         fake._lib, fake._h = cap, C.c_void_p(1)
         mine = EnhancedFogSynthesizer(level=c["level"], seed=c["seed"], context=fake, exact_noise=True, **KW)
         mine.synthesize(clean)
-        h, w, depth, sky, vgrad, xgrad = cap.geo
-        assert (h, w) == (c["h"], c["w"]) and np.array_equal(depth, meta["depth"]), c["i"]
-        assert mine._geo["horizon"] == meta["y_h"]
+        h, w, depth = cap.geo[:3]
+        assert (h, w) == (c["h"], c["w"]) and mine._geo["horizon"] == int(KW["y_h_ratio"] * h), c["i"]
         fr = cap.frame
         beta = value_noise(fr, cap.lattice, h, w)
-        assert np.abs(beta - meta["beta_map"]).max() <= 2e-7, (c["i"], np.abs(beta - meta["beta_map"]).max())
+        assert abs(float(beta.mean()) - c["mean_beta"]) <= 2e-8, (c["i"], float(beta.mean()), c["mean_beta"])
+        t = np.clip(np.exp(-beta * depth), 0.05, 1.0).astype(np.float32)
+        assert fr.edge_guided
+        t = np.clip(cv2.bilateralFilter(t, 17, 12, 12), 0.05, 1.0)
+        half_ulp = np.spacing(c["t"].astype(np.float16)).astype(np.float32) / 2
+        assert (np.abs(t - c["t"]) <= half_ulp + 1e-6).all(), (c["i"], float(np.abs(t - c["t"]).max()))
         assert (fr.gamma > 0) == c["gamma"] and (fr.noise_sigma > 0) == c["noise"], c["i"]
         assert (cap.noise is not None) == c["noise"]
         assert fr.glow_k % 2 == 1 and fr.glow_k2 % 2 == 1 and fr.fade_d % 2 == 1 and fr.octaves == 2
         assert all(0.7 - 1e-6 <= fr.A_bgr[k] <= 1.0 for k in range(3)) and 0.8 <= fr.a_target <= 1.0
-        assert abs(meta["A_map"].mean() - fr.a_target) < 0.02           # the airlight map is scaled to this mean, then clipped
+        assert abs(c["mean_A"] - fr.a_target) < 0.02                    # the airlight map is scaled to this mean, then clipped
 
 
 def test_host_shortcuts_equal_the_plain_formulas():
@@ -219,27 +202,18 @@ def test_fog_fixtures_made_by_the_reference(ctx):
 
 
 @pytest.mark.gpu
-def test_fog_live_against_the_reference_at_full_size(ctx):
-    """1080p, fresh seeds, all three levels: the reference runs on the host (1-2 s per frame), this package on the GPU."""
-    Ref = reference_fog_class()
-    if Ref is None:
-        pytest.skip("reference tree not available (oracle/_ref is installed by __graft_entry__.build())")
-    import time
+def test_fog_against_the_reference_pool_at_full_size(ctx):
+    """1080p, all three levels: every frame of the benchmark pool is a clean scene fogged by the reference's synthesiser with these
+    parameters and the recorded level and seed, then streaked by this package's deterministic add_rain.  The same steps with the
+    GPU synthesiser must reproduce each frame within the per-pixel tolerances."""
+    import cv2
     from rvb200 import synth
     from rvb200.augment import EnhancedFogSynthesizer
-    clean = synth.clean_scene(1080, 1920, 900)
-    for level, seed in (("light", 41), ("medium", 42), ("heavy", 43)):
-        t0 = time.perf_counter()
-        want, wmeta = Ref(level=level, seed=seed, **KW).synthesize(clean)
-        t1 = time.perf_counter()
-        fog = EnhancedFogSynthesizer(level=level, seed=seed, context=ctx, exact_noise=True, **KW)
-        fog.synthesize(clean)                                            # first call uploads the geometry
-        fog = EnhancedFogSynthesizer(level=level, seed=seed, context=ctx, exact_noise=True, **KW)
-        fog._geo = None
-        t2 = time.perf_counter()
-        got, meta = fog.synthesize(clean)
-        t3 = time.perf_counter()
-        rms = float(np.sqrt(np.mean((meta["t"] - wmeta["t"]) ** 2)))
-        print(level, "reference %.2f s, GPU %.3f s (incl. host maps), t rms %.2e" % (t1 - t0, t3 - t2, rms))
-        assert rms <= 1.0e-6
-        compare(got, want, f"1080p {level}")
+    d = os.path.join(ROOT, "tests", "golden", "pool_1080p")
+    rows = [ln.strip().split("|") for ln in open(os.path.join(d, "index.txt")) if ln.strip() and not ln.startswith("#")]
+    assert len(rows) == 8
+    for name, level, seed, *_ in rows:
+        want = cv2.imread(os.path.join(d, name), cv2.IMREAD_COLOR)
+        clean = synth.clean_scene(1080, 1920, int(seed))
+        hazy, _ = EnhancedFogSynthesizer(level=level, seed=int(seed), context=ctx, exact_noise=True, **KW).synthesize(clean)
+        compare(synth.add_rain(hazy, seed=int(seed)), want, f"pool {name} {level}")
