@@ -15,6 +15,10 @@
  *   rv_clahe_dehaze    CLAHEDehaze.__call__ alone             clahe_dehaze.py:13-32
  *   rv_median          MedianDerain.__call__ alone            median_derain.py:10-14
  *   rv_gray_span       PreprocessPipeline._low_contrast       pipeline.py:24-30
+ *   rv_chain_u16       rv_chain_u8 for uint16 frames: the same PreprocessPipeline.__call__ / CLAHEDehaze.__call__ /
+ *                      MedianDerain.__call__ (pipeline.py:32-45, clahe_dehaze.py:13-32, median_derain.py:10-14) when the
+ *                      reference is handed a 16-bit frame, which it passes to cv2's CV_16U path unchanged
+ *   rv_gray_span_u16   PreprocessPipeline._low_contrast on a 16-bit frame   pipeline.py:24-30
  *   rv_submit/rv_wait  (new) batched multi-frame entry fed from pinned host buffers; no reference
  *                      counterpart (the reference loop is one frame in flight, main_preview.py:88-142)
  *   rv_submit_io       (new) the same with every end of the job placed independently: what src/io_video/capture.py:18-21
@@ -225,6 +229,21 @@ int rv_fog_u8(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int h, int w, const 
 
 /* span: n ints = max(gray) - min(gray) per frame */
 int rv_gray_span(rv_ctx *ctx, const uint8_t *in, int n, int h, int w, size_t pitch, int32_t *span, int mem_kind);
+
+/* ---- 16-bit frames (uint16 BGR, e.g. HDR automotive sensors or cv2.imread(..., IMREAD_ANYDEPTH)).  The chain as cv2 computes it on
+ * CV_16U: cvtColor BGR2YCrCb / YCrCb2BGR in 16-bit fixed point, CLAHE with 65,536-bin histograms, medianBlur k = 3 / 5
+ * (reference: pipeline.py:32-45, clahe_dehaze.py:13-32, median_derain.py:10-14; arithmetic in csrc/rv_u16.cu).
+ * rv_chain_u16 behaves like rv_chain_u8 except:
+ *   - pitches are in bytes, even, and >= 6*w; buffers are 2-byte aligned;
+ *   - RV_SPACE_LAB, a ksize outside {0, 3, 5} (cv2 has neither at 16 bits), "nothing to do" or a tile grid outside [2, 64] (a dense
+ *     grid-64 LUT set is already 512 MB per frame) -> RV_ERR_ARG;
+ *   - RV_MEM_DEVICE with a `stream` is asynchronous on that stream (as rv_chain_letterbox_f16) unless `processed` is asked for together
+ *     with the gate; host memory and device memory without a stream are synchronous.
+ * The gate compares the span of cv2's 16-bit BGR2GRAY, (3735 B + 19235 G + 9798 R + 16384) >> 15, with gate_thresh. */
+int rv_chain_u16(rv_ctx *ctx, const uint16_t *in, uint16_t *out, int n, int h, int w, size_t in_pitch, size_t out_pitch,
+                 const rv_params *p, int mem_kind, int32_t *processed, void *stream);
+/* span: n ints = max(gray) - min(gray) per 16-bit frame (synchronous) */
+int rv_gray_span_u16(rv_ctx *ctx, const uint16_t *in, int n, int h, int w, size_t pitch, int32_t *span, int mem_kind);
 
 #ifdef __cplusplus
 }

@@ -206,6 +206,9 @@ EXPORTS = {
     "rv_fog_u8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.POINTER(C.c_float), C.POINTER(C.c_float),
                             C.POINTER(C.c_float), C.POINTER(C.c_float), C.POINTER(C.c_float)]),
     "rv_gray_span": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_int]),
+    "rv_chain_u16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t,
+                               C.POINTER(Params), C.c_int, _i32p, C.c_void_p]),
+    "rv_gray_span_u16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_int]),
 }
 
 
@@ -237,6 +240,34 @@ def _check_frames(frames):
         raise ValueError(f"(N,H,W,3) uint8 expected, got shape {frames.shape}")
     if frames.shape[1] < 1 or frames.shape[2] < 1:
         raise ValueError("empty frame")
+
+
+U16_MAX_GRID = 64
+
+
+def check_u16_params(params):
+    """The chain's parameters on 16-bit frames: what cv2 has no CV_16U path for (LAB, median k 7 / 9) and the tile grid limit of
+    this build raise ValueError here, before anything reaches the GPU."""
+    if params.space == SPACE_LAB:
+        raise ValueError("LAB is not supported on uint16 frames (cv2.cvtColor BGR2LAB has no 16-bit path); use space YCrCb")
+    if params.ksize not in (0, 3, 5):
+        raise ValueError(f"median ksize {params.ksize} is not supported on uint16 frames (cv2.medianBlur: k = 3 or 5 at 16 bits)")
+    if params.clahe and not 2 <= params.grid <= U16_MAX_GRID:
+        raise ValueError(f"tile_grid {params.grid} is not supported on uint16 frames (limit {U16_MAX_GRID}: each tile has a "
+                         "65,536-entry LUT)")
+    if not params.clahe and params.ksize == 0:
+        raise ValueError("nothing to do (no CLAHE, no median)")
+
+
+def _check_frames_u16(frames):
+    if frames.ndim != 4 or frames.shape[3] != 3:
+        raise ValueError(f"(N,H,W,3) uint16 expected, got shape {frames.shape}")
+    if frames.shape[1] < 1 or frames.shape[2] < 1:
+        raise ValueError("empty frame")
+
+
+def _is_u16(frames):
+    return isinstance(frames, np.ndarray) and frames.dtype != np.uint8 and frames.dtype == np.uint16
 
 
 class _Lease(np.ndarray):
@@ -363,7 +394,9 @@ class Context:
 
     # -- the chain -----------------------------------------------------------------------
     def chain(self, frames, params, out=None, processed=None):
-        """rv_chain_u8 over host frames (N,H,W,3) uint8; returns a new (or `out`) array."""
+        """rv_chain_u8 over host frames (N,H,W,3) uint8 (rv_chain_u16 for uint16 frames); returns a new (or `out`) array."""
+        if _is_u16(frames):
+            return self._chain_u16(frames, params, out, processed)
         _check_frames(frames)
         if not frames.flags.c_contiguous:
             frames = np.ascontiguousarray(frames)
@@ -389,6 +422,30 @@ class Context:
         if rc != 0:
             self._ck(rc)
         return out
+
+    def _chain_u16(self, frames, params, out=None, processed=None):
+        """rv_chain_u16 over host frames (N,H,W,3) uint16."""
+        _check_frames_u16(frames)
+        check_u16_params(params)
+        if not frames.flags.c_contiguous:
+            frames = np.ascontiguousarray(frames)
+        n, h, w, _ = frames.shape
+        if out is None:
+            out = self._pooled_pinned(frames.shape, np.uint16) if frames.nbytes <= (64 << 20) else np.empty_like(frames)
+        elif out.shape != frames.shape or out.dtype != np.uint16 or not out.flags.c_contiguous:
+            raise ValueError("out must be a C-contiguous uint16 array of the input's shape")
+        kind = MEM_PINNED if (self.mem_kind(frames) == MEM_PINNED and self.mem_kind(out) == MEM_PINNED) else MEM_HOST
+        pp = processed.ctypes.data_as(_i32p) if processed is not None else None
+        self._ck(self._lib.rv_chain_u16(self._h, frames.ctypes.data, out.ctypes.data, n, h, w, 6 * w, 6 * w, C.byref(params), kind,
+                                        pp, None))
+        return out
+
+    def chain_u16_device(self, in_ptr, out_ptr, n, h, w, params, in_pitch=None, out_pitch=None, stream=None):
+        """rv_chain_u16 over device pointers (ints, pitches in bytes): asynchronous on `stream` (a cudaStream_t int) when given,
+        else synchronous on the context's stream."""
+        check_u16_params(params)
+        self._ck(self._lib.rv_chain_u16(self._h, C.c_void_p(in_ptr), C.c_void_p(out_ptr), n, h, w, in_pitch or 6 * w,
+                                        out_pitch or 6 * w, C.byref(params), MEM_DEVICE, None, C.c_void_p(stream) if stream else None))
 
     def chain_device(self, in_ptr, out_ptr, n, h, w, params, in_pitch=None, out_pitch=None, stream=None):
         """rv_chain_u8 over device pointers (ints); synchronises the stream before returning."""
@@ -493,6 +550,8 @@ class Context:
         return lut
 
     def clahe_dehaze(self, frames, space, clip_limit, grid):
+        if _is_u16(frames):
+            return self._chain_u16(frames, Params.make(space, clip_limit, grid, 0, clahe=True))
         _check_frames(frames)
         frames = np.ascontiguousarray(frames)
         n, h, w, _ = frames.shape
@@ -502,6 +561,8 @@ class Context:
         return out
 
     def median(self, frames, ksize):
+        if _is_u16(frames):
+            return self._chain_u16(frames, Params.make(ksize=ksize, clahe=False))
         _check_frames(frames)
         frames = np.ascontiguousarray(frames)
         n, h, w, _ = frames.shape
@@ -562,6 +623,13 @@ class Context:
                                                   C.c_void_p(stream) if stream else None))
 
     def gray_span(self, frames):
+        if _is_u16(frames):
+            _check_frames_u16(frames)
+            frames = np.ascontiguousarray(frames)
+            n, h, w, _ = frames.shape
+            span = np.empty(n, np.int32)
+            self._ck(self._lib.rv_gray_span_u16(self._h, frames.ctypes.data, n, h, w, 6 * w, span.ctypes.data, MEM_HOST))
+            return span
         _check_frames(frames)
         frames = np.ascontiguousarray(frames)
         n, h, w, _ = frames.shape

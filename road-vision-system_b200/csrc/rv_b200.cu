@@ -178,6 +178,8 @@ struct rv_ctx {
     int32_t *fflag = nullptr;               // page-locked: gate decision of the single-frame path
     void *fog = nullptr;                    // state of rv_fog.cu (fog synthesis), destroyed through fog_destroy
     void (*fog_destroy)(void *) = nullptr;
+    void *u16 = nullptr;                    // state of rv_u16.cu (16-bit frames), destroyed through u16_destroy
+    void (*u16_destroy)(void *) = nullptr;
     StagePool *stage = nullptr;             // helper threads + page-locked staging frame for pageable single-frame input
     HostBuf fstage;                         // page-locked staging frame of the optional helper-thread upload
     long stage_threads = 0;                 // option "stage_threads": helpers next to the caller; 0 (default) = the driver stages pageable
@@ -1169,6 +1171,8 @@ int rv_internal_fail(rv_ctx *ctx, int code, const char *fmt, ...)
 void rv_internal_count_launches(rv_ctx *ctx, long n) { ctx->launches += n; }
 void *rv_internal_get_fog(rv_ctx *ctx) { return ctx->fog; }
 void rv_internal_set_fog(rv_ctx *ctx, void *state, void (*destroy)(void *)) { ctx->fog = state; ctx->fog_destroy = destroy; }
+void *rv_internal_get_u16(rv_ctx *ctx) { return ctx->u16; }
+void rv_internal_set_u16(rv_ctx *ctx, void *state, void (*destroy)(void *)) { ctx->u16 = state; ctx->u16_destroy = destroy; }
 
 extern "C" {
 
@@ -1266,6 +1270,7 @@ void rv_destroy(rv_ctx *ctx)
     if (ctx->stage) { ctx->stage->stop(); delete ctx->stage; }
     if (ctx->fstage.p) cudaFreeHost(ctx->fstage.p);
     if (ctx->fog && ctx->fog_destroy) ctx->fog_destroy(ctx->fog);
+    if (ctx->u16 && ctx->u16_destroy) ctx->u16_destroy(ctx->u16);
     if (ctx->fstream) cudaStreamDestroy(ctx->fstream);
     if (ctx->fflag) cudaFreeHost(ctx->fflag);
     for (const TimedLaunch &t : ctx->timed) { cudaEventDestroy(t.a); cudaEventDestroy(t.b); }

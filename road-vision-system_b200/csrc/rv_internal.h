@@ -1,5 +1,5 @@
 /*
- * rv_internal.h -- the few things other translation units of librv_b200.so (rv_fog.cu) need from the context that rv_b200.cu
+ * rv_internal.h -- the few things other translation units of librv_b200.so (rv_fog.cu, rv_u16.cu) need from the context that rv_b200.cu
  * owns.  Not part of the C ABI (include/rv_b200.h).
  */
 #pragma once
@@ -11,3 +11,5 @@ int rv_internal_fail(rv_ctx *ctx, int code, const char *fmt, ...);      /* recor
 void rv_internal_count_launches(rv_ctx *ctx, long n);
 void *rv_internal_get_fog(rv_ctx *ctx);
 void rv_internal_set_fog(rv_ctx *ctx, void *state, void (*destroy)(void *));
+void *rv_internal_get_u16(rv_ctx *ctx);
+void rv_internal_set_u16(rv_ctx *ctx, void *state, void (*destroy)(void *));

@@ -6,7 +6,7 @@ import numpy as np
 
 
 class PreprocessOp(ABC):
-    """`op(image) -> image`; image is BGR (H,W,3) uint8; unknown params are kept and ignored."""
+    """`op(image) -> image`; image is BGR (H,W,3) uint8 (or uint16); unknown params are kept and ignored."""
 
     def __init__(self, **params: Any):
         self.params = params
@@ -32,3 +32,15 @@ def as_bgr_u8(image):
     if image.shape[0] < 1 or image.shape[1] < 1:
         raise ValueError("empty image")
     return np.ascontiguousarray(image)
+
+
+def as_bgr_frame(image):
+    """as_bgr_u8, but also admitting (H,W,3) uint16 frames (HDR sensors, cv2.imread(..., IMREAD_ANYDEPTH)), which the reference
+    hands to cv2's 16-bit path unchanged.  Any strides; returns a C-contiguous array of the input's dtype."""
+    if isinstance(image, np.ndarray) and image.dtype == np.uint16:
+        if image.ndim != 3 or image.shape[2] != 3:
+            raise ValueError(f"image must have shape (H,W,3), got {image.shape}")
+        if image.shape[0] < 1 or image.shape[1] < 1:
+            raise ValueError("empty image")
+        return np.ascontiguousarray(image)
+    return as_bgr_u8(image)

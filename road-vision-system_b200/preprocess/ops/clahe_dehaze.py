@@ -3,8 +3,10 @@
 Same name, params and per-frame contract; the cv2.cvtColor / split / createCLAHE().apply /
 merge / cvtColor sequence (:19-30) runs as the sm_100a kernels behind rv_clahe_dehaze.
 """
-from ..._native import default_context
-from ..base import PreprocessOp, as_bgr_u8
+import numpy as np
+
+from ..._native import Params, check_u16_params, default_context
+from ..base import PreprocessOp, as_bgr_frame
 
 
 def coerce(params):
@@ -16,10 +18,15 @@ def coerce(params):
 
 
 class CLAHEDehaze(PreprocessOp):
-    """CLAHE on the luminance channel. params: space "YCrCb"|"LAB", clip_limit float, tile_grid int."""
+    """CLAHE on the luminance channel. params: space "YCrCb"|"LAB", clip_limit float, tile_grid int.
+
+    uint16 frames run cv2's 16-bit chain (65,536-bin histograms) in YCrCb with tile_grid <= 64; LAB raises ValueError there, as
+    cv2 has no 16-bit LAB."""
 
     def __call__(self, image):
         space, clip_limit, grid = coerce(self.params)
-        img = as_bgr_u8(image)
+        img = as_bgr_frame(image)
+        if img.dtype == np.uint16:
+            check_u16_params(Params.make(space, clip_limit, grid, 0, clahe=True))      # LAB / grid > 64: before the GPU
         ctx = default_context(self.params.get("device"))
         return ctx.clahe_dehaze(img[None], space, clip_limit, grid)[0]

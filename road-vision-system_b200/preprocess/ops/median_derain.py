@@ -1,6 +1,8 @@
 """MedianDerain -- drop-in for /root/reference/src/preprocess/ops/median_derain.py:4-14."""
-from ..._native import default_context
-from ..base import PreprocessOp, as_bgr_u8
+import numpy as np
+
+from ..._native import Params, check_u16_params, default_context
+from ..base import PreprocessOp, as_bgr_frame
 
 
 def coerce(params):
@@ -12,10 +14,12 @@ def coerce(params):
 
 
 class MedianDerain(PreprocessOp):
-    """k x k median per channel, BORDER_REPLICATE (cv2.medianBlur semantics). params: ksize 3/5/7/9."""
+    """k x k median per channel, BORDER_REPLICATE (cv2.medianBlur semantics). params: ksize 3/5/7/9 (3/5 on uint16 frames, as cv2)."""
 
     def __call__(self, image):
         k = coerce(self.params)
-        img = as_bgr_u8(image)
+        img = as_bgr_frame(image)
+        if img.dtype == np.uint16:
+            check_u16_params(Params.make(ksize=k, clahe=False))        # k 7 / 9: before the GPU
         ctx = default_context(self.params.get("device"))
         return ctx.median(img[None], k)[0]

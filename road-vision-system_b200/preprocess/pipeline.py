@@ -10,8 +10,8 @@ from typing import Any, Dict
 
 import numpy as np
 
-from .._native import DeviceArray, Params, default_context
-from .base import as_bgr_u8
+from .._native import DeviceArray, Params, check_u16_params, default_context
+from .base import as_bgr_frame
 from .ops import CLAHEDehaze, MedianDerain
 from .ops import clahe_dehaze as _clahe
 from .ops import median_derain as _median
@@ -50,7 +50,7 @@ class PreprocessPipeline:
 
     def _low_contrast(self, image) -> bool:
         """pipeline.py:24-30: gray span < thresh (gray = cv2 BGR2GRAY fixed point, computed on the GPU)."""
-        span = int(self._ctx().gray_span(as_bgr_u8(image)[None])[0])
+        span = int(self._ctx().gray_span(as_bgr_frame(image)[None])[0])
         return span < self._gate()[1]
 
     def _segments(self):
@@ -93,32 +93,43 @@ class PreprocessPipeline:
                 i += 1
         return segs
 
+    @staticmethod
+    def _check_u16(segs):
+        """16-bit frames: every fused GPU pass must have a 16-bit path (YCrCb, k 3 / 5, grid <= 64) -- checked before any frame
+        reaches the GPU, so that a LAB / k 7 / 9 chain fails with ValueError instead of after the gate or a foreign operator ran."""
+        for sg in segs:
+            if isinstance(sg, Params):
+                check_u16_params(sg)
+
     # -- per-frame contract --------------------------------------------------------------
     def __call__(self, image: np.ndarray, ts: float = None) -> np.ndarray:
         if not self.enabled or not self.ops:
             return image
         segs = self._segments()
+        if isinstance(image, np.ndarray) and image.dtype != np.uint8 and image.dtype == np.uint16:
+            self._check_u16(segs)
         if self._gate()[0]:
             if len(segs) == 1 and isinstance(segs[0], Params):
                 # one fused pass: the gate's gray span comes out of the histogram pass of the same upload
                 seg = segs[0]
                 seg.gate_enable, seg.gate_thresh = 1, self._gate()[1]
                 flag = np.ones(1, np.int32)
-                out = self._ctx().chain(as_bgr_u8(image)[None], seg, processed=flag)[0]
+                out = self._ctx().chain(as_bgr_frame(image)[None], seg, processed=flag)[0]
                 return out if flag[0] else image          # skipped: the input object itself, as pipeline.py:39-40
             if not self._low_contrast(image):
                 return image
         out = image
         for seg in segs:
             if isinstance(seg, Params):
-                out = self._ctx().chain(as_bgr_u8(out)[None], seg)[0]
+                out = self._ctx().chain(as_bgr_frame(out)[None], seg)[0]
             else:
                 out = seg(out)
         return out
 
     # -- new: batched multi-frame entry --------------------------------------------------
     def process_batch(self, frames: np.ndarray, out: np.ndarray = None) -> np.ndarray:
-        """(B,H,W,3) uint8 -> (B,H,W,3) uint8; equals B per-frame calls bit for bit.
+        """(B,H,W,3) uint8 -> (B,H,W,3) uint8; equals B per-frame calls bit for bit.  uint16 frames give uint16 results (cv2's
+        16-bit chain: YCrCb only, median k 3 / 5, tile_grid <= 64).
 
         `frames` / `out` may be pinned arrays from `Context.pinned_empty` (fastest: H2D, kernels
         and D2H of consecutive chunks overlap).  Frames the low-contrast gate skips are copied
@@ -132,8 +143,11 @@ class PreprocessPipeline:
             if out != "device":
                 raise ValueError('out must be an array, None or "device"')
             return self._process_batch_keep(frames)
-        if not isinstance(frames, np.ndarray) or frames.ndim != 4 or frames.shape[3] != 3 or frames.dtype != np.uint8:
-            raise ValueError("frames must be a (B,H,W,3) uint8 numpy array (or a torch CUDA uint8 tensor of that shape)")
+        if not isinstance(frames, np.ndarray) or frames.ndim != 4 or frames.shape[3] != 3 or \
+                (frames.dtype != np.uint8 and frames.dtype != np.uint16):
+            raise ValueError("frames must be a (B,H,W,3) uint8 or uint16 numpy array (or a torch CUDA tensor of that shape)")
+        if frames.dtype == np.uint16 and self.enabled and self.ops:
+            self._check_u16(self._segments())
         if not self.enabled or not self.ops:
             if out is None:
                 return frames
@@ -171,17 +185,30 @@ class PreprocessPipeline:
 
     def _process_batch_keep(self, frames):
         """Host frames in, result left on the GPU (no D2H at all)."""
-        if not isinstance(frames, np.ndarray) or frames.ndim != 4 or frames.shape[3] != 3 or frames.dtype != np.uint8:
-            raise ValueError("frames must be a (B,H,W,3) uint8 numpy array")
+        if not isinstance(frames, np.ndarray) or frames.ndim != 4 or frames.shape[3] != 3 or \
+                (frames.dtype != np.uint8 and frames.dtype != np.uint16):
+            raise ValueError("frames must be a (B,H,W,3) uint8 or uint16 numpy array")
+        segs = self._segments() if (self.enabled and self.ops) else []
+        if frames.dtype == np.uint16:
+            self._check_u16(segs)
         ctx = self._ctx()
         frames = np.ascontiguousarray(frames)
-        segs = self._segments() if (self.enabled and self.ops) else []
         if not segs or self._gate()[0] or not all(isinstance(sg, Params) for sg in segs):
             # identity, gated or foreign operators: compute on the host path, then upload
             res = self.process_batch(frames)
-            dev = DeviceArray(ctx, res.shape)
+            dev = DeviceArray(ctx, res.shape, res.dtype)
             ctx._ck(ctx._lib.rv_memcpy(ctx._h, dev.ptr, np.ascontiguousarray(res).ctypes.data, dev.nbytes, 0))
             return dev
+        if frames.dtype == np.uint16:
+            # upload once, then every pass runs device to device
+            b, h, w, _ = frames.shape
+            cur = DeviceArray(ctx, frames.shape, np.uint16)
+            ctx._ck(ctx._lib.rv_memcpy(ctx._h, cur.ptr, frames.ctypes.data, cur.nbytes, 0))
+            for sg in segs:
+                dst = DeviceArray(ctx, frames.shape, np.uint16)
+                ctx.chain_u16_device(cur.ptr, dst.ptr, b, h, w, sg)
+                cur = dst
+            return cur
         cur = frames
         for sg in segs:
             dst = DeviceArray(ctx, frames.shape)
@@ -194,11 +221,15 @@ class PreprocessPipeline:
         """Device-resident batch: a contiguous torch CUDA uint8 tensor (B,H,W,3) in, a tensor of the same kind out.
         Work is enqueued on torch's current stream (no host synchronisation): use the result with torch as usual."""
         import torch
-        if frames.dtype != torch.uint8 or frames.dim() != 4 or frames.shape[3] != 3 or not frames.is_contiguous():
-            raise ValueError("frames must be a contiguous (B,H,W,3) uint8 CUDA tensor")
-        if out is not None and not (_is_cuda_tensor(out) and out.dtype == torch.uint8 and tuple(out.shape) == tuple(frames.shape)
+        if (frames.dtype != torch.uint8 and frames.dtype != torch.uint16) or frames.dim() != 4 or frames.shape[3] != 3 or \
+                not frames.is_contiguous():
+            raise ValueError("frames must be a contiguous (B,H,W,3) uint8 or uint16 CUDA tensor")
+        if out is not None and not (_is_cuda_tensor(out) and out.dtype == frames.dtype and tuple(out.shape) == tuple(frames.shape)
                                     and out.device == frames.device and out.is_contiguous()):
-            raise ValueError("out must be a contiguous uint8 CUDA tensor of the input's shape on the input's device")
+            raise ValueError("out must be a contiguous CUDA tensor of the input's shape, dtype and device")
+        wide = frames.dtype == torch.uint16
+        if wide and self.enabled and self.ops:
+            self._check_u16(self._segments())
         if not self.enabled or not self.ops:
             return frames if out is None else out.copy_(frames)
         if self._gate()[0]:
@@ -213,7 +244,11 @@ class PreprocessPipeline:
         cur = frames
         for idx, sg in enumerate(segs):
             dst = out if (idx == len(segs) - 1 and out is not None) else torch.empty_like(frames)
-            if stream == 0:        # legacy default stream: run on the context's stream, synchronously
+            if wide:
+                if stream == 0:
+                    torch.cuda.current_stream(frames.device).synchronize()
+                ctx.chain_u16_device(cur.data_ptr(), dst.data_ptr(), b, h, w, sg, stream=stream or None)
+            elif stream == 0:        # legacy default stream: run on the context's stream, synchronously
                 torch.cuda.current_stream(frames.device).synchronize()
                 ctx.chain_device(cur.data_ptr(), dst.data_ptr(), b, h, w, sg)
             else:
@@ -237,6 +272,9 @@ class PreprocessPipeline:
         CLAHEDehaze -> MedianDerain pair and the down-scale is an exact integer (1080p -> 640), the resize happens inside
         the chain kernel and the full-resolution frames are only written if `want_frames` is set.
         """
+        if isinstance(frames, np.ndarray) and frames.dtype == np.uint16:
+            raise ValueError("process_batch_to_tensor takes uint8 frames: the detector input is built from 8-bit frames "
+                             "(run process_batch on uint16 frames and convert them to 8 bits first)")
         if not isinstance(frames, np.ndarray) or frames.ndim != 4 or frames.shape[3] != 3 or frames.dtype != np.uint8:
             raise ValueError("frames must be a (B,H,W,3) uint8 numpy array")
         ctx = self._ctx()
