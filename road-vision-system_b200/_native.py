@@ -231,13 +231,18 @@ def load_library():
     return _lib
 
 
-def _check_frames(frames):
+_U8 = (np.dtype(np.uint8),)
+_U8_U16 = (np.dtype(np.uint8), np.dtype(np.uint16))
+
+
+def _check_frames(frames, dtypes=_U8):
+    """(N,H,W,3) BGR frames of one of `dtypes`."""
     if not isinstance(frames, np.ndarray):
         raise TypeError("frames must be a numpy.ndarray")
-    if frames.dtype != np.uint8:
-        raise ValueError(f"uint8 BGR frames expected, got dtype {frames.dtype}")
+    if frames.dtype not in dtypes:
+        raise ValueError(f"{' or '.join(d.name for d in dtypes)} BGR frames expected, got dtype {frames.dtype}")
     if frames.ndim != 4 or frames.shape[3] != 3:
-        raise ValueError(f"(N,H,W,3) uint8 expected, got shape {frames.shape}")
+        raise ValueError(f"(N,H,W,3) {frames.dtype} expected, got shape {frames.shape}")
     if frames.shape[1] < 1 or frames.shape[2] < 1:
         raise ValueError("empty frame")
 
@@ -257,17 +262,6 @@ def check_u16_params(params):
                          "65,536-entry LUT)")
     if not params.clahe and params.ksize == 0:
         raise ValueError("nothing to do (no CLAHE, no median)")
-
-
-def _check_frames_u16(frames):
-    if frames.ndim != 4 or frames.shape[3] != 3:
-        raise ValueError(f"(N,H,W,3) uint16 expected, got shape {frames.shape}")
-    if frames.shape[1] < 1 or frames.shape[2] < 1:
-        raise ValueError("empty frame")
-
-
-def _is_u16(frames):
-    return isinstance(frames, np.ndarray) and frames.dtype != np.uint8 and frames.dtype == np.uint16
 
 
 class _Lease(np.ndarray):
@@ -394,10 +388,13 @@ class Context:
 
     # -- the chain -----------------------------------------------------------------------
     def chain(self, frames, params, out=None, processed=None):
-        """rv_chain_u8 over host frames (N,H,W,3) uint8 (rv_chain_u16 for uint16 frames); returns a new (or `out`) array."""
-        if _is_u16(frames):
-            return self._chain_u16(frames, params, out, processed)
-        _check_frames(frames)
+        """rv_chain_u8 over host frames (N,H,W,3) uint8, rv_chain_u16 over uint16 ones; returns a new (or `out`) array."""
+        _check_frames(frames, _U8_U16)
+        if frames.dtype == np.uint8:
+            fn, bpp = self._lib.rv_chain_u8, 3
+        else:
+            check_u16_params(params)
+            fn, bpp = self._lib.rv_chain_u16, 6
         if not frames.flags.c_contiguous:
             frames = np.ascontiguousarray(frames)
         n, h, w, _ = frames.shape
@@ -405,12 +402,12 @@ class Context:
         if out is None:
             # small results (the per-frame contract) land in recycled page-locked memory: the D2H copy is a plain DMA
             if frames.nbytes <= (64 << 20):
-                out = self._pooled_pinned(frames.shape)
+                out = self._pooled_pinned(frames.shape, frames.dtype)
                 out_addr = self._last_lease_addr
             else:
                 out = np.empty_like(frames)
-        elif out.shape != frames.shape or out.dtype != np.uint8 or not out.flags.c_contiguous:
-            raise ValueError("out must be a C-contiguous uint8 array of the input's shape")
+        elif out.shape != frames.shape or out.dtype != frames.dtype or not out.flags.c_contiguous:
+            raise ValueError(f"out must be a C-contiguous {frames.dtype} array of the input's shape")
         if out_addr is None:
             out_addr = out.ctypes.data
         if n == 1:
@@ -418,26 +415,9 @@ class Context:
         else:
             kind = MEM_PINNED if (self.mem_kind(frames) == MEM_PINNED and self.mem_kind(out) == MEM_PINNED) else MEM_HOST
         pp = processed.ctypes.data_as(_i32p) if processed is not None else None
-        rc = self._lib.rv_chain_u8(self._h, frames.ctypes.data, out_addr, n, h, w, 3 * w, 3 * w, C.byref(params), kind, pp, None)
+        rc = fn(self._h, frames.ctypes.data, out_addr, n, h, w, bpp * w, bpp * w, C.byref(params), kind, pp, None)
         if rc != 0:
             self._ck(rc)
-        return out
-
-    def _chain_u16(self, frames, params, out=None, processed=None):
-        """rv_chain_u16 over host frames (N,H,W,3) uint16."""
-        _check_frames_u16(frames)
-        check_u16_params(params)
-        if not frames.flags.c_contiguous:
-            frames = np.ascontiguousarray(frames)
-        n, h, w, _ = frames.shape
-        if out is None:
-            out = self._pooled_pinned(frames.shape, np.uint16) if frames.nbytes <= (64 << 20) else np.empty_like(frames)
-        elif out.shape != frames.shape or out.dtype != np.uint16 or not out.flags.c_contiguous:
-            raise ValueError("out must be a C-contiguous uint16 array of the input's shape")
-        kind = MEM_PINNED if (self.mem_kind(frames) == MEM_PINNED and self.mem_kind(out) == MEM_PINNED) else MEM_HOST
-        pp = processed.ctypes.data_as(_i32p) if processed is not None else None
-        self._ck(self._lib.rv_chain_u16(self._h, frames.ctypes.data, out.ctypes.data, n, h, w, 6 * w, 6 * w, C.byref(params), kind,
-                                        pp, None))
         return out
 
     def chain_u16_device(self, in_ptr, out_ptr, n, h, w, params, in_pitch=None, out_pitch=None, stream=None):
@@ -550,25 +530,10 @@ class Context:
         return lut
 
     def clahe_dehaze(self, frames, space, clip_limit, grid):
-        if _is_u16(frames):
-            return self._chain_u16(frames, Params.make(space, clip_limit, grid, 0, clahe=True))
-        _check_frames(frames)
-        frames = np.ascontiguousarray(frames)
-        n, h, w, _ = frames.shape
-        out = self._pooled_pinned(frames.shape) if frames.nbytes <= (64 << 20) else np.empty_like(frames)
-        self._ck(self._lib.rv_clahe_dehaze(self._h, frames.ctypes.data, out.ctypes.data, n, h, w, 3 * w, 3 * w,
-                                           SPACE_LAB if space == "LAB" else SPACE_YCRCB, float(clip_limit), int(grid), MEM_HOST))
-        return out
+        return self.chain(frames, Params.make(space, clip_limit, grid, 0, clahe=True))
 
     def median(self, frames, ksize):
-        if _is_u16(frames):
-            return self._chain_u16(frames, Params.make(ksize=ksize, clahe=False))
-        _check_frames(frames)
-        frames = np.ascontiguousarray(frames)
-        n, h, w, _ = frames.shape
-        out = self._pooled_pinned(frames.shape) if frames.nbytes <= (64 << 20) else np.empty_like(frames)
-        self._ck(self._lib.rv_median(self._h, frames.ctypes.data, out.ctypes.data, n, h, w, 3 * w, 3 * w, int(ksize), MEM_HOST))
-        return out
+        return self.chain(frames, Params.make(ksize=ksize, clahe=False))
 
     # -- detector-input stage (letterbox + RGB + CHW + /255 + fp16) ---------------------------
     @staticmethod
@@ -623,18 +588,12 @@ class Context:
                                                   C.c_void_p(stream) if stream else None))
 
     def gray_span(self, frames):
-        if _is_u16(frames):
-            _check_frames_u16(frames)
-            frames = np.ascontiguousarray(frames)
-            n, h, w, _ = frames.shape
-            span = np.empty(n, np.int32)
-            self._ck(self._lib.rv_gray_span_u16(self._h, frames.ctypes.data, n, h, w, 6 * w, span.ctypes.data, MEM_HOST))
-            return span
-        _check_frames(frames)
+        _check_frames(frames, _U8_U16)
+        fn, bpp = (self._lib.rv_gray_span, 3) if frames.dtype == np.uint8 else (self._lib.rv_gray_span_u16, 6)
         frames = np.ascontiguousarray(frames)
         n, h, w, _ = frames.shape
         span = np.empty(n, np.int32)
-        self._ck(self._lib.rv_gray_span(self._h, frames.ctypes.data, n, h, w, 3 * w, span.ctypes.data, MEM_HOST))
+        self._ck(fn(self._h, frames.ctypes.data, n, h, w, bpp * w, span.ctypes.data, MEM_HOST))
         return span
 
 

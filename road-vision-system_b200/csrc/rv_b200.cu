@@ -37,22 +37,9 @@ constexpr int NPIPE = RV_NPIPE;          // streams (and buffer sets) of the chu
 constexpr int NWS = NPIPE + 3;               // workspace sets: [0, NPIPE) host pipeline, NPIPE / NPIPE+1 device path, NPIPE+2 single-frame path
 constexpr int WS_FRAME = NPIPE + 2;
 
-struct Buf {
-    void *p = nullptr;
-    size_t cap = 0;
-};
-
 struct TimedLaunch {
     cudaEvent_t a, b;
     int which;                              // 0 k_luma_hist, 1 k_build_lut, 2 k_chain
-};
-
-// Ordering of a workspace set between streams: the event is recorded after the last kernel that touches the set; the next
-// user on a different stream waits for it first (two batches submitted on different caller streams never overlap on a set).
-struct WsSync {
-    cudaEvent_t ev = nullptr;
-    cudaStream_t last = nullptr;
-    bool used = false;
 };
 
 // Read-only device tables that depend on the frame geometry only; built once per geometry, uploaded on the stream that
@@ -73,7 +60,6 @@ struct LbTab {                              // cv2.resize tables of k_letterbox 
 constexpr int MAX_TABS = 32;
 constexpr int MAX_FRAME_GRAPHS = 16;
                 // geometries cached per context before the cache is flushed
-constexpr int MAX_FRAMES_PER_LAUNCH = 32768; // frames ride on gridDim.z / gridDim.y (limit 65535)
 
 }  // namespace
 
@@ -178,8 +164,7 @@ struct rv_ctx {
     int32_t *fflag = nullptr;               // page-locked: gate decision of the single-frame path
     void *fog = nullptr;                    // state of rv_fog.cu (fog synthesis), destroyed through fog_destroy
     void (*fog_destroy)(void *) = nullptr;
-    void *u16 = nullptr;                    // state of rv_u16.cu (16-bit frames), destroyed through u16_destroy
-    void (*u16_destroy)(void *) = nullptr;
+    U16Ws u16;                              // workspaces of rv_u16.cu (16-bit frames)
     StagePool *stage = nullptr;             // helper threads + page-locked staging frame for pageable single-frame input
     HostBuf fstage;                         // page-locked staging frame of the optional helper-thread upload
     long stage_threads = 0;                 // option "stage_threads": helpers next to the caller; 0 (default) = the driver stages pageable
@@ -248,6 +233,11 @@ void build_lab_hist_table(LabHistTabs &t)
     }
 }
 
+}  // namespace
+
+// ---- the host toolkit declared in rv_internal.h (shared with rv_fog.cu and rv_u16.cu) ------------------------------------
+namespace rv {
+
 int fail(rv_ctx *c, int code, const char *fmt, ...)
 {
     if (c) {
@@ -258,19 +248,6 @@ int fail(rv_ctx *c, int code, const char *fmt, ...)
     }
     return code;
 }
-
-#define CK(call)                                                                                         \
-    do {                                                                                                 \
-        cudaError_t e_ = (call);                                                                         \
-        if (e_ != cudaSuccess)                                                                           \
-            return fail(ctx, RV_ERR_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
-    } while (0)
-
-#define RV_TRY(call)              \
-    do {                          \
-        int rc_ = (call);         \
-        if (rc_ != RV_OK) return rc_; \
-    } while (0)
 
 int ensure(rv_ctx *ctx, Buf &b, size_t bytes)
 {
@@ -284,6 +261,83 @@ int ensure(rv_ctx *ctx, Buf &b, size_t bytes)
     b.cap = want;
     return RV_OK;
 }
+
+int ws_acquire(rv_ctx *ctx, WsSync &w, cudaStream_t st)
+{
+    if (w.used && w.last != st) CK(cudaStreamWaitEvent(st, w.ev, 0));
+    return RV_OK;
+}
+
+// (re-)arm the ordering event of a workspace set after the last work queued on `st` that touches it
+int ws_release(rv_ctx *ctx, WsSync &w, cudaStream_t st)
+{
+    CK(cudaEventRecord(w.ev, st));
+    w.last = st;
+    w.used = true;
+    return RV_OK;
+}
+
+int check_frames(rv_ctx *ctx, const void *in, const void *out, int n, int h, int w, size_t ipitch, size_t opitch, int bytes_per_pixel)
+{
+    if (!ctx) return RV_ERR_ARG;
+    if (!in || !out) return fail(ctx, RV_ERR_ARG, "null frame pointer");
+    if (n < 0 || h < 1 || w < 1) return fail(ctx, RV_ERR_ARG, "bad frame shape n=%d h=%d w=%d", n, h, w);
+    if (h > 32768 || w > 32768) return fail(ctx, RV_ERR_ARG, "frame too large (%dx%d)", w, h);
+    const size_t row = (size_t)bytes_per_pixel * w;
+    if (ipitch < row || opitch < row) return fail(ctx, RV_ERR_ARG, "pitch smaller than %d*w", bytes_per_pixel);
+    if (bytes_per_pixel == 6) {
+        if ((ipitch | opitch) & 1) return fail(ctx, RV_ERR_ARG, "16-bit frames need even pitches");
+        if (((uintptr_t)in | (uintptr_t)out) & 1) return fail(ctx, RV_ERR_ARG, "16-bit frames need 2-byte aligned buffers");
+    }
+    if (in != out && n > 0) {
+        // unified addressing: host and device ranges never coincide, so a numeric overlap is a real one.  Tiles read their
+        // neighbours' halo, so partially overlapping buffers would race exactly like in-place operation.
+        const uintptr_t a0 = (uintptr_t)in, a1 = a0 + (size_t)n * h * ipitch, b0 = (uintptr_t)out, b1 = b0 + (size_t)n * h * opitch;
+        if (a0 < b1 && b0 < a1) return fail(ctx, RV_ERR_ARG, "input and output ranges overlap");
+    }
+    return RV_OK;
+}
+
+int check_kind(rv_ctx *ctx, int kind)
+{
+    if (kind != RV_MEM_HOST && kind != RV_MEM_HOST_PINNED && kind != RV_MEM_DEVICE) return fail(ctx, RV_ERR_ARG, "bad memory kind %d", kind);
+    return RV_OK;
+}
+
+// pipeline.py:24-30 compares an integer span with a Python float: span < t  <=>  span < ceil(t) for integer spans.  The
+// decision is taken in integers on the device so that it can never differ from the per-frame path at the boundary.  A gray
+// span is at most 65535 (16-bit frames), so every threshold above 65536 decides like 65536.
+static int gate_thresh_int(double t)
+{
+    if (!(t == t)) return -1;                               // NaN: every comparison is false, nothing is processed
+    const double c = ceil(t);
+    if (c > 65536.0) return 65536;
+    if (c < -1.0) return -1;
+    return (int)c;
+}
+
+void launch_gate_flags(rv_ctx *ctx, const int32_t *mm, int n, double thresh, int32_t *flags, cudaStream_t st)
+{
+    k_gate_flags<<<(n + 127) / 128, 128, 0, st>>>(mm, n, gate_thresh_int(thresh), flags);
+    ctx->launches++;
+}
+
+int write_spans(rv_ctx *ctx, const int32_t *mm, int n, int32_t *span, int mem_kind)
+{
+    int32_t *tmp = mem_kind == RV_MEM_DEVICE ? new (std::nothrow) int32_t[n] : span;
+    if (!tmp) return fail(ctx, RV_ERR_NOMEM, "host alloc");
+    for (int i = 0; i < n; ++i) tmp[i] = mm[2 * i + 1] - mm[2 * i];
+    if (mem_kind == RV_MEM_DEVICE) {
+        const cudaError_t e = cudaMemcpy(span, tmp, (size_t)n * 4, cudaMemcpyHostToDevice);
+        delete[] tmp;
+        if (e != cudaSuccess) return fail(ctx, RV_ERR_CUDA, "gray span copy: %s", cudaGetErrorString(e));
+    }
+    return RV_OK;
+}
+
+}  // namespace rv
+
+namespace {
 
 cudaEvent_t get_event(rv_ctx *ctx)
 {
@@ -309,55 +363,11 @@ struct ScopedTiming {                       // records an event pair around one 
     }
 };
 
-// clahe.cpp geometry (A.3): both dimensions are padded when either is not divisible by the grid
-Geo make_geo(int h, int w, int grid)
-{
-    Geo g;
-    g.H = h; g.W = w; g.grid = grid;
-    int eh = h, ew = w;
-    if (w % grid != 0 || h % grid != 0) {
-        ew = w + (grid - w % grid);
-        eh = h + (grid - h % grid);
-    }
-    g.tw = ew / grid;
-    g.th = eh / grid;
-    g.inv_tw = 1.0f / (float)g.tw;
-    g.inv_th = 1.0f / (float)g.th;
-    return g;
-}
-
 int clip_int(double clip_limit, const Geo &g)
 {
     if (!(clip_limit > 0.0)) return 0;
     int c = (int)(clip_limit * (double)(g.tw * g.th) / 256.0);
     return std::max(c, 1);
-}
-
-int check_frames(rv_ctx *ctx, const void *in, const void *out, int n, int h, int w, size_t ipitch, size_t opitch)
-{
-    if (!ctx) return RV_ERR_ARG;
-    if (!in || !out) return fail(ctx, RV_ERR_ARG, "null frame pointer");
-    if (n < 0 || h < 1 || w < 1) return fail(ctx, RV_ERR_ARG, "bad frame shape n=%d h=%d w=%d", n, h, w);
-    if (h > 32768 || w > 32768) return fail(ctx, RV_ERR_ARG, "frame too large (%dx%d)", w, h);
-    if (ipitch < (size_t)3 * w || opitch < (size_t)3 * w) return fail(ctx, RV_ERR_ARG, "pitch smaller than 3*w");
-    if (in != out && n > 0) {
-        // unified addressing: host and device ranges never coincide, so a numeric overlap is a real one.  Tiles read their
-        // neighbours' halo, so partially overlapping buffers would race exactly like in-place operation.
-        const uintptr_t a0 = (uintptr_t)in, a1 = a0 + (size_t)n * h * ipitch, b0 = (uintptr_t)out, b1 = b0 + (size_t)n * h * opitch;
-        if (a0 < b1 && b0 < a1) return fail(ctx, RV_ERR_ARG, "input and output ranges overlap");
-    }
-    return RV_OK;
-}
-
-// pipeline.py:24-30 compares an integer span with a Python float: span < t  <=>  span < ceil(t) for integer spans.  The
-// decision is taken in integers on the device so that it can never differ from the per-frame path at the boundary.
-int gate_thresh_int(double t)
-{
-    if (!(t == t)) return -1;                               // NaN: every comparison is false, nothing is processed
-    const double c = ceil(t);
-    if (c > 1024.0) return 1024;
-    if (c < -1.0) return -1;
-    return (int)c;
 }
 
 int check_params(rv_ctx *ctx, const rv_params *p)
@@ -608,10 +618,9 @@ int run_group(rv_ctx *ctx, int ws, const uint8_t *din, size_t ipitch, size_t ifs
     // the previous user of this workspace set may have been on another stream (two caller streams, or a stage-level call)
     WsSync &wsy = ctx->wsync[ws];
     if (!capturing) {
-        if (wsy.used && wsy.last != sp) CK(cudaStreamWaitEvent(sp, wsy.ev, 0));
-        if (wsy.used && st != sp && wsy.last != st) CK(cudaStreamWaitEvent(st, wsy.ev, 0));
+        RV_TRY(ws_acquire(ctx, wsy, sp));
+        if (st != sp) RV_TRY(ws_acquire(ctx, wsy, st));
     }
-    const int gate_t = gate_thresh_int(p->gate_thresh);
     ChainArgs a;
     a.src = din; a.spitch = ipitch; a.sfstride = ifs;
     a.dst = dout; a.dpitch = opitch; a.dfstride = ofs;
@@ -628,8 +637,7 @@ int run_group(rv_ctx *ctx, int ws, const uint8_t *din, size_t ipitch, size_t ifs
             RV_TRY(ensure(ctx, ctx->flags[ws], (size_t)n * 4));
             RV_TRY(launch_hist(ctx, din, ipitch, ifs, a.g, RV_SPACE_YCRCB, n, (int32_t *)ctx->hist[ws].p, nullptr,
                                (int32_t *)ctx->mm[ws].p, sp));
-            k_gate_flags<<<(n + 127) / 128, 128, 0, sp>>>((int32_t *)ctx->mm[ws].p, n, gate_t, (int32_t *)ctx->flags[ws].p);
-            ctx->launches++;
+            launch_gate_flags(ctx, (int32_t *)ctx->mm[ws].p, n, p->gate_thresh, (int32_t *)ctx->flags[ws].p, sp);
             a.flags = (int32_t *)ctx->flags[ws].p;
         }
         RV_TRY(launch_chain(ctx, 2, a, n, p->ksize, st));
@@ -648,8 +656,7 @@ int run_group(rv_ctx *ctx, int ws, const uint8_t *din, size_t ipitch, size_t ifs
         RV_TRY(launch_hist(ctx, din, ipitch, ifs, g, p->space, n, (int32_t *)ctx->hist[ws].p, nullptr, mm, sp));
         RV_TRY(launch_lut(ctx, (int32_t *)ctx->hist[ws].p, g, p->clip_limit, n, nullptr, (uint32_t *)ctx->quads[ws].p, sp));
         if (p->gate_enable) {
-            k_gate_flags<<<(n + 127) / 128, 128, 0, sp>>>(mm, n, gate_t, (int32_t *)ctx->flags[ws].p);
-            ctx->launches++;
+            launch_gate_flags(ctx, mm, n, p->gate_thresh, (int32_t *)ctx->flags[ws].p, sp);
             a.flags = (int32_t *)ctx->flags[ws].p;
         }
         a.quads = (uint32_t *)ctx->quads[ws].p;
@@ -671,27 +678,7 @@ int run_group(rv_ctx *ctx, int ws, const uint8_t *din, size_t ipitch, size_t ifs
     }
     CK(cudaGetLastError());
     if (capturing) return RV_OK;
-    CK(cudaEventRecord(wsy.ev, st));        // (a caller that reads the flags afterwards records it again, see ws_release)
-    wsy.last = st;
-    wsy.used = true;
-    return RV_OK;
-}
-
-// re-arm the ordering event of a workspace set after more work that reads it has been queued on `st`
-int ws_release(rv_ctx *ctx, int ws, cudaStream_t st)
-{
-    WsSync &wsy = ctx->wsync[ws];
-    CK(cudaEventRecord(wsy.ev, st));
-    wsy.last = st;
-    wsy.used = true;
-    return RV_OK;
-}
-
-int ws_acquire(rv_ctx *ctx, int ws, cudaStream_t st)
-{
-    WsSync &wsy = ctx->wsync[ws];
-    if (wsy.used && wsy.last != st) CK(cudaStreamWaitEvent(st, wsy.ev, 0));
-    return RV_OK;
+    return ws_release(ctx, wsy, st);        // (a caller that reads the flags afterwards releases the set again)
 }
 
 long auto_group(const rv_ctx *ctx, int h, int w)
@@ -1004,7 +991,7 @@ int chain_pipe(rv_ctx *ctx, const PipeJob &j, int n, int h, int w, const rv_para
             if (flags) CK(cudaMemcpyAsync(j.processed + f0, flags, (size_t)g * 4, cudaMemcpyDeviceToHost, st));
             else for (int i = 0; i < g; ++i) j.processed[f0 + i] = 1;
         }
-        RV_TRY(ws_release(ctx, s, st));
+        RV_TRY(ws_release(ctx, ctx->wsync[s], st));
     }
     return RV_OK;
 }
@@ -1158,21 +1145,10 @@ int check_lb_args(rv_ctx *ctx, const void *tensor, int S, int pad_value)
 
 int rv_internal_device(const rv_ctx *ctx) { return ctx->device; }
 void *rv_internal_stream(rv_ctx *ctx) { return ctx->stream; }
-int rv_internal_fail(rv_ctx *ctx, int code, const char *fmt, ...)
-{
-    if (ctx) {
-        va_list ap;
-        va_start(ap, fmt);
-        vsnprintf(ctx->err, sizeof ctx->err, fmt, ap);
-        va_end(ap);
-    }
-    return code;
-}
 void rv_internal_count_launches(rv_ctx *ctx, long n) { ctx->launches += n; }
 void *rv_internal_get_fog(rv_ctx *ctx) { return ctx->fog; }
 void rv_internal_set_fog(rv_ctx *ctx, void *state, void (*destroy)(void *)) { ctx->fog = state; ctx->fog_destroy = destroy; }
-void *rv_internal_get_u16(rv_ctx *ctx) { return ctx->u16; }
-void rv_internal_set_u16(rv_ctx *ctx, void *state, void (*destroy)(void *)) { ctx->u16 = state; ctx->u16_destroy = destroy; }
+U16Ws &rv_internal_u16(rv_ctx *ctx) { return ctx->u16; }
 
 extern "C" {
 
@@ -1220,6 +1196,7 @@ int rv_create(int device, rv_ctx **out)
             if (cudaEventCreateWithFlags(e, cudaEventDisableTiming) != cudaSuccess) { delete ctx; return RV_ERR_CUDA; }
         for (WsSync &w : ctx->wsync)
             if (cudaEventCreateWithFlags(&w.ev, cudaEventDisableTiming) != cudaSuccess) { delete ctx; return RV_ERR_CUDA; }
+        if (cudaEventCreateWithFlags(&ctx->u16.sync.ev, cudaEventDisableTiming) != cudaSuccess) { delete ctx; return RV_ERR_CUDA; }
         if (cudaStreamCreateWithFlags(&ctx->fstream, cudaStreamNonBlocking) != cudaSuccess) { delete ctx; return RV_ERR_CUDA; }
         if (cudaHostAlloc((void **)&ctx->fflag, 64, cudaHostAllocDefault) != cudaSuccess) { delete ctx; return RV_ERR_NOMEM; }
     }
@@ -1260,17 +1237,20 @@ void rv_destroy(rv_ctx *ctx)
             if (set[i].p) cudaFree(set[i].p);
     for (Buf &b : ctx->dlb)
         if (b.p) cudaFree(b.p);
+    for (Buf *b : {&ctx->u16.lut, &ctx->u16.mid, &ctx->u16.din, &ctx->u16.dout, &ctx->u16.mm, &ctx->u16.flags})
+        if (b->p) cudaFree(b->p);
+    if (ctx->u16.hflags) cudaFreeHost(ctx->u16.hflags);
     if (ctx->scratch.p) cudaFree(ctx->scratch.p);
     if (ctx->lbfull.p) cudaFree(ctx->lbfull.p);
     for (ColTab &t : ctx->coltabs) { cudaFree(t.dev); cudaFreeHost(t.host); cudaEventDestroy(t.ready); }
     for (LbTab &t : ctx->lbtabs) { cudaFree(t.dev); cudaFreeHost(t.host); cudaEventDestroy(t.ready); }
     for (WsSync &w : ctx->wsync)
         if (w.ev) cudaEventDestroy(w.ev);
+    if (ctx->u16.sync.ev) cudaEventDestroy(ctx->u16.sync.ev);
     drop_frame_graphs(ctx);
     if (ctx->stage) { ctx->stage->stop(); delete ctx->stage; }
     if (ctx->fstage.p) cudaFreeHost(ctx->fstage.p);
     if (ctx->fog && ctx->fog_destroy) ctx->fog_destroy(ctx->fog);
-    if (ctx->u16 && ctx->u16_destroy) ctx->u16_destroy(ctx->u16);
     if (ctx->fstream) cudaStreamDestroy(ctx->fstream);
     if (ctx->fflag) cudaFreeHost(ctx->fflag);
     for (const TimedLaunch &t : ctx->timed) { cudaEventDestroy(t.a); cudaEventDestroy(t.b); }
@@ -1413,14 +1393,9 @@ int rv_kernel_time_reset(rv_ctx *ctx)
 }
 
 namespace {
-int check_kind(rv_ctx *ctx, int kind)
-{
-    if (kind != RV_MEM_HOST && kind != RV_MEM_HOST_PINNED && kind != RV_MEM_DEVICE) return fail(ctx, RV_ERR_ARG, "bad memory kind %d", kind);
-    return RV_OK;
-}
 int check_chain_call(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h, int w, size_t in_pitch, size_t out_pitch, const rv_params *p)
 {
-    RV_TRY(check_frames(ctx, in, out, n, h, w, in_pitch, out_pitch));
+    RV_TRY(check_frames(ctx, in, out, n, h, w, in_pitch, out_pitch, 3));
     RV_TRY(check_params(ctx, p));
     if (!p->clahe && p->ksize == 0) return fail(ctx, RV_ERR_ARG, "nothing to do (no CLAHE, no median)");
     if (in == out) return fail(ctx, RV_ERR_ARG, "in-place operation is not supported (tiles read their neighbours' halo)");
@@ -1451,7 +1426,7 @@ int rv_submit_io(rv_ctx *ctx, const rv_io *io, int n, int h, int w, const rv_par
     if (!io->out && !io->tensor) return fail(ctx, RV_ERR_ARG, "neither a frame output nor a tensor output was given");
     RV_TRY(check_kind(ctx, io->in_kind));
     // with no frame output the input stands in for it in the shape / pitch checks
-    RV_TRY(check_frames(ctx, io->in, io->out ? io->out : io->in, n, h, w, io->in_pitch, io->out ? io->out_pitch : io->in_pitch));
+    RV_TRY(check_frames(ctx, io->in, io->out ? io->out : io->in, n, h, w, io->in_pitch, io->out ? io->out_pitch : io->in_pitch, 3));
     RV_TRY(check_params(ctx, p));
     if (!p->clahe && p->ksize == 0) return fail(ctx, RV_ERR_ARG, "nothing to do (no CLAHE, no median)");
     if (io->out) {
@@ -1502,7 +1477,7 @@ int rv_chain_u8(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h, int 
 int rv_luma_hist(rv_ctx *ctx, const uint8_t *in, int n, int h, int w, size_t pitch, int space, int grid, int32_t *hist,
                  uint8_t *luma, int32_t *gray_minmax, int mem_kind)
 {
-    RV_TRY(check_frames(ctx, in, in, n, h, w, pitch, pitch));
+    RV_TRY(check_frames(ctx, in, in, n, h, w, pitch, pitch, 3));
     if (!hist) return fail(ctx, RV_ERR_ARG, "null hist");
     if (grid < 1 || grid > 256) return fail(ctx, RV_ERR_ARG, "bad grid %d", grid);
     if (n == 0) return RV_OK;
@@ -1575,7 +1550,7 @@ int rv_letterbox_geometry(int h, int w, int S, int32_t *new_w, int32_t *new_h, i
 
 int rv_letterbox_f16(rv_ctx *ctx, const uint8_t *in, int n, int h, int w, size_t pitch, uint16_t *out, int S, int pad_value, int mem_kind)
 {
-    RV_TRY(check_frames(ctx, in, in, n, h, w, pitch, pitch));
+    RV_TRY(check_frames(ctx, in, in, n, h, w, pitch, pitch, 3));
     if (!out || S < 1 || S > 8192 || pad_value < 0 || pad_value > 255) return fail(ctx, RV_ERR_ARG, "bad letterbox arguments");
     if (n == 0) return RV_OK;
     CK(cudaSetDevice(ctx->device));
@@ -1593,7 +1568,7 @@ int rv_letterbox_f16(rv_ctx *ctx, const uint8_t *in, int n, int h, int w, size_t
 int rv_chain_letterbox_f16(rv_ctx *ctx, const uint8_t *in, int n, int h, int w, size_t in_pitch, const rv_params *p,
                            uint16_t *out, int S, int pad_value, uint8_t *full_out, size_t full_pitch, int mem_kind, void *stream)
 {
-    RV_TRY(check_frames(ctx, in, full_out ? full_out : in, n, h, w, in_pitch, full_out ? full_pitch : in_pitch));
+    RV_TRY(check_frames(ctx, in, full_out ? full_out : in, n, h, w, in_pitch, full_out ? full_pitch : in_pitch, 3));
     RV_TRY(check_params(ctx, p));
     RV_TRY(check_kind(ctx, mem_kind));
     if (!p->clahe && p->ksize == 0) return fail(ctx, RV_ERR_ARG, "nothing to do (no CLAHE, no median)");
@@ -1617,7 +1592,7 @@ int rv_chain_letterbox_f16(rv_ctx *ctx, const uint8_t *in, int n, int h, int w, 
     size_t dpitch = full_pitch;
     if (!full_out && g.scale == 0) {
         dpitch = ((size_t)3 * w + 15) & ~(size_t)15;        // unfused: the resize reads a full-resolution intermediate
-        RV_TRY(ws_acquire(ctx, NPIPE, st));                 // lbfull belongs to workspace set NPIPE
+        RV_TRY(ws_acquire(ctx, ctx->wsync[NPIPE], st));     // lbfull belongs to workspace set NPIPE
         RV_TRY(ensure(ctx, ctx->lbfull, dpitch * h * n));
         dfull = (uint8_t *)ctx->lbfull.p;
     }
@@ -1629,7 +1604,7 @@ int rv_chain_letterbox_f16(rv_ctx *ctx, const uint8_t *in, int n, int h, int w, 
     } else {
         RV_TRY(run_group(ctx, NPIPE, in, in_pitch, in_pitch * h, dfull, dpitch, dpitch * h, n, h, w, p, st, nullptr, nullptr));
         RV_TRY(launch_letterbox(ctx, dfull, dpitch, dpitch * h, n, h, w, g, pad_value, false, out, st));
-        RV_TRY(ws_release(ctx, NPIPE, st));
+        RV_TRY(ws_release(ctx, ctx->wsync[NPIPE], st));
     }
     if (!stream) CK(cudaStreamSynchronize(st));
     return RV_OK;
@@ -1637,14 +1612,14 @@ int rv_chain_letterbox_f16(rv_ctx *ctx, const uint8_t *in, int n, int h, int w, 
 
 int rv_gray_span(rv_ctx *ctx, const uint8_t *in, int n, int h, int w, size_t pitch, int32_t *span, int mem_kind)
 {
-    RV_TRY(check_frames(ctx, in, in, n, h, w, pitch, pitch));
+    RV_TRY(check_frames(ctx, in, in, n, h, w, pitch, pitch, 3));
     if (!span) return fail(ctx, RV_ERR_ARG, "null span");
     if (n == 0) return RV_OK;
     CK(cudaSetDevice(ctx->device));
     const Geo g = make_geo(h, w, 2);
     Staged si;
     RV_TRY(stage_in(ctx, si, in, pitch * h * n, mem_kind));
-    RV_TRY(ws_acquire(ctx, NPIPE, ctx->stream));
+    RV_TRY(ws_acquire(ctx, ctx->wsync[NPIPE], ctx->stream));
     RV_TRY(ensure(ctx, ctx->hist[NPIPE], (size_t)n * 4 * 256 * 4));
     RV_TRY(ensure(ctx, ctx->mm[NPIPE], (size_t)n * 8));
     RV_TRY(launch_hist(ctx, (const uint8_t *)si.dev, pitch, pitch * h, g, RV_SPACE_YCRCB, n, (int32_t *)ctx->hist[NPIPE].p, nullptr,
@@ -1657,18 +1632,9 @@ int rv_gray_span(rv_ctx *ctx, const uint8_t *in, int n, int h, int w, size_t pit
     ctx->wsync[NPIPE].used = true;
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
     if (e != cudaSuccess) { delete[] mm; return fail(ctx, RV_ERR_CUDA, "gray span: %s", cudaGetErrorString(e)); }
-    if (mem_kind == RV_MEM_DEVICE) {
-        int32_t *tmp = new (std::nothrow) int32_t[n];
-        if (!tmp) { delete[] mm; return fail(ctx, RV_ERR_NOMEM, "host alloc"); }
-        for (int i = 0; i < n; ++i) tmp[i] = mm[2 * i + 1] - mm[2 * i];
-        e = cudaMemcpy(span, tmp, (size_t)n * 4, cudaMemcpyHostToDevice);
-        delete[] tmp;
-    } else {
-        for (int i = 0; i < n; ++i) span[i] = mm[2 * i + 1] - mm[2 * i];
-    }
+    const int rc = write_spans(ctx, mm, n, span, mem_kind);
     delete[] mm;
-    if (e != cudaSuccess) return fail(ctx, RV_ERR_CUDA, "gray span copy: %s", cudaGetErrorString(e));
-    return RV_OK;
+    return rc;
 }
 
 }  // extern "C"

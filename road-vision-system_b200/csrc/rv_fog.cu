@@ -36,6 +36,8 @@
 
 #include "rv_internal.h"
 
+using namespace rv;
+
 namespace {
 
 constexpr int MAX_TAPS = 95;                 // largest Gaussian kernel (k2 of the glow at 4K x heavy fog is 47)
@@ -433,19 +435,6 @@ Taps gaussian_taps(int k, double sigma)
     return t;
 }
 
-#define RV_TRY_(call)             \
-    do {                          \
-        int rc_ = (call);         \
-        if (rc_ != RV_OK) return rc_; \
-    } while (0)
-
-#define FCK(call)                                                                                              \
-    do {                                                                                                       \
-        cudaError_t e_ = (call);                                                                               \
-        if (e_ != cudaSuccess)                                                                                 \
-            return rv_internal_fail(ctx, RV_ERR_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
-    } while (0)
-
 void fog_free(FogState *s)
 {
     if (!s) return;
@@ -464,7 +453,7 @@ void fog_destroy_hook(void *p) { fog_free(static_cast<FogState *>(p)); }
 
 int gauss(rv_ctx *ctx, cudaStream_t st, const float *src, float *tmp, float *dst, int h, int w, int nc, int k, double sigma, float lo, float hi)
 {
-    if (k > MAX_TAPS) return rv_internal_fail(ctx, RV_ERR_ARG, "Gaussian kernel %d larger than %d taps", k, MAX_TAPS);
+    if (k > MAX_TAPS) return fail(ctx, RV_ERR_ARG, "Gaussian kernel %d larger than %d taps", k, MAX_TAPS);
     const Taps tp = gaussian_taps(k, sigma);
     dim3 grid((w + 127) / 128, h);
     k_gauss_rows<<<grid, 128, 0, st>>>(src, tmp, h, w, nc, tp);
@@ -481,9 +470,9 @@ int rv_fog_set_geometry(rv_ctx *ctx, int h, int w, const float *depth, const flo
 {
     if (!ctx) return RV_ERR_ARG;
     if (h < 1 || w < 1 || h > 32768 || w > 32768 || !depth || !sky_weight || !vgrad || !xgrad)
-        return rv_internal_fail(ctx, RV_ERR_ARG, "bad fog geometry arguments");
-    FCK(cudaSetDevice(rv_internal_device(ctx)));
-    FCK(cudaDeviceSynchronize());
+        return fail(ctx, RV_ERR_ARG, "bad fog geometry arguments");
+    CK(cudaSetDevice(rv_internal_device(ctx)));
+    CK(cudaDeviceSynchronize());
     fog_free(static_cast<FogState *>(rv_internal_get_fog(ctx)));
     rv_internal_set_fog(ctx, nullptr, nullptr);
     FogState *s = new (std::nothrow) FogState();
@@ -491,19 +480,19 @@ int rv_fog_set_geometry(rv_ctx *ctx, int h, int w, const float *depth, const flo
     rv_internal_set_fog(ctx, s, fog_destroy_hook);
     const size_t npx = (size_t)h * w;
     s->h = h; s->w = w; s->cap_px = npx;
-    FCK(cudaMalloc(&s->depth, npx * 4));
-    FCK(cudaMalloc(&s->sky, npx * 4));
-    FCK(cudaMalloc(&s->vgrad, (size_t)h * 4));
-    FCK(cudaMalloc(&s->xgrad, (size_t)w * 4));
-    for (float *&p : s->f3) FCK(cudaMalloc(&p, npx * 12));
-    for (float *&p : s->p1) FCK(cudaMalloc(&p, npx * 4));
-    for (int i = 0; i < 5; ++i) FCK(cudaMalloc(&s->u8[i], i < 2 ? npx * 3 : npx));
-    FCK(cudaMalloc(&s->ysm, npx));
-    FCK(cudaMalloc(&s->red, 8 * sizeof(double)));
-    FCK(cudaMemcpy(s->depth, depth, npx * 4, cudaMemcpyHostToDevice));
-    FCK(cudaMemcpy(s->sky, sky_weight, npx * 4, cudaMemcpyHostToDevice));
-    FCK(cudaMemcpy(s->vgrad, vgrad, (size_t)h * 4, cudaMemcpyHostToDevice));
-    FCK(cudaMemcpy(s->xgrad, xgrad, (size_t)w * 4, cudaMemcpyHostToDevice));
+    CK(cudaMalloc(&s->depth, npx * 4));
+    CK(cudaMalloc(&s->sky, npx * 4));
+    CK(cudaMalloc(&s->vgrad, (size_t)h * 4));
+    CK(cudaMalloc(&s->xgrad, (size_t)w * 4));
+    for (float *&p : s->f3) CK(cudaMalloc(&p, npx * 12));
+    for (float *&p : s->p1) CK(cudaMalloc(&p, npx * 4));
+    for (int i = 0; i < 5; ++i) CK(cudaMalloc(&s->u8[i], i < 2 ? npx * 3 : npx));
+    CK(cudaMalloc(&s->ysm, npx));
+    CK(cudaMalloc(&s->red, 8 * sizeof(double)));
+    CK(cudaMemcpy(s->depth, depth, npx * 4, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(s->sky, sky_weight, npx * 4, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(s->vgrad, vgrad, (size_t)h * 4, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(s->xgrad, xgrad, (size_t)w * 4, cudaMemcpyHostToDevice));
     return RV_OK;
 }
 
@@ -512,10 +501,10 @@ int rv_fog_u8(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int h, int w, const 
 {
     if (!ctx) return RV_ERR_ARG;
     FogState *s = static_cast<FogState *>(rv_internal_get_fog(ctx));
-    if (!s || s->h != h || s->w != w) return rv_internal_fail(ctx, RV_ERR_ARG, "rv_fog_set_geometry(%d, %d) has not been called", h, w);
-    if (!in || !out || !f || !lattice) return rv_internal_fail(ctx, RV_ERR_ARG, "null pointer");
-    if (f->octaves < 1 || f->octaves > MAX_OCT) return rv_internal_fail(ctx, RV_ERR_ARG, "octaves %d not in [1,%d]", f->octaves, MAX_OCT);
-    FCK(cudaSetDevice(rv_internal_device(ctx)));
+    if (!s || s->h != h || s->w != w) return fail(ctx, RV_ERR_ARG, "rv_fog_set_geometry(%d, %d) has not been called", h, w);
+    if (!in || !out || !f || !lattice) return fail(ctx, RV_ERR_ARG, "null pointer");
+    if (f->octaves < 1 || f->octaves > MAX_OCT) return fail(ctx, RV_ERR_ARG, "octaves %d not in [1,%d]", f->octaves, MAX_OCT);
+    CK(cudaSetDevice(rv_internal_device(ctx)));
     cudaStream_t st = (cudaStream_t)rv_internal_stream(ctx);
     const size_t npx = (size_t)h * w;
     const int TB = 256;
@@ -529,7 +518,7 @@ int rv_fog_u8(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int h, int w, const 
     size_t lat_floats = 0;
     double amp = 1.0, norm = 0.0;
     for (int o = 0; o < L.n; ++o) {
-        if (f->lat_gh[o] < 1 || f->lat_gw[o] < 1) return rv_internal_fail(ctx, RV_ERR_ARG, "bad lattice size");
+        if (f->lat_gh[o] < 1 || f->lat_gw[o] < 1) return fail(ctx, RV_ERR_ARG, "bad lattice size");
         L.gh[o] = f->lat_gh[o]; L.gw[o] = f->lat_gw[o]; L.off[o] = (int)lat_floats; L.amp[o] = amp;
         lat_floats += (size_t)(L.gh[o] + 1) * (L.gw[o] + 1);
         norm += amp;
@@ -537,24 +526,24 @@ int rv_fog_u8(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int h, int w, const 
     }
     L.norm = (float)norm;
     if (s->lat_cap < lat_floats) {
-        if (s->lat) FCK(cudaFree(s->lat));
+        if (s->lat) CK(cudaFree(s->lat));
         s->lat = nullptr; s->lat_cap = 0;
-        FCK(cudaMalloc(&s->lat, lat_floats * 4));
+        CK(cudaMalloc(&s->lat, lat_floats * 4));
         s->lat_cap = lat_floats;
     }
-    FCK(cudaMemcpyAsync(s->lat, lattice, lat_floats * 4, cudaMemcpyHostToDevice, st));
-    FCK(cudaMemcpyAsync(s->u8[0], in, npx * 3, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(s->lat, lattice, lat_floats * 4, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(s->u8[0], in, npx * 3, cudaMemcpyHostToDevice, st));
     const float *dnoise = nullptr;
     if (noise && f->noise_sigma > 0.f) {
-        if (!s->noise) FCK(cudaMalloc(&s->noise, npx * 12));
-        FCK(cudaMemcpyAsync(s->noise, noise, npx * 12, cudaMemcpyHostToDevice, st));
+        if (!s->noise) CK(cudaMalloc(&s->noise, npx * 12));
+        CK(cudaMemcpyAsync(s->noise, noise, npx * 12, cudaMemcpyHostToDevice, st));
         dnoise = s->noise;
     }
     // reductions: min / max bit patterns, sum(A), sum(gray), sum(gray^2)
     {
         int mm[4] = {0x7f7fffff, 0, 0, 0};
-        FCK(cudaMemsetAsync(s->red, 0, 8 * sizeof(double), st));
-        FCK(cudaMemcpyAsync(s->red + 6, mm, sizeof mm, cudaMemcpyHostToDevice, st));
+        CK(cudaMemsetAsync(s->red, 0, 8 * sizeof(double), st));
+        CK(cudaMemcpyAsync(s->red + 6, mm, sizeof mm, cudaMemcpyHostToDevice, st));
     }
     int *mm = reinterpret_cast<int *>(s->red + 6);
     float *base = s->p1[0], *beta = s->p1[1], *t0 = s->p1[2], *t = s->p1[3];
@@ -563,7 +552,7 @@ int rv_fog_u8(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int h, int w, const 
     k_fog_noise<<<g2, b2, 0, st>>>(s->lat, L, h, w, base, mm);
     k_fog_trans<<<gpx, TB, 0, st>>>(base, mm, s->depth, f->base_beta, npx, beta, t0);
     rv_internal_count_launches(ctx, 2);
-    if (beta_out) FCK(cudaMemcpyAsync(beta_out, beta, npx * 4, cudaMemcpyDeviceToHost, st));      // the plane is reused below
+    if (beta_out) CK(cudaMemcpyAsync(beta_out, beta, npx * 4, cudaMemcpyDeviceToHost, st));      // the plane is reused below
     const float cs = (float)(-0.5 / (12.0 * 12.0)), cc = cs;
     if (f->edge_guided) {
         const int R = 8;
@@ -586,23 +575,23 @@ int rv_fog_u8(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int h, int w, const 
     // glow (fog.py:188-198)
     float *gray = s->p1[0], *hard = s->p1[1], *soft = s->p1[4], *tmp1 = s->p1[5];
     float *blur = s->f3[0], *tmp3 = s->f3[3], *glow = s->f3[1];          // A0 and A are free from here on
-    if (airlight_out) FCK(cudaMemcpyAsync(airlight_out, A, npx * 12, cudaMemcpyDeviceToHost, st));
+    if (airlight_out) CK(cudaMemcpyAsync(airlight_out, A, npx * 12, cudaMemcpyDeviceToHost, st));
     k_fog_gray_stats<<<592, TB, 0, st>>>(hazy, npx, gray, s->red + 3);
     k_fog_hard<<<gpx, TB, 0, st>>>(gray, s->red + 3, npx, hard);
     rv_internal_count_launches(ctx, 2);
     {
         // k = int(9 + 20 s) | 1 and k2 = int(max(7, (h + w)(0.003 + 0.01 s))) | 1 come from the host (evaluated there in double)
         const int k = f->glow_k, k2 = f->glow_k2;
-        if (k < 1 || k2 < 1 || !(k & 1) || !(k2 & 1)) return rv_internal_fail(ctx, RV_ERR_ARG, "bad glow kernel sizes %d, %d", k, k2);
-        RV_TRY_(gauss(ctx, st, hard, tmp1, soft, h, w, 1, k, k * 0.35, 0.f, 1.f));
-        RV_TRY_(gauss(ctx, st, hazy, tmp3, blur, h, w, 3, k2, k2 * 0.25, -3.0e38f, 3.0e38f));
+        if (k < 1 || k2 < 1 || !(k & 1) || !(k2 & 1)) return fail(ctx, RV_ERR_ARG, "bad glow kernel sizes %d, %d", k, k2);
+        RV_TRY(gauss(ctx, st, hard, tmp1, soft, h, w, 1, k, k * 0.35, 0.f, 1.f));
+        RV_TRY(gauss(ctx, st, hazy, tmp3, blur, h, w, 3, k2, k2 * 0.25, -3.0e38f, 3.0e38f));
     }
     k_fog_glow<<<gpx, TB, 0, st>>>(hazy, blur, soft, f->glow, npx, glow);
     rv_internal_count_launches(ctx, 1);
 
     // depth blur in three bands (fog.py:201-221): every band blurs the glow image, not the running result
     float *outp = s->f3[2];
-    FCK(cudaMemcpyAsync(outp, glow, npx * 12, cudaMemcpyDeviceToDevice, st));
+    CK(cudaMemcpyAsync(outp, glow, npx * 12, cudaMemcpyDeviceToDevice, st));
     {
         const float edges[4] = {0.0f, 0.33f, 0.66f, 1.0f};
         for (int b = 0; b < 3; ++b) {
@@ -610,8 +599,8 @@ int rv_fog_u8(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int h, int w, const 
             if (rad <= 1) continue;
             float *mask = s->p1[0], *m = s->p1[1];
             k_fog_band_mask<<<gpx, TB, 0, st>>>(s->depth, edges[b], edges[b + 1], npx, mask);
-            RV_TRY_(gauss(ctx, st, glow, tmp3, blur, h, w, 3, rad, rad * 0.5, -3.0e38f, 3.0e38f));
-            RV_TRY_(gauss(ctx, st, mask, tmp1, m, h, w, 1, rad | 1, rad * 0.5, -3.0e38f, 3.0e38f));
+            RV_TRY(gauss(ctx, st, glow, tmp3, blur, h, w, 3, rad, rad * 0.5, -3.0e38f, 3.0e38f));
+            RV_TRY(gauss(ctx, st, mask, tmp1, m, h, w, 1, rad | 1, rad * 0.5, -3.0e38f, 3.0e38f));
             k_fog_band_mix<<<gpx, TB, 0, st>>>(outp, blur, m, npx);
             rv_internal_count_launches(ctx, 2);
         }
@@ -620,7 +609,7 @@ int rv_fog_u8(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int h, int w, const 
     k_fog_to_ycc<<<gpx, TB, 0, st>>>(outp, npx, s->u8[2], s->u8[3], s->u8[4]);
     {
         const int d = f->fade_d;                   // int(5 + 20 a) | 1, from the host
-        if (d < 1 || d > 63) return rv_internal_fail(ctx, RV_ERR_ARG, "bad fade kernel size %d", d);
+        if (d < 1 || d > 63) return fail(ctx, RV_ERR_ARG, "bad fade kernel size %d", d);
         const int R = d / 2;
         const double sg = (double)f->fade_sigma;   // 25 + 50 a
         const float c2 = (float)(-0.5 / (sg * sg));
@@ -632,10 +621,10 @@ int rv_fog_u8(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int h, int w, const 
     fin.gamma = f->gamma; fin.noise_sigma = f->noise_sigma; fin.seed = f->noise_seed;
     k_fog_finish<<<gpx, TB, 0, st>>>(s->u8[2], s->ysm, s->u8[3], s->u8[4], fin, dnoise, npx, s->u8[1]);
     rv_internal_count_launches(ctx, 3);
-    FCK(cudaGetLastError());
-    FCK(cudaMemcpyAsync(out, s->u8[1], npx * 3, cudaMemcpyDeviceToHost, st));
-    if (t_out) FCK(cudaMemcpyAsync(t_out, t, npx * 4, cudaMemcpyDeviceToHost, st));
-    FCK(cudaStreamSynchronize(st));
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(out, s->u8[1], npx * 3, cudaMemcpyDeviceToHost, st));
+    if (t_out) CK(cudaMemcpyAsync(t_out, t, npx * 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
     return RV_OK;
 }
 

@@ -24,31 +24,28 @@
  *   k_u16_median<K>   k = 3 / 5 with the generated selection networks of rv_median_net.h on u16x2 lanes (two output rows), in
  *                     their ALU form only (__vminu2 / __vmaxu2): the FMA-pipe form of the 8-bit kernel relies on values below
  *                     0x400 and is wrong for 16-bit data
- *   k_u16_gray_minmax, k_u16_gate_flags, k_u16_gate_copy   the low-contrast gate
+ *   k_u16_gray_minmax, k_u16_gate_copy   the low-contrast gate; its decision is the 8-bit path's k_gate_flags (launch_gate_flags)
+ *
+ * The host side is the 8-bit path's (rv_internal.h): argument checks, CLAHE geometry, the gate threshold, workspaces and their
+ * ordering between streams.
  */
 #include "../../include/rv_b200.h"
 
 #include <cuda_runtime.h>
-#include <math.h>
-#include <stdio.h>
-#include <string.h>
 
 #include <algorithm>
-#include <new>
 
 #include "rv_common.cuh"        // Geo, reflect101
 #include "rv_internal.h"
 #include "rv_median_net.h"      // RV_CEX is not overridden here: every compare-exchange is __vminu2 / __vmaxu2
 
-namespace {
+using namespace rv;
 
-using rv::Geo;
-using rv::reflect101;
+namespace {
 
 constexpr int U16_MAX_GRID = 64;            // a dense grid-64 LUT set is 512 MB per frame
 constexpr int HALF_BINS = 32768;
 constexpr int HL_THREADS = 1024;
-constexpr int MAX_FRAMES_PER_LAUNCH = 32768;
 constexpr size_t LUT_GROUP_BYTES = (size_t)48 << 20;    // LUTs of one frame group: well inside the 126 MB L2 of a B200
 
 __device__ __forceinline__ int d14(int x) { return (x + 8192) >> 14; }
@@ -265,12 +262,6 @@ __global__ void __launch_bounds__(256) k_u16_gray_minmax(const uint16_t *__restr
     }
 }
 
-__global__ void k_u16_gate_flags(const int32_t *__restrict__ mm, int n, int thresh, int32_t *__restrict__ flags)
-{
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) flags[i] = (mm[2 * i + 1] - mm[2 * i] < thresh) ? 1 : 0;
-}
-
 // frames the gate skipped are passed through unchanged
 __global__ void k_u16_gate_copy(const uint8_t *__restrict__ src, size_t spitch, size_t sfstride, uint8_t *__restrict__ dst, size_t dpitch,
                                 size_t dfstride, int H, int rowbytes, const int32_t *__restrict__ flags)
@@ -285,152 +276,16 @@ __global__ void k_u16_gate_copy(const uint8_t *__restrict__ src, size_t spitch, 
 }
 
 // ------------------------------------------------------------------------------------------------ host side
-struct DBuf {
-    void *p = nullptr;
-    size_t cap = 0;
-};
-
-// Workspaces of the 16-bit path of one context.  They are used on whichever stream a call runs on; an event recorded after
-// the last use orders the next user on a different stream behind it (as the 8-bit workspace sets are ordered).
-struct U16State {
-    DBuf lut, mid, din, dout, mm, flags;
-    int32_t *hflags = nullptr;                  // page-locked copy of the gate decisions
-    size_t hflags_cap = 0;
-    cudaEvent_t ev = nullptr;
-    cudaStream_t last = nullptr;
-    bool used = false;
-    bool attr_set = false;
-};
-
-void destroy_state(void *p)
-{
-    U16State *s = (U16State *)p;
-    DBuf *bufs[] = {&s->lut, &s->mid, &s->din, &s->dout, &s->mm, &s->flags};
-    for (DBuf *b : bufs)
-        if (b->p) cudaFree(b->p);
-    if (s->hflags) cudaFreeHost(s->hflags);
-    if (s->ev) cudaEventDestroy(s->ev);
-    delete s;
-}
-
-#define FAIL(code, ...) rv_internal_fail(ctx, code, __VA_ARGS__)
-#define CK(call)                                                                                                          \
-    do {                                                                                                                  \
-        cudaError_t e_ = (call);                                                                                          \
-        if (e_ != cudaSuccess) return FAIL(RV_ERR_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
-    } while (0)
-#define RV_TRY(call)                  \
-    do {                              \
-        int rc_ = (call);             \
-        if (rc_ != RV_OK) return rc_; \
-    } while (0)
-
-int get_state(rv_ctx *ctx, U16State **out)
-{
-    U16State *s = (U16State *)rv_internal_get_u16(ctx);
-    if (!s) {
-        s = new (std::nothrow) U16State();
-        if (!s) return FAIL(RV_ERR_NOMEM, "host alloc");
-        if (cudaEventCreateWithFlags(&s->ev, cudaEventDisableTiming) != cudaSuccess) {
-            delete s;
-            return FAIL(RV_ERR_CUDA, "cudaEventCreate failed");
-        }
-        rv_internal_set_u16(ctx, s, destroy_state);
-    }
-    if (!s->attr_set) {
-        CK(cudaFuncSetAttribute(k_u16_hist_lut, cudaFuncAttributeMaxDynamicSharedMemorySize, (HALF_BINS + 64) * 4));
-        s->attr_set = true;
-    }
-    *out = s;
-    return RV_OK;
-}
-
-int ensure(rv_ctx *ctx, DBuf &b, size_t bytes)
-{
-    if (b.cap >= bytes) return RV_OK;
-    if (b.p) CK(cudaFree(b.p));
-    b.p = nullptr;
-    b.cap = 0;
-    const size_t want = (bytes + 255) & ~(size_t)255;
-    const cudaError_t e = cudaMalloc(&b.p, want);
-    if (e != cudaSuccess) return FAIL(RV_ERR_NOMEM, "cudaMalloc(%zu) failed: %s", want, cudaGetErrorString(e));
-    b.cap = want;
-    return RV_OK;
-}
-
-int acquire(rv_ctx *ctx, U16State *s, cudaStream_t st)
-{
-    if (s->used && s->last != st) CK(cudaStreamWaitEvent(st, s->ev, 0));
-    return RV_OK;
-}
-
-int release(rv_ctx *ctx, U16State *s, cudaStream_t st)
-{
-    CK(cudaEventRecord(s->ev, st));
-    s->last = st;
-    s->used = true;
-    return RV_OK;
-}
-
-// clahe.cpp geometry (A.3): both dimensions are padded when either is not divisible by the grid
-Geo make_geo(int h, int w, int grid)
-{
-    Geo g;
-    g.H = h; g.W = w; g.grid = grid;
-    int eh = h, ew = w;
-    if (w % grid != 0 || h % grid != 0) {
-        ew = w + (grid - w % grid);
-        eh = h + (grid - h % grid);
-    }
-    g.tw = ew / grid;
-    g.th = eh / grid;
-    g.inv_tw = 1.0f / (float)g.tw;
-    g.inv_th = 1.0f / (float)g.th;
-    return g;
-}
-
-// pipeline.py:24-30 compares an integer span with a Python float: span < t  <=>  span < ceil(t) for integer spans
-int gate_thresh_int(double t)
-{
-    if (!(t == t)) return -1;
-    const double c = ceil(t);
-    if (c > 65536.0) return 65536;
-    if (c < -1.0) return -1;
-    return (int)c;
-}
-
-int check_frames(rv_ctx *ctx, const void *in, const void *out, int n, int h, int w, size_t ipitch, size_t opitch)
-{
-    if (!ctx) return RV_ERR_ARG;
-    if (!in || !out) return FAIL(RV_ERR_ARG, "null frame pointer");
-    if (n < 0 || h < 1 || w < 1) return FAIL(RV_ERR_ARG, "bad frame shape n=%d h=%d w=%d", n, h, w);
-    if (h > 32768 || w > 32768) return FAIL(RV_ERR_ARG, "frame too large (%dx%d)", w, h);
-    if (ipitch < (size_t)6 * w || opitch < (size_t)6 * w) return FAIL(RV_ERR_ARG, "pitch smaller than 6*w");
-    if ((ipitch | opitch) & 1) return FAIL(RV_ERR_ARG, "16-bit frames need even pitches");
-    if (((uintptr_t)in | (uintptr_t)out) & 1) return FAIL(RV_ERR_ARG, "16-bit frames need 2-byte aligned buffers");
-    if (in != out && n > 0) {
-        const uintptr_t a0 = (uintptr_t)in, a1 = a0 + (size_t)n * h * ipitch, b0 = (uintptr_t)out, b1 = b0 + (size_t)n * h * opitch;
-        if (a0 < b1 && b0 < a1) return FAIL(RV_ERR_ARG, "input and output ranges overlap");
-    }
-    return RV_OK;
-}
-
-int check_kind(rv_ctx *ctx, int kind)
-{
-    if (kind != RV_MEM_HOST && kind != RV_MEM_HOST_PINNED && kind != RV_MEM_DEVICE) return FAIL(RV_ERR_ARG, "bad memory kind %d", kind);
-    return RV_OK;
-}
-
 int check_params(rv_ctx *ctx, const rv_params *p)
 {
-    if (!p) return FAIL(RV_ERR_ARG, "null params");
-    if (p->space == RV_SPACE_LAB) return FAIL(RV_ERR_ARG, "LAB has no 16-bit path (cv2.cvtColor BGR2LAB rejects CV_16U)");
-    if (p->space != RV_SPACE_YCRCB) return FAIL(RV_ERR_ARG, "bad space %d", p->space);
+    if (!p) return fail(ctx, RV_ERR_ARG, "null params");
+    if (p->space == RV_SPACE_LAB) return fail(ctx, RV_ERR_ARG, "LAB has no 16-bit path (cv2.cvtColor BGR2LAB rejects CV_16U)");
+    if (p->space != RV_SPACE_YCRCB) return fail(ctx, RV_ERR_ARG, "bad space %d", p->space);
     if (p->clahe && (p->grid < 2 || p->grid > U16_MAX_GRID))
-        return FAIL(RV_ERR_ARG, "tile grid %d out of range [2,%d] for 16-bit frames", p->grid, U16_MAX_GRID);
+        return fail(ctx, RV_ERR_ARG, "tile grid %d out of range [2,%d] for 16-bit frames", p->grid, U16_MAX_GRID);
     if (!(p->ksize == 0 || p->ksize == 3 || p->ksize == 5))
-        return FAIL(RV_ERR_ARG, "ksize %d not in {0,3,5} for 16-bit frames (cv2.medianBlur has no 16-bit k > 5)", p->ksize);
-    if (!p->clahe && p->ksize == 0) return FAIL(RV_ERR_ARG, "nothing to do (no CLAHE, no median)");
+        return fail(ctx, RV_ERR_ARG, "ksize %d not in {0,3,5} for 16-bit frames (cv2.medianBlur has no 16-bit k > 5)", p->ksize);
+    if (!p->clahe && p->ksize == 0) return fail(ctx, RV_ERR_ARG, "nothing to do (no CLAHE, no median)");
     return RV_OK;
 }
 
@@ -464,10 +319,10 @@ int launch_median(rv_ctx *ctx, int k, const uint16_t *src, size_t sp, size_t sfs
     return RV_OK;
 }
 
-int launch_gray(rv_ctx *ctx, U16State *s, const uint16_t *src, size_t sp, size_t sfs, int n, int h, int w, cudaStream_t st)
+int launch_gray(rv_ctx *ctx, U16Ws &s, const uint16_t *src, size_t sp, size_t sfs, int n, int h, int w, cudaStream_t st)
 {
-    RV_TRY(ensure(ctx, s->mm, (size_t)n * 8));
-    int32_t *mm = (int32_t *)s->mm.p;
+    RV_TRY(ensure(ctx, s.mm, (size_t)n * 8));
+    int32_t *mm = (int32_t *)s.mm.p;
     k_u16_init_minmax<<<(n + 127) / 128, 128, 0, st>>>(mm, n);
     for (int f0 = 0; f0 < n; f0 += MAX_FRAMES_PER_LAUNCH) {
         const int nf = std::min(MAX_FRAMES_PER_LAUNCH, n - f0);
@@ -480,35 +335,38 @@ int launch_gray(rv_ctx *ctx, U16State *s, const uint16_t *src, size_t sp, size_t
 }
 
 // The chain on one group of frames that are on the device.  Returns the device gate flags (or nullptr) through flags_out.
-int run_group(rv_ctx *ctx, U16State *s, const uint16_t *din, size_t ip, size_t ifs, uint16_t *dout, size_t op, size_t ofs, int n,
+int run_group(rv_ctx *ctx, U16Ws &s, const uint16_t *din, size_t ip, size_t ifs, uint16_t *dout, size_t op, size_t ofs, int n,
               int h, int w, const rv_params *p, cudaStream_t st, const int32_t **flags_out)
 {
     const int32_t *flags = nullptr;
     if (p->gate_enable) {
         RV_TRY(launch_gray(ctx, s, din, ip, ifs, n, h, w, st));
-        RV_TRY(ensure(ctx, s->flags, (size_t)n * 4));
-        k_u16_gate_flags<<<(n + 127) / 128, 128, 0, st>>>((const int32_t *)s->mm.p, n, gate_thresh_int(p->gate_thresh), (int32_t *)s->flags.p);
-        rv_internal_count_launches(ctx, 1);
-        flags = (const int32_t *)s->flags.p;
+        RV_TRY(ensure(ctx, s.flags, (size_t)n * 4));
+        launch_gate_flags(ctx, (const int32_t *)s.mm.p, n, p->gate_thresh, (int32_t *)s.flags.p, st);
+        flags = (const int32_t *)s.flags.p;
     }
     if (p->clahe) {
         const Geo g = make_geo(h, w, p->grid);
         const int tiles = g.grid * g.grid;
-        RV_TRY(ensure(ctx, s->lut, (size_t)n * tiles * 65536 * 2));
+        RV_TRY(ensure(ctx, s.lut, (size_t)n * tiles * 65536 * 2));
+        if (!s.attr_set) {
+            CK(cudaFuncSetAttribute(k_u16_hist_lut, cudaFuncAttributeMaxDynamicSharedMemorySize, (HALF_BINS + 64) * 4));
+            s.attr_set = true;
+        }
         // clahe.cpp: clipLimit = max(int(clip * tileArea / histSize), 1) when clip > 0
         const int area = g.tw * g.th;
         int clip = 0;
         if (p->clip_limit > 0.0) clip = std::max((int)(p->clip_limit * (double)area / 65536.0), 1);
         const float lut_scale = 65535.0f / (float)area;
-        uint16_t *lut = (uint16_t *)s->lut.p;
+        uint16_t *lut = (uint16_t *)s.lut.p;
         k_u16_hist_lut<<<dim3(tiles, n), HL_THREADS, (HALF_BINS + 64) * 4, st>>>(din, ip, ifs, g, clip, lut_scale, lut, flags);
         uint16_t *ao = dout;
         size_t aop = op, aofs = ofs;
         if (p->ksize) {
             aop = (size_t)6 * w;
             aofs = aop * h;
-            RV_TRY(ensure(ctx, s->mid, aofs * n));
-            ao = (uint16_t *)s->mid.p;
+            RV_TRY(ensure(ctx, s.mid, aofs * n));
+            ao = (uint16_t *)s.mid.p;
         }
         k_u16_apply<<<dim3((w + 255) / 256, h, n), 256, 0, st>>>(din, ip, ifs, ao, aop, aofs, g, lut, flags);
         rv_internal_count_launches(ctx, 2);
@@ -527,14 +385,14 @@ int run_group(rv_ctx *ctx, U16State *s, const uint16_t *din, size_t ip, size_t i
     return RV_OK;
 }
 
-int host_flags(rv_ctx *ctx, U16State *s, int n)
+int host_flags(rv_ctx *ctx, U16Ws &s, int n)
 {
-    if (s->hflags_cap >= (size_t)n) return RV_OK;
-    if (s->hflags) CK(cudaFreeHost(s->hflags));
-    s->hflags = nullptr;
-    s->hflags_cap = 0;
-    CK(cudaHostAlloc((void **)&s->hflags, (size_t)std::max(n, 64) * 4, cudaHostAllocDefault));
-    s->hflags_cap = (size_t)std::max(n, 64);
+    if (s.hflags_cap >= (size_t)n) return RV_OK;
+    if (s.hflags) CK(cudaFreeHost(s.hflags));
+    s.hflags = nullptr;
+    s.hflags_cap = 0;
+    CK(cudaHostAlloc((void **)&s.hflags, (size_t)std::max(n, 64) * 4, cudaHostAllocDefault));
+    s.hflags_cap = (size_t)std::max(n, 64);
     return RV_OK;
 }
 
@@ -545,17 +403,16 @@ extern "C" {
 int rv_chain_u16(rv_ctx *ctx, const uint16_t *in, uint16_t *out, int n, int h, int w, size_t in_pitch, size_t out_pitch,
                  const rv_params *p, int mem_kind, int32_t *processed, void *stream)
 {
-    RV_TRY(check_frames(ctx, in, out, n, h, w, in_pitch, out_pitch));
+    RV_TRY(check_frames(ctx, in, out, n, h, w, in_pitch, out_pitch, 6));
     RV_TRY(check_params(ctx, p));
     RV_TRY(check_kind(ctx, mem_kind));
-    if (in == out) return FAIL(RV_ERR_ARG, "in-place operation is not supported (tiles read their neighbours' halo)");
+    if (in == out) return fail(ctx, RV_ERR_ARG, "in-place operation is not supported (tiles read their neighbours' halo)");
     if (n == 0) return RV_OK;
     CK(cudaSetDevice(rv_internal_device(ctx)));
-    U16State *s = nullptr;
-    RV_TRY(get_state(ctx, &s));
+    U16Ws &s = rv_internal_u16(ctx);
     const bool dev = mem_kind == RV_MEM_DEVICE;
     cudaStream_t st = (dev && stream) ? (cudaStream_t)stream : (cudaStream_t)rv_internal_stream(ctx);
-    RV_TRY(acquire(ctx, s, st));
+    RV_TRY(ws_acquire(ctx, s.sync, st));
     if (processed && p->gate_enable) RV_TRY(host_flags(ctx, s, n));
     const long G = group_frames(p, h, w);
     const size_t fb = (size_t)6 * w * h;
@@ -569,39 +426,38 @@ int rv_chain_u16(rv_ctx *ctx, const uint16_t *in, uint16_t *out, int n, int h, i
             gout = (uint16_t *)((uint8_t *)out + (size_t)f0 * h * out_pitch);
         } else {
             // host frames: one group at a time through packed device buffers (allocated once per shape, then reused)
-            RV_TRY(ensure(ctx, s->din, fb * g));
-            RV_TRY(ensure(ctx, s->dout, fb * g));
-            CK(cudaMemcpy2DAsync(s->din.p, (size_t)6 * w, (const uint8_t *)in + (size_t)f0 * h * in_pitch, in_pitch, (size_t)6 * w,
+            RV_TRY(ensure(ctx, s.din, fb * g));
+            RV_TRY(ensure(ctx, s.dout, fb * g));
+            CK(cudaMemcpy2DAsync(s.din.p, (size_t)6 * w, (const uint8_t *)in + (size_t)f0 * h * in_pitch, in_pitch, (size_t)6 * w,
                                  (size_t)h * g, cudaMemcpyHostToDevice, st));
-            gin = (const uint16_t *)s->din.p;
-            gout = (uint16_t *)s->dout.p;
+            gin = (const uint16_t *)s.din.p;
+            gout = (uint16_t *)s.dout.p;
             ip = op = (size_t)6 * w;
         }
         const int32_t *flags = nullptr;
         RV_TRY(run_group(ctx, s, gin, ip, ip * h, gout, op, op * h, g, h, w, p, st, &flags));
         if (!dev)
-            CK(cudaMemcpy2DAsync((uint8_t *)out + (size_t)f0 * h * out_pitch, out_pitch, s->dout.p, (size_t)6 * w, (size_t)6 * w,
+            CK(cudaMemcpy2DAsync((uint8_t *)out + (size_t)f0 * h * out_pitch, out_pitch, s.dout.p, (size_t)6 * w, (size_t)6 * w,
                                  (size_t)h * g, cudaMemcpyDeviceToHost, st));
-        if (processed && flags) CK(cudaMemcpyAsync(s->hflags + f0, flags, (size_t)g * 4, cudaMemcpyDeviceToHost, st));
+        if (processed && flags) CK(cudaMemcpyAsync(s.hflags + f0, flags, (size_t)g * 4, cudaMemcpyDeviceToHost, st));
     }
-    RV_TRY(release(ctx, s, st));
+    RV_TRY(ws_release(ctx, s.sync, st));
     if (!dev || !stream || (processed && p->gate_enable)) CK(cudaStreamSynchronize(st));
     if (processed)
-        for (int i = 0; i < n; ++i) processed[i] = p->gate_enable ? s->hflags[i] : 1;
+        for (int i = 0; i < n; ++i) processed[i] = p->gate_enable ? s.hflags[i] : 1;
     return RV_OK;
 }
 
 int rv_gray_span_u16(rv_ctx *ctx, const uint16_t *in, int n, int h, int w, size_t pitch, int32_t *span, int mem_kind)
 {
-    RV_TRY(check_frames(ctx, in, in, n, h, w, pitch, pitch));
+    RV_TRY(check_frames(ctx, in, in, n, h, w, pitch, pitch, 6));
     RV_TRY(check_kind(ctx, mem_kind));
-    if (!span) return FAIL(RV_ERR_ARG, "null span");
+    if (!span) return fail(ctx, RV_ERR_ARG, "null span");
     if (n == 0) return RV_OK;
     CK(cudaSetDevice(rv_internal_device(ctx)));
-    U16State *s = nullptr;
-    RV_TRY(get_state(ctx, &s));
+    U16Ws &s = rv_internal_u16(ctx);
     cudaStream_t st = (cudaStream_t)rv_internal_stream(ctx);
-    RV_TRY(acquire(ctx, s, st));
+    RV_TRY(ws_acquire(ctx, s.sync, st));
     RV_TRY(host_flags(ctx, s, 2 * n));
     const size_t fb = (size_t)6 * w * h;
     const int G = (int)std::max<long>(1, std::min<long>(256, (long)(((size_t)1 << 30) / fb)));
@@ -610,25 +466,17 @@ int rv_gray_span_u16(rv_ctx *ctx, const uint16_t *in, int n, int h, int w, size_
         const uint16_t *gin = (const uint16_t *)((const uint8_t *)in + (size_t)f0 * h * pitch);
         size_t ip = pitch;
         if (mem_kind != RV_MEM_DEVICE) {
-            RV_TRY(ensure(ctx, s->din, fb * g));
-            CK(cudaMemcpy2DAsync(s->din.p, (size_t)6 * w, gin, pitch, (size_t)6 * w, (size_t)h * g, cudaMemcpyHostToDevice, st));
-            gin = (const uint16_t *)s->din.p;
+            RV_TRY(ensure(ctx, s.din, fb * g));
+            CK(cudaMemcpy2DAsync(s.din.p, (size_t)6 * w, gin, pitch, (size_t)6 * w, (size_t)h * g, cudaMemcpyHostToDevice, st));
+            gin = (const uint16_t *)s.din.p;
             ip = (size_t)6 * w;
         }
         RV_TRY(launch_gray(ctx, s, gin, ip, ip * h, g, h, w, st));
-        CK(cudaMemcpyAsync(s->hflags + 2 * (size_t)f0, s->mm.p, (size_t)g * 8, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(s.hflags + 2 * (size_t)f0, s.mm.p, (size_t)g * 8, cudaMemcpyDeviceToHost, st));
     }
-    RV_TRY(release(ctx, s, st));
+    RV_TRY(ws_release(ctx, s.sync, st));
     CK(cudaStreamSynchronize(st));
-    int32_t *tmp = mem_kind == RV_MEM_DEVICE ? new (std::nothrow) int32_t[n] : span;
-    if (!tmp) return FAIL(RV_ERR_NOMEM, "host alloc");
-    for (int i = 0; i < n; ++i) tmp[i] = s->hflags[2 * i + 1] - s->hflags[2 * i];
-    if (mem_kind == RV_MEM_DEVICE) {
-        const cudaError_t e = cudaMemcpy(span, tmp, (size_t)n * 4, cudaMemcpyHostToDevice);
-        delete[] tmp;
-        if (e != cudaSuccess) return FAIL(RV_ERR_CUDA, "gray span copy: %s", cudaGetErrorString(e));
-    }
-    return RV_OK;
+    return write_spans(ctx, s.hflags, n, span, mem_kind);
 }
 
 }  // extern "C"
