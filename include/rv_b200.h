@@ -19,6 +19,9 @@
  *                      MedianDerain.__call__ (pipeline.py:32-45, clahe_dehaze.py:13-32, median_derain.py:10-14) when the
  *                      reference is handed a 16-bit frame, which it passes to cv2's CV_16U path unchanged
  *   rv_gray_span_u16   PreprocessPipeline._low_contrast on a 16-bit frame   pipeline.py:24-30
+ *   rv_chain_ex        rv_chain_u8 / rv_chain_u16 for 1-, 3- and 4-channel frames (gray; BGR; BGRA / BGRx) at either depth, as
+ *                      cv2 treats the arrays the reference hands it unchanged
+ *   rv_gray_span_ex    rv_gray_span / rv_gray_span_u16 for 3- and 4-channel frames
  *   rv_submit/rv_wait  (new) batched multi-frame entry fed from pinned host buffers; no reference
  *                      counterpart (the reference loop is one frame in flight, main_preview.py:88-142)
  *   rv_submit_io       (new) the same with every end of the job placed independently: what src/io_video/capture.py:18-21
@@ -244,6 +247,23 @@ int rv_chain_u16(rv_ctx *ctx, const uint16_t *in, uint16_t *out, int n, int h, i
                  const rv_params *p, int mem_kind, int32_t *processed, void *stream);
 /* span: n ints = max(gray) - min(gray) per 16-bit frame (synchronous) */
 int rv_gray_span_u16(rv_ctx *ctx, const uint16_t *in, int n, int h, int w, size_t pitch, int32_t *span, int mem_kind);
+
+/* ---- 1-, 3- and 4-channel frames at 8 and 16 bits: gray (monochrome, NIR and thermal cameras, IMREAD_GRAYSCALE), BGR, and BGRA / BGRx
+ * (IMREAD_UNCHANGED on PNGs with alpha, video decoder and converter surfaces), as cv2 computes on them (arithmetic in csrc/rv_channels.cu):
+ *   - CLAHE reads B, G, R and returns 3 channels (cv2.cvtColor ignores alpha and drops it): output channels are 3 when p->clahe,
+ *     else `channels`; the median filters every channel on its own, alpha included; the gate's gray ignores alpha.
+ *   - channels == 3 is exactly rv_chain_u8 (bits 8) / rv_chain_u16 (bits 16), launch for launch.
+ *   - pitches are in bytes: in_pitch >= channels * w * bits / 8, out_pitch >= out_channels * w * bits / 8; 16-bit frames need even
+ *     pitches and 2-byte aligned buffers; the rules of rv_chain_u8 / rv_chain_u16 apply otherwise (LAB and ksize 7 / 9 only at 8 bits).
+ *   - RV_ERR_ARG: bits not in {8, 16}, channels not in {1, 3, 4}, CLAHE or the gate on one channel (cv2.cvtColor rejects it), and the gate
+ *     with CLAHE on 4 channels without `processed` -- those frames it skips are left unwritten in `out` (their result would have 4
+ *     channels, not 3).  A median-only pass copies skipped frames through.
+ *   - host memory goes group by group through device buffers (synchronous); RV_MEM_DEVICE with a `stream` is asynchronous on it unless
+ *     `processed` is asked for together with the gate. */
+int rv_chain_ex(rv_ctx *ctx, const void *in, void *out, int n, int h, int w, size_t in_pitch, size_t out_pitch, int bits, int channels,
+                const rv_params *p, int mem_kind, int32_t *processed, void *stream);
+/* span: n ints = max(gray) - min(gray) per 3- or 4-channel frame (synchronous; one channel -> RV_ERR_ARG) */
+int rv_gray_span_ex(rv_ctx *ctx, const void *in, int n, int h, int w, size_t pitch, int bits, int channels, int32_t *span, int mem_kind);
 
 #ifdef __cplusplus
 }

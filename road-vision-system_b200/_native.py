@@ -209,6 +209,9 @@ EXPORTS = {
     "rv_chain_u16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t,
                                C.POINTER(Params), C.c_int, _i32p, C.c_void_p]),
     "rv_gray_span_u16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_int]),
+    "rv_chain_ex": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_int, C.c_int,
+                              C.POINTER(Params), C.c_int, _i32p, C.c_void_p]),
+    "rv_gray_span_ex": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_int, C.c_int, C.c_void_p, C.c_int]),
 }
 
 
@@ -233,16 +236,18 @@ def load_library():
 
 _U8 = (np.dtype(np.uint8),)
 _U8_U16 = (np.dtype(np.uint8), np.dtype(np.uint16))
+CHANNELS = (1, 3, 4)        # gray, BGR, BGRA / BGRx
 
 
-def _check_frames(frames, dtypes=_U8):
-    """(N,H,W,3) BGR frames of one of `dtypes`."""
+def _check_frames(frames, dtypes=_U8, channels=(3,)):
+    """(N,H,W,C) frames of one of `dtypes`, C in `channels` (BGR only by default)."""
     if not isinstance(frames, np.ndarray):
         raise TypeError("frames must be a numpy.ndarray")
     if frames.dtype not in dtypes:
         raise ValueError(f"{' or '.join(d.name for d in dtypes)} BGR frames expected, got dtype {frames.dtype}")
-    if frames.ndim != 4 or frames.shape[3] != 3:
-        raise ValueError(f"(N,H,W,3) {frames.dtype} expected, got shape {frames.shape}")
+    if frames.ndim != 4 or frames.shape[3] not in channels:
+        want = "3" if channels == (3,) else "C" + f" with C in {channels}"
+        raise ValueError(f"(N,H,W,{want}) {frames.dtype} expected, got shape {frames.shape}")
     if frames.shape[1] < 1 or frames.shape[2] < 1:
         raise ValueError("empty frame")
 
@@ -262,6 +267,21 @@ def check_u16_params(params):
                          "65,536-entry LUT)")
     if not params.clahe and params.ksize == 0:
         raise ValueError("nothing to do (no CLAHE, no median)")
+
+
+def check_frame_params(params, dtype, channels):
+    """What cv2 rejects for a pass over (..., channels) frames of `dtype` raises ValueError here, before the GPU: the 16-bit limits
+    (check_u16_params), CLAHE and the low-contrast gate on a single channel (cv2.cvtColor has no BGR2YCrCb / BGR2LAB / BGR2GRAY for
+    one channel).  Returns the channel count of the result: 3 after CLAHE (which drops alpha, as cv2.cvtColor does), else `channels`."""
+    if np.dtype(dtype) == np.uint16:
+        check_u16_params(params)
+    if channels not in CHANNELS:
+        raise ValueError(f"frames with {channels} channels are not supported (1, 3 or 4)")
+    if channels == 1 and params.clahe:
+        raise ValueError("CLAHEDehaze needs BGR or BGRA frames: cv2.cvtColor BGR2YCrCb / BGR2LAB reject single-channel input")
+    if channels == 1 and params.gate_enable:
+        raise ValueError("the low-contrast gate needs BGR or BGRA frames: cv2.cvtColor BGR2GRAY rejects single-channel input")
+    return 3 if params.clahe else channels
 
 
 class _Lease(np.ndarray):
@@ -388,26 +408,33 @@ class Context:
 
     # -- the chain -----------------------------------------------------------------------
     def chain(self, frames, params, out=None, processed=None):
-        """rv_chain_u8 over host frames (N,H,W,3) uint8, rv_chain_u16 over uint16 ones; returns a new (or `out`) array."""
-        _check_frames(frames, _U8_U16)
-        if frames.dtype == np.uint8:
-            fn, bpp = self._lib.rv_chain_u8, 3
-        else:
+        """rv_chain_u8 over host frames (N,H,W,3) uint8, rv_chain_u16 over uint16 ones, rv_chain_ex over (N,H,W,1) gray and
+        (N,H,W,4) BGRA frames of either dtype; returns a new (or `out`) array, with 3 channels after CLAHE (cv2 drops alpha)."""
+        _check_frames(frames, _U8_U16, CHANNELS)
+        n, h, w, c = frames.shape
+        bits = 8 * frames.dtype.itemsize
+        if c == 3 and bits == 8:
+            fn = self._lib.rv_chain_u8
+        elif c == 3:
             check_u16_params(params)
-            fn, bpp = self._lib.rv_chain_u16, 6
+            fn = self._lib.rv_chain_u16
+        else:
+            check_frame_params(params, frames.dtype, c)
+            fn = None
+        oc = 3 if params.clahe else c
+        shape = (n, h, w, oc)
         if not frames.flags.c_contiguous:
             frames = np.ascontiguousarray(frames)
-        n, h, w, _ = frames.shape
         out_addr = None
         if out is None:
             # small results (the per-frame contract) land in recycled page-locked memory: the D2H copy is a plain DMA
             if frames.nbytes <= (64 << 20):
-                out = self._pooled_pinned(frames.shape, frames.dtype)
+                out = self._pooled_pinned(shape, frames.dtype)
                 out_addr = self._last_lease_addr
             else:
-                out = np.empty_like(frames)
-        elif out.shape != frames.shape or out.dtype != frames.dtype or not out.flags.c_contiguous:
-            raise ValueError(f"out must be a C-contiguous {frames.dtype} array of the input's shape")
+                out = np.empty(shape, frames.dtype)
+        elif out.shape != shape or out.dtype != frames.dtype or not out.flags.c_contiguous:
+            raise ValueError(f"out must be a C-contiguous {frames.dtype} array of shape {shape}")
         if out_addr is None:
             out_addr = out.ctypes.data
         if n == 1:
@@ -415,10 +442,23 @@ class Context:
         else:
             kind = MEM_PINNED if (self.mem_kind(frames) == MEM_PINNED and self.mem_kind(out) == MEM_PINNED) else MEM_HOST
         pp = processed.ctypes.data_as(_i32p) if processed is not None else None
-        rc = fn(self._h, frames.ctypes.data, out_addr, n, h, w, bpp * w, bpp * w, C.byref(params), kind, pp, None)
+        sb = frames.dtype.itemsize
+        if fn is None:
+            rc = self._lib.rv_chain_ex(self._h, frames.ctypes.data, out_addr, n, h, w, c * sb * w, oc * sb * w, bits, c, C.byref(params),
+                                       kind, pp, None)
+        else:
+            rc = fn(self._h, frames.ctypes.data, out_addr, n, h, w, 3 * sb * w, 3 * sb * w, C.byref(params), kind, pp, None)
         if rc != 0:
             self._ck(rc)
         return out
+
+    def chain_ex_device(self, in_ptr, out_ptr, n, h, w, params, bits, channels, stream=None):
+        """rv_chain_ex over contiguous device frames (ints) of `channels` channels and `bits` bits: asynchronous on `stream` (a
+        cudaStream_t int) when given, else synchronous on the context's stream."""
+        oc = check_frame_params(params, np.uint8 if bits == 8 else np.uint16, channels)
+        sb = bits // 8
+        self._ck(self._lib.rv_chain_ex(self._h, C.c_void_p(in_ptr), C.c_void_p(out_ptr), n, h, w, channels * sb * w, oc * sb * w, bits,
+                                       channels, C.byref(params), MEM_DEVICE, None, C.c_void_p(stream) if stream else None))
 
     def chain_u16_device(self, in_ptr, out_ptr, n, h, w, params, in_pitch=None, out_pitch=None, stream=None):
         """rv_chain_u16 over device pointers (ints, pitches in bytes): asynchronous on `stream` (a cudaStream_t int) when given,
@@ -588,12 +628,17 @@ class Context:
                                                   C.c_void_p(stream) if stream else None))
 
     def gray_span(self, frames):
-        _check_frames(frames, _U8_U16)
-        fn, bpp = (self._lib.rv_gray_span, 3) if frames.dtype == np.uint8 else (self._lib.rv_gray_span_u16, 6)
+        """Gray span (max - min of cv2's BGR2GRAY) of every (N,H,W,3) BGR or (N,H,W,4) BGRA frame (alpha ignored)."""
+        _check_frames(frames, _U8_U16, (3, 4))
         frames = np.ascontiguousarray(frames)
-        n, h, w, _ = frames.shape
+        n, h, w, c = frames.shape
         span = np.empty(n, np.int32)
-        self._ck(fn(self._h, frames.ctypes.data, n, h, w, bpp * w, span.ctypes.data, MEM_HOST))
+        sb = frames.dtype.itemsize
+        if c == 4:
+            self._ck(self._lib.rv_gray_span_ex(self._h, frames.ctypes.data, n, h, w, 4 * sb * w, 8 * sb, 4, span.ctypes.data, MEM_HOST))
+            return span
+        fn = self._lib.rv_gray_span if sb == 1 else self._lib.rv_gray_span_u16
+        self._ck(fn(self._h, frames.ctypes.data, n, h, w, 3 * sb * w, span.ctypes.data, MEM_HOST))
         return span
 
 

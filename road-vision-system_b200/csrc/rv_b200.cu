@@ -165,6 +165,7 @@ struct rv_ctx {
     void *fog = nullptr;                    // state of rv_fog.cu (fog synthesis), destroyed through fog_destroy
     void (*fog_destroy)(void *) = nullptr;
     U16Ws u16;                              // workspaces of rv_u16.cu (16-bit frames)
+    ChWs ch;                                // workspaces of rv_channels.cu (1- and 4-channel frames)
     StagePool *stage = nullptr;             // helper threads + page-locked staging frame for pageable single-frame input
     HostBuf fstage;                         // page-locked staging frame of the optional helper-thread upload
     long stage_threads = 0;                 // option "stage_threads": helpers next to the caller; 0 (default) = the driver stages pageable
@@ -277,15 +278,16 @@ int ws_release(rv_ctx *ctx, WsSync &w, cudaStream_t st)
     return RV_OK;
 }
 
-int check_frames(rv_ctx *ctx, const void *in, const void *out, int n, int h, int w, size_t ipitch, size_t opitch, int bytes_per_pixel)
+int check_frames(rv_ctx *ctx, const void *in, const void *out, int n, int h, int w, size_t ipitch, size_t opitch, int in_bpp,
+                 int out_bpp, int sample_bytes)
 {
     if (!ctx) return RV_ERR_ARG;
     if (!in || !out) return fail(ctx, RV_ERR_ARG, "null frame pointer");
     if (n < 0 || h < 1 || w < 1) return fail(ctx, RV_ERR_ARG, "bad frame shape n=%d h=%d w=%d", n, h, w);
     if (h > 32768 || w > 32768) return fail(ctx, RV_ERR_ARG, "frame too large (%dx%d)", w, h);
-    const size_t row = (size_t)bytes_per_pixel * w;
-    if (ipitch < row || opitch < row) return fail(ctx, RV_ERR_ARG, "pitch smaller than %d*w", bytes_per_pixel);
-    if (bytes_per_pixel == 6) {
+    if (ipitch < (size_t)in_bpp * w) return fail(ctx, RV_ERR_ARG, "pitch smaller than %d*w", in_bpp);
+    if (opitch < (size_t)out_bpp * w) return fail(ctx, RV_ERR_ARG, "pitch smaller than %d*w", out_bpp);
+    if (sample_bytes == 2) {
         if ((ipitch | opitch) & 1) return fail(ctx, RV_ERR_ARG, "16-bit frames need even pitches");
         if (((uintptr_t)in | (uintptr_t)out) & 1) return fail(ctx, RV_ERR_ARG, "16-bit frames need 2-byte aligned buffers");
     }
@@ -370,7 +372,9 @@ int clip_int(double clip_limit, const Geo &g)
     return std::max(c, 1);
 }
 
-int check_params(rv_ctx *ctx, const rv_params *p)
+}  // namespace
+
+int rv::check_params_u8(rv_ctx *ctx, const rv_params *p)
 {
     if (!p) return fail(ctx, RV_ERR_ARG, "null params");
     if (p->space != RV_SPACE_YCRCB && p->space != RV_SPACE_LAB) return fail(ctx, RV_ERR_ARG, "bad space %d", p->space);
@@ -379,6 +383,8 @@ int check_params(rv_ctx *ctx, const rv_params *p)
         return fail(ctx, RV_ERR_ARG, "ksize %d not in {0,3,5,7,9}", p->ksize);
     return RV_OK;
 }
+
+namespace {
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
                                   const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
@@ -609,7 +615,7 @@ struct LbFused {            // fused detector-input stage of one group (integer 
 
 int run_group(rv_ctx *ctx, int ws, const uint8_t *din, size_t ipitch, size_t ifs, uint8_t *dout, size_t opitch, size_t ofs,
               int n, int h, int w, const rv_params *p, cudaStream_t st, int32_t **flags_out, const LbFused *lb = nullptr,
-              cudaStream_t st_pre = nullptr, cudaEvent_t ev_pre = nullptr, bool capturing = false)
+              cudaStream_t st_pre = nullptr, cudaEvent_t ev_pre = nullptr, bool capturing = false, bool copy_skipped = true)
 {
     // capturing: `st` is in stream capture (single-frame graph): nothing may allocate, wait for or record outside events; the
     // set WS_FRAME is only ever used on that one stream, so it needs no cross-stream ordering
@@ -668,7 +674,7 @@ int run_group(rv_ctx *ctx, int ws, const uint8_t *din, size_t ipitch, size_t ifs
         RV_TRY(launch_chain(ctx, p->space == RV_SPACE_LAB ? 1 : 0, a, n, p->ksize, st));
     }
     if (a.flags) {
-        for (int f0 = 0; f0 < n; f0 += MAX_FRAMES_PER_LAUNCH) {
+        for (int f0 = 0; copy_skipped && f0 < n; f0 += MAX_FRAMES_PER_LAUNCH) {
             dim3 grid(4, std::min(h, 64), std::min(MAX_FRAMES_PER_LAUNCH, n - f0));
             k_gate_copy<<<grid, 256, 0, st>>>(din + (size_t)f0 * ifs, ipitch, ifs, dout + (size_t)f0 * ofs, opitch, ofs, h, 3 * w,
                                               a.flags + f0);
@@ -697,8 +703,10 @@ long auto_chunk(const rv_ctx *ctx, int h, int w)
     return std::max<long>(1, (long)((24u << 20) / fb));
 }
 
-int chain_device(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h, int w, size_t ipitch, size_t opitch,
-                 const rv_params *p, int32_t *processed_host, cudaStream_t st)
+}  // namespace
+
+int rv::chain_device(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h, int w, size_t ipitch, size_t opitch,
+                     const rv_params *p, int32_t *processed_host, cudaStream_t st, bool copy_skipped)
 {
     const size_t ifs = ipitch * h, ofs = opitch * h;
     // Overlap: the batch is cut into a few groups; histogram + LUT of group i+1 run on a high-priority side stream while
@@ -725,7 +733,8 @@ int chain_device(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h, int
     for (int f0 = 0; f0 < n; f0 += (int)G) {
         const int g = (int)std::min<long>(G, n - f0);
         int32_t *flags = nullptr;
-        RV_TRY(run_group(ctx, NPIPE, in + (size_t)f0 * ifs, ipitch, ifs, out + (size_t)f0 * ofs, opitch, ofs, g, h, w, p, st, &flags));
+        RV_TRY(run_group(ctx, NPIPE, in + (size_t)f0 * ifs, ipitch, ifs, out + (size_t)f0 * ofs, opitch, ofs, g, h, w, p, st, &flags,
+                         nullptr, nullptr, nullptr, false, copy_skipped));
         if (processed_host) {
             if (flags) {
                 CK(cudaMemcpyAsync(processed_host + f0, flags, (size_t)g * 4, cudaMemcpyDeviceToHost, st));
@@ -737,6 +746,8 @@ int chain_device(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h, int
     }
     return RV_OK;
 }
+
+namespace {
 
 int wait_all(rv_ctx *ctx)
 {
@@ -1149,6 +1160,7 @@ void rv_internal_count_launches(rv_ctx *ctx, long n) { ctx->launches += n; }
 void *rv_internal_get_fog(rv_ctx *ctx) { return ctx->fog; }
 void rv_internal_set_fog(rv_ctx *ctx, void *state, void (*destroy)(void *)) { ctx->fog = state; ctx->fog_destroy = destroy; }
 U16Ws &rv_internal_u16(rv_ctx *ctx) { return ctx->u16; }
+ChWs &rv_internal_ch(rv_ctx *ctx) { return ctx->ch; }
 
 extern "C" {
 
@@ -1197,6 +1209,7 @@ int rv_create(int device, rv_ctx **out)
         for (WsSync &w : ctx->wsync)
             if (cudaEventCreateWithFlags(&w.ev, cudaEventDisableTiming) != cudaSuccess) { delete ctx; return RV_ERR_CUDA; }
         if (cudaEventCreateWithFlags(&ctx->u16.sync.ev, cudaEventDisableTiming) != cudaSuccess) { delete ctx; return RV_ERR_CUDA; }
+        if (cudaEventCreateWithFlags(&ctx->ch.sync.ev, cudaEventDisableTiming) != cudaSuccess) { delete ctx; return RV_ERR_CUDA; }
         if (cudaStreamCreateWithFlags(&ctx->fstream, cudaStreamNonBlocking) != cudaSuccess) { delete ctx; return RV_ERR_CUDA; }
         if (cudaHostAlloc((void **)&ctx->fflag, 64, cudaHostAllocDefault) != cudaSuccess) { delete ctx; return RV_ERR_NOMEM; }
     }
@@ -1240,6 +1253,9 @@ void rv_destroy(rv_ctx *ctx)
     for (Buf *b : {&ctx->u16.lut, &ctx->u16.mid, &ctx->u16.din, &ctx->u16.dout, &ctx->u16.mm, &ctx->u16.flags})
         if (b->p) cudaFree(b->p);
     if (ctx->u16.hflags) cudaFreeHost(ctx->u16.hflags);
+    for (Buf *b : {&ctx->ch.pack, &ctx->ch.din, &ctx->ch.dout, &ctx->ch.mm, &ctx->ch.flags})
+        if (b->p) cudaFree(b->p);
+    if (ctx->ch.hflags) cudaFreeHost(ctx->ch.hflags);
     if (ctx->scratch.p) cudaFree(ctx->scratch.p);
     if (ctx->lbfull.p) cudaFree(ctx->lbfull.p);
     for (ColTab &t : ctx->coltabs) { cudaFree(t.dev); cudaFreeHost(t.host); cudaEventDestroy(t.ready); }
@@ -1247,6 +1263,7 @@ void rv_destroy(rv_ctx *ctx)
     for (WsSync &w : ctx->wsync)
         if (w.ev) cudaEventDestroy(w.ev);
     if (ctx->u16.sync.ev) cudaEventDestroy(ctx->u16.sync.ev);
+    if (ctx->ch.sync.ev) cudaEventDestroy(ctx->ch.sync.ev);
     drop_frame_graphs(ctx);
     if (ctx->stage) { ctx->stage->stop(); delete ctx->stage; }
     if (ctx->fstage.p) cudaFreeHost(ctx->fstage.p);
@@ -1396,7 +1413,7 @@ namespace {
 int check_chain_call(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h, int w, size_t in_pitch, size_t out_pitch, const rv_params *p)
 {
     RV_TRY(check_frames(ctx, in, out, n, h, w, in_pitch, out_pitch, 3));
-    RV_TRY(check_params(ctx, p));
+    RV_TRY(check_params_u8(ctx, p));
     if (!p->clahe && p->ksize == 0) return fail(ctx, RV_ERR_ARG, "nothing to do (no CLAHE, no median)");
     if (in == out) return fail(ctx, RV_ERR_ARG, "in-place operation is not supported (tiles read their neighbours' halo)");
     return RV_OK;
@@ -1427,7 +1444,7 @@ int rv_submit_io(rv_ctx *ctx, const rv_io *io, int n, int h, int w, const rv_par
     RV_TRY(check_kind(ctx, io->in_kind));
     // with no frame output the input stands in for it in the shape / pitch checks
     RV_TRY(check_frames(ctx, io->in, io->out ? io->out : io->in, n, h, w, io->in_pitch, io->out ? io->out_pitch : io->in_pitch, 3));
-    RV_TRY(check_params(ctx, p));
+    RV_TRY(check_params_u8(ctx, p));
     if (!p->clahe && p->ksize == 0) return fail(ctx, RV_ERR_ARG, "nothing to do (no CLAHE, no median)");
     if (io->out) {
         RV_TRY(check_kind(ctx, io->out_kind));
@@ -1569,7 +1586,7 @@ int rv_chain_letterbox_f16(rv_ctx *ctx, const uint8_t *in, int n, int h, int w, 
                            uint16_t *out, int S, int pad_value, uint8_t *full_out, size_t full_pitch, int mem_kind, void *stream)
 {
     RV_TRY(check_frames(ctx, in, full_out ? full_out : in, n, h, w, in_pitch, full_out ? full_pitch : in_pitch, 3));
-    RV_TRY(check_params(ctx, p));
+    RV_TRY(check_params_u8(ctx, p));
     RV_TRY(check_kind(ctx, mem_kind));
     if (!p->clahe && p->ksize == 0) return fail(ctx, RV_ERR_ARG, "nothing to do (no CLAHE, no median)");
     if (p->gate_enable) return fail(ctx, RV_ERR_ARG, "the gate is not supported together with the letterbox stage");

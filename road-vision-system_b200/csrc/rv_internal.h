@@ -1,5 +1,6 @@
 /*
- * rv_internal.h -- the host toolkit shared by the translation units of librv_b200.so (rv_b200.cu, rv_fog.cu, rv_u16.cu): error
+ * rv_internal.h -- the host toolkit shared by the translation units of librv_b200.so (rv_b200.cu, rv_fog.cu, rv_u16.cu,
+ * rv_channels.cu): error
  * recording, device buffers, workspace ordering between streams, and the argument rules and CLAHE geometry that every entry must
  * apply alike.  What is not defined here is defined once, in rv_b200.cu, which owns the context.  Not part of the C ABI
  * (include/rv_b200.h).
@@ -36,6 +37,14 @@ struct U16Ws {
     bool attr_set = false;                      // k_u16_hist_lut's dynamic shared-memory limit is raised
 };
 
+// Workspaces of the 1- and 4-channel path (rv_channels.cu) of one context, used on whichever stream a call runs on.
+struct ChWs {
+    Buf pack, din, dout, mm, flags;             // pack: BGR without alpha, the input of the 3-channel chains
+    int32_t *hflags = nullptr;                  // page-locked copy of the gate decisions / gray min-max pairs
+    size_t hflags_cap = 0;
+    WsSync sync;
+};
+
 int fail(rv_ctx *ctx, int code, const char *fmt, ...);     // records the message, returns code
 
 #define CK(call)                                                                                         \
@@ -55,10 +64,16 @@ int ensure(rv_ctx *ctx, Buf &b, size_t bytes);              // b holds at least 
 int ws_acquire(rv_ctx *ctx, WsSync &w, cudaStream_t st);    // `st` waits for the set's last user on another stream
 int ws_release(rv_ctx *ctx, WsSync &w, cudaStream_t st);    // after the last work queued on `st` that touches the set
 
-// Shape, pitch and overlap rules of frame arguments; bytes_per_pixel 3 (uint8 BGR) or 6 (uint16 BGR, which also needs even
-// pitches and 2-byte aligned buffers).
-int check_frames(rv_ctx *ctx, const void *in, const void *out, int n, int h, int w, size_t ipitch, size_t opitch,
-                 int bytes_per_pixel);
+// Shape, pitch and overlap rules of frame arguments: pitches of at least in_bpp * w (input) and out_bpp * w (output) bytes;
+// 2-byte samples (16-bit frames) also need even pitches and 2-byte aligned buffers.
+int check_frames(rv_ctx *ctx, const void *in, const void *out, int n, int h, int w, size_t ipitch, size_t opitch, int in_bpp,
+                 int out_bpp, int sample_bytes);
+// BGR frames: bytes_per_pixel 3 (uint8) or 6 (uint16)
+inline int check_frames(rv_ctx *ctx, const void *in, const void *out, int n, int h, int w, size_t ipitch, size_t opitch,
+                        int bytes_per_pixel)
+{
+    return check_frames(ctx, in, out, n, h, w, ipitch, opitch, bytes_per_pixel, bytes_per_pixel, bytes_per_pixel == 6 ? 2 : 1);
+}
 int check_kind(rv_ctx *ctx, int kind);
 
 // clahe.cpp geometry (A.3): both dimensions are padded when either is not divisible by the grid
@@ -84,11 +99,27 @@ void launch_gate_flags(rv_ctx *ctx, const int32_t *mm, int n, double thresh, int
 // span[i] = mm[2i+1] - mm[2i] for host (min, max) pairs; span is device memory when mem_kind is RV_MEM_DEVICE
 int write_spans(rv_ctx *ctx, const int32_t *mm, int n, int32_t *span, int mem_kind);
 
+// The chains' parameter rules: 8-bit (rv_b200.cu) and 16-bit (rv_u16.cu, which also rejects "nothing to do").
+int check_params_u8(rv_ctx *ctx, const rv_params *p);
+int check_params_u16(rv_ctx *ctx, const rv_params *p);
+
+// rv_b200.cu: the 8-bit chain over n device frames on stream `st`, group by group on the device path's workspace set.  With the
+// gate, processed_host (optional, host) receives the decisions and the frames it skips are copied through if copy_skipped.
+int chain_device(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h, int w, size_t ipitch, size_t opitch,
+                 const rv_params *p, int32_t *processed_host, cudaStream_t st, bool copy_skipped = true);
+
+// rv_u16.cu: frames per group of the 16-bit chain, and the chain on one group of device frames (workspaces `s`, which the caller
+// has acquired for `st`).  *flags_out receives the device gate flags or nullptr.
+long group_frames_u16(const rv_params *p, int h, int w);
+int run_group_u16(rv_ctx *ctx, U16Ws &s, const uint16_t *din, size_t ip, size_t ifs, uint16_t *dout, size_t op, size_t ofs, int n,
+                  int h, int w, const rv_params *p, cudaStream_t st, const int32_t **flags_out, bool copy_skipped = true);
+
 }  // namespace rv
 
 int rv_internal_device(const rv_ctx *ctx);
 void *rv_internal_stream(rv_ctx *ctx);                                  /* the context's main cudaStream_t */
 void rv_internal_count_launches(rv_ctx *ctx, long n);
 rv::U16Ws &rv_internal_u16(rv_ctx *ctx);
+rv::ChWs &rv_internal_ch(rv_ctx *ctx);
 void *rv_internal_get_fog(rv_ctx *ctx);
 void rv_internal_set_fog(rv_ctx *ctx, void *state, void (*destroy)(void *));

@@ -275,8 +275,12 @@ __global__ void k_u16_gate_copy(const uint8_t *__restrict__ src, size_t spitch, 
     }
 }
 
+}  // namespace
+
 // ------------------------------------------------------------------------------------------------ host side
-int check_params(rv_ctx *ctx, const rv_params *p)
+namespace rv {
+
+int check_params_u16(rv_ctx *ctx, const rv_params *p)
 {
     if (!p) return fail(ctx, RV_ERR_ARG, "null params");
     if (p->space == RV_SPACE_LAB) return fail(ctx, RV_ERR_ARG, "LAB has no 16-bit path (cv2.cvtColor BGR2LAB rejects CV_16U)");
@@ -289,7 +293,7 @@ int check_params(rv_ctx *ctx, const rv_params *p)
     return RV_OK;
 }
 
-long group_frames(const rv_params *p, int h, int w)
+long group_frames_u16(const rv_params *p, int h, int w)
 {
     const size_t fb = (size_t)6 * w * h;
     long g = std::max<long>(1, std::min<long>(256, (long)(((size_t)1 << 30) / fb)));
@@ -300,7 +304,7 @@ long group_frames(const rv_params *p, int h, int w)
     return g;
 }
 
-int launch_median(rv_ctx *ctx, int k, const uint16_t *src, size_t sp, size_t sfs, uint16_t *dst, size_t dp, size_t dfs, int n, int h,
+static int launch_median(rv_ctx *ctx, int k, const uint16_t *src, size_t sp, size_t sfs, uint16_t *dst, size_t dp, size_t dfs, int n, int h,
                   int w, const int32_t *flags, cudaStream_t st)
 {
     for (int f0 = 0; f0 < n; f0 += MAX_FRAMES_PER_LAUNCH) {
@@ -319,7 +323,7 @@ int launch_median(rv_ctx *ctx, int k, const uint16_t *src, size_t sp, size_t sfs
     return RV_OK;
 }
 
-int launch_gray(rv_ctx *ctx, U16Ws &s, const uint16_t *src, size_t sp, size_t sfs, int n, int h, int w, cudaStream_t st)
+static int launch_gray(rv_ctx *ctx, U16Ws &s, const uint16_t *src, size_t sp, size_t sfs, int n, int h, int w, cudaStream_t st)
 {
     RV_TRY(ensure(ctx, s.mm, (size_t)n * 8));
     int32_t *mm = (int32_t *)s.mm.p;
@@ -335,8 +339,8 @@ int launch_gray(rv_ctx *ctx, U16Ws &s, const uint16_t *src, size_t sp, size_t sf
 }
 
 // The chain on one group of frames that are on the device.  Returns the device gate flags (or nullptr) through flags_out.
-int run_group(rv_ctx *ctx, U16Ws &s, const uint16_t *din, size_t ip, size_t ifs, uint16_t *dout, size_t op, size_t ofs, int n,
-              int h, int w, const rv_params *p, cudaStream_t st, const int32_t **flags_out)
+int run_group_u16(rv_ctx *ctx, U16Ws &s, const uint16_t *din, size_t ip, size_t ifs, uint16_t *dout, size_t op, size_t ofs, int n,
+                  int h, int w, const rv_params *p, cudaStream_t st, const int32_t **flags_out, bool copy_skipped)
 {
     const int32_t *flags = nullptr;
     if (p->gate_enable) {
@@ -375,7 +379,7 @@ int run_group(rv_ctx *ctx, U16Ws &s, const uint16_t *din, size_t ip, size_t ifs,
     } else {
         RV_TRY(launch_median(ctx, p->ksize, din, ip, ifs, dout, op, ofs, n, h, w, flags, st));
     }
-    if (flags) {
+    if (flags && copy_skipped) {
         k_u16_gate_copy<<<dim3(4, std::min(h, 64), n), 256, 0, st>>>((const uint8_t *)din, ip, ifs, (uint8_t *)dout, op, ofs, h, 6 * w,
                                                                      flags);
         rv_internal_count_launches(ctx, 1);
@@ -385,7 +389,7 @@ int run_group(rv_ctx *ctx, U16Ws &s, const uint16_t *din, size_t ip, size_t ifs,
     return RV_OK;
 }
 
-int host_flags(rv_ctx *ctx, U16Ws &s, int n)
+static int host_flags(rv_ctx *ctx, U16Ws &s, int n)
 {
     if (s.hflags_cap >= (size_t)n) return RV_OK;
     if (s.hflags) CK(cudaFreeHost(s.hflags));
@@ -396,7 +400,7 @@ int host_flags(rv_ctx *ctx, U16Ws &s, int n)
     return RV_OK;
 }
 
-}  // namespace
+}  // namespace rv
 
 extern "C" {
 
@@ -404,7 +408,7 @@ int rv_chain_u16(rv_ctx *ctx, const uint16_t *in, uint16_t *out, int n, int h, i
                  const rv_params *p, int mem_kind, int32_t *processed, void *stream)
 {
     RV_TRY(check_frames(ctx, in, out, n, h, w, in_pitch, out_pitch, 6));
-    RV_TRY(check_params(ctx, p));
+    RV_TRY(check_params_u16(ctx, p));
     RV_TRY(check_kind(ctx, mem_kind));
     if (in == out) return fail(ctx, RV_ERR_ARG, "in-place operation is not supported (tiles read their neighbours' halo)");
     if (n == 0) return RV_OK;
@@ -414,7 +418,7 @@ int rv_chain_u16(rv_ctx *ctx, const uint16_t *in, uint16_t *out, int n, int h, i
     cudaStream_t st = (dev && stream) ? (cudaStream_t)stream : (cudaStream_t)rv_internal_stream(ctx);
     RV_TRY(ws_acquire(ctx, s.sync, st));
     if (processed && p->gate_enable) RV_TRY(host_flags(ctx, s, n));
-    const long G = group_frames(p, h, w);
+    const long G = group_frames_u16(p, h, w);
     const size_t fb = (size_t)6 * w * h;
     for (int f0 = 0; f0 < n; f0 += (int)G) {
         const int g = (int)std::min<long>(G, n - f0);
@@ -435,7 +439,7 @@ int rv_chain_u16(rv_ctx *ctx, const uint16_t *in, uint16_t *out, int n, int h, i
             ip = op = (size_t)6 * w;
         }
         const int32_t *flags = nullptr;
-        RV_TRY(run_group(ctx, s, gin, ip, ip * h, gout, op, op * h, g, h, w, p, st, &flags));
+        RV_TRY(run_group_u16(ctx, s, gin, ip, ip * h, gout, op, op * h, g, h, w, p, st, &flags));
         if (!dev)
             CK(cudaMemcpy2DAsync((uint8_t *)out + (size_t)f0 * h * out_pitch, out_pitch, s.dout.p, (size_t)6 * w, (size_t)6 * w,
                                  (size_t)h * g, cudaMemcpyDeviceToHost, st));

@@ -44,3 +44,15 @@ def as_bgr_frame(image):
             raise ValueError("empty image")
         return np.ascontiguousarray(image)
     return as_bgr_u8(image)
+
+
+def as_frame(image):
+    """as_bgr_frame, but also admitting what cv2 accepts beyond BGR: (H,W,4) BGRA / BGRx frames (cv2.imread(..., IMREAD_UNCHANGED) on
+    PNGs with alpha, video decoder surfaces) and single-channel (H,W) or (H,W,1) frames (monochrome, NIR and thermal cameras), uint8
+    or uint16, any strides.  Returns a C-contiguous (H,W,C) array (a single channel as (H,W,1)) of the input's dtype."""
+    if isinstance(image, np.ndarray) and image.dtype in (np.uint8, np.uint16) and \
+            (image.ndim == 2 or (image.ndim == 3 and image.shape[2] in (1, 4))):
+        if image.shape[0] < 1 or image.shape[1] < 1:
+            raise ValueError("empty image")
+        return np.ascontiguousarray(image.reshape(image.shape[0], image.shape[1], -1))
+    return as_bgr_frame(image)

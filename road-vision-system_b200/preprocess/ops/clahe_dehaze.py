@@ -3,10 +3,8 @@
 Same name, params and per-frame contract; the cv2.cvtColor / split / createCLAHE().apply /
 merge / cvtColor sequence (:19-30) runs as the sm_100a kernels behind rv_clahe_dehaze.
 """
-import numpy as np
-
-from ..._native import Params, check_u16_params, default_context
-from ..base import PreprocessOp, as_bgr_frame
+from ..._native import Params, check_frame_params, default_context
+from ..base import PreprocessOp, as_frame
 
 
 def coerce(params):
@@ -21,12 +19,13 @@ class CLAHEDehaze(PreprocessOp):
     """CLAHE on the luminance channel. params: space "YCrCb"|"LAB", clip_limit float, tile_grid int.
 
     uint16 frames run cv2's 16-bit chain (65,536-bin histograms) in YCrCb with tile_grid <= 64; LAB raises ValueError there, as
-    cv2 has no 16-bit LAB."""
+    cv2 has no 16-bit LAB.  (H,W,4) BGRA frames give a (H,W,3) result, as cv2.cvtColor ignores and drops alpha; single-channel
+    frames raise ValueError (cv2 has no colour conversion for them)."""
 
     def __call__(self, image):
         space, clip_limit, grid = coerce(self.params)
-        img = as_bgr_frame(image)
-        if img.dtype == np.uint16:
-            check_u16_params(Params.make(space, clip_limit, grid, 0, clahe=True))      # LAB / grid > 64: before the GPU
+        img = as_frame(image)
+        # LAB / grid > 64 at 16 bits, a single channel: before the GPU
+        check_frame_params(Params.make(space, clip_limit, grid, 0, clahe=True), img.dtype, img.shape[2])
         ctx = default_context(self.params.get("device"))
         return ctx.clahe_dehaze(img[None], space, clip_limit, grid)[0]

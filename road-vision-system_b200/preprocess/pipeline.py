@@ -10,8 +10,8 @@ from typing import Any, Dict
 
 import numpy as np
 
-from .._native import DeviceArray, Params, check_u16_params, default_context
-from .base import as_bgr_frame
+from .._native import DeviceArray, Params, check_frame_params, check_u16_params, default_context
+from .base import as_bgr_frame, as_frame
 from .ops import CLAHEDehaze, MedianDerain
 from .ops import clahe_dehaze as _clahe
 from .ops import median_derain as _median
@@ -49,8 +49,8 @@ class PreprocessPipeline:
         return enable, float(self.auto_gate_cfg.get("contrast_thresh", 20.0))
 
     def _low_contrast(self, image) -> bool:
-        """pipeline.py:24-30: gray span < thresh (gray = cv2 BGR2GRAY fixed point, computed on the GPU)."""
-        span = int(self._ctx().gray_span(as_bgr_frame(image)[None])[0])
+        """pipeline.py:24-30: gray span < thresh (gray = cv2 BGR2GRAY fixed point, computed on the GPU; BGRA: alpha ignored)."""
+        span = int(self._ctx().gray_span(as_frame(image)[None])[0])
         return span < self._gate()[1]
 
     def _segments(self):
@@ -101,6 +101,24 @@ class PreprocessPipeline:
             if isinstance(sg, Params):
                 check_u16_params(sg)
 
+    def _check_channels(self, segs, dtype, channels):
+        """What cv2 would reject on (..., channels) frames -- the gate or a CLAHE pass on a single channel -- raises ValueError before
+        any frame reaches the GPU.  Channel counts are followed through the GPU passes (CLAHE gives 3) up to the first foreign
+        operator, whose output is unknown until it runs.  Returns the channel count after the passes, or None if a foreign op
+        decides it."""
+        if self._gate()[0]:
+            check_frame_params(Params.make(clahe=False, ksize=3, gate=True), dtype, channels)
+        for sg in segs:
+            if not isinstance(sg, Params):
+                return None
+            channels = check_frame_params(sg, dtype, channels)
+        return channels
+
+    def _pass(self, image, seg, **kw):
+        """One fused GPU pass on one frame; a single-channel result comes back as (H,W), as from cv2."""
+        out = self._ctx().chain(as_frame(image)[None], seg, **kw)[0]
+        return out[..., 0] if out.shape[2] == 1 else out
+
     # -- per-frame contract --------------------------------------------------------------
     def __call__(self, image: np.ndarray, ts: float = None) -> np.ndarray:
         if not self.enabled or not self.ops:
@@ -108,20 +126,24 @@ class PreprocessPipeline:
         segs = self._segments()
         if isinstance(image, np.ndarray) and image.dtype != np.uint8 and image.dtype == np.uint16:
             self._check_u16(segs)
+        frame = image
+        if self._gate()[0] or isinstance(segs[0], Params):
+            frame = as_frame(image)
+            self._check_channels(segs, frame.dtype, frame.shape[2])
         if self._gate()[0]:
             if len(segs) == 1 and isinstance(segs[0], Params):
                 # one fused pass: the gate's gray span comes out of the histogram pass of the same upload
                 seg = segs[0]
                 seg.gate_enable, seg.gate_thresh = 1, self._gate()[1]
                 flag = np.ones(1, np.int32)
-                out = self._ctx().chain(as_bgr_frame(image)[None], seg, processed=flag)[0]
+                out = self._pass(frame, seg, processed=flag)
                 return out if flag[0] else image          # skipped: the input object itself, as pipeline.py:39-40
-            if not self._low_contrast(image):
+            if not self._low_contrast(frame):
                 return image
         out = image
         for seg in segs:
             if isinstance(seg, Params):
-                out = self._ctx().chain(as_bgr_frame(out)[None], seg)[0]
+                out = self._pass(out, seg)
             else:
                 out = seg(out)
         return out
@@ -143,11 +165,14 @@ class PreprocessPipeline:
             if out != "device":
                 raise ValueError('out must be an array, None or "device"')
             return self._process_batch_keep(frames)
-        if not isinstance(frames, np.ndarray) or frames.ndim != 4 or frames.shape[3] != 3 or \
+        if not isinstance(frames, np.ndarray) or frames.ndim != 4 or frames.shape[3] not in (1, 3, 4) or \
                 (frames.dtype != np.uint8 and frames.dtype != np.uint16):
-            raise ValueError("frames must be a (B,H,W,3) uint8 or uint16 numpy array (or a torch CUDA tensor of that shape)")
+            raise ValueError("frames must be a (B,H,W,C) uint8 or uint16 numpy array with C = 1 (gray), 3 (BGR) or 4 (BGRA) (or a torch "
+                             "CUDA tensor of that shape)")
         if frames.dtype == np.uint16 and self.enabled and self.ops:
             self._check_u16(self._segments())
+        if self.enabled and self.ops:
+            self._check_batch_channels(self._segments(), frames.dtype, frames.shape[3])
         if not self.enabled or not self.ops:
             if out is None:
                 return frames
@@ -183,14 +208,23 @@ class PreprocessPipeline:
                     cur = out
         return cur
 
+    def _check_batch_channels(self, segs, dtype, channels):
+        """_check_channels for a batch, which must have one result shape: with the gate, a CLAHE pass on BGRA frames would give
+        3-channel processed frames next to 4-channel skipped ones."""
+        self._check_channels(segs, dtype, channels)
+        if self._gate()[0] and channels == 4 and any(isinstance(sg, Params) and sg.clahe for sg in segs):
+            raise ValueError("the low-contrast gate with CLAHEDehaze on BGRA batches would mix 3-channel (processed) and 4-channel "
+                             "(skipped) frames; call the pipeline per frame, or drop alpha first")
+
     def _process_batch_keep(self, frames):
         """Host frames in, result left on the GPU (no D2H at all)."""
-        if not isinstance(frames, np.ndarray) or frames.ndim != 4 or frames.shape[3] != 3 or \
+        if not isinstance(frames, np.ndarray) or frames.ndim != 4 or frames.shape[3] not in (1, 3, 4) or \
                 (frames.dtype != np.uint8 and frames.dtype != np.uint16):
-            raise ValueError("frames must be a (B,H,W,3) uint8 or uint16 numpy array")
+            raise ValueError("frames must be a (B,H,W,C) uint8 or uint16 numpy array with C = 1, 3 or 4")
         segs = self._segments() if (self.enabled and self.ops) else []
         if frames.dtype == np.uint16:
             self._check_u16(segs)
+        self._check_batch_channels(segs, frames.dtype, frames.shape[3])
         ctx = self._ctx()
         frames = np.ascontiguousarray(frames)
         if not segs or self._gate()[0] or not all(isinstance(sg, Params) for sg in segs):
@@ -199,6 +233,17 @@ class PreprocessPipeline:
             dev = DeviceArray(ctx, res.shape, res.dtype)
             ctx._ck(ctx._lib.rv_memcpy(ctx._h, dev.ptr, np.ascontiguousarray(res).ctypes.data, dev.nbytes, 0))
             return dev
+        if frames.shape[3] != 3:
+            # gray / BGRA: upload once, then every pass runs device to device (CLAHE passes give 3 channels)
+            b, h, w, c = frames.shape
+            cur = DeviceArray(ctx, frames.shape, frames.dtype)
+            ctx._ck(ctx._lib.rv_memcpy(ctx._h, cur.ptr, frames.ctypes.data, cur.nbytes, 0))
+            for sg in segs:
+                oc = 3 if sg.clahe else c
+                dst = DeviceArray(ctx, (b, h, w, oc), frames.dtype)
+                ctx.chain_ex_device(cur.ptr, dst.ptr, b, h, w, sg, 8 * frames.dtype.itemsize, c)
+                cur, c = dst, oc
+            return cur
         if frames.dtype == np.uint16:
             # upload once, then every pass runs device to device
             b, h, w, _ = frames.shape
@@ -218,18 +263,24 @@ class PreprocessPipeline:
         return cur
 
     def _process_batch_device(self, frames, out=None):
-        """Device-resident batch: a contiguous torch CUDA uint8 tensor (B,H,W,3) in, a tensor of the same kind out.
-        Work is enqueued on torch's current stream (no host synchronisation): use the result with torch as usual."""
+        """Device-resident batch: a contiguous torch CUDA uint8 / uint16 tensor (B,H,W,C), C = 1, 3 or 4, in, a tensor of the same
+        kind out (3 channels after a CLAHE pass).  Work is enqueued on torch's current stream (no host synchronisation): use the
+        result with torch as usual."""
         import torch
-        if (frames.dtype != torch.uint8 and frames.dtype != torch.uint16) or frames.dim() != 4 or frames.shape[3] != 3 or \
+        if (frames.dtype != torch.uint8 and frames.dtype != torch.uint16) or frames.dim() != 4 or frames.shape[3] not in (1, 3, 4) or \
                 not frames.is_contiguous():
-            raise ValueError("frames must be a contiguous (B,H,W,3) uint8 or uint16 CUDA tensor")
-        if out is not None and not (_is_cuda_tensor(out) and out.dtype == frames.dtype and tuple(out.shape) == tuple(frames.shape)
-                                    and out.device == frames.device and out.is_contiguous()):
-            raise ValueError("out must be a contiguous CUDA tensor of the input's shape, dtype and device")
+            raise ValueError("frames must be a contiguous (B,H,W,C) uint8 or uint16 CUDA tensor with C = 1, 3 or 4")
         wide = frames.dtype == torch.uint16
         if wide and self.enabled and self.ops:
             self._check_u16(self._segments())
+        final = tuple(frames.shape)
+        if self.enabled and self.ops:
+            self._check_batch_channels(self._segments(), np.uint16 if wide else np.uint8, frames.shape[3])
+            if any(isinstance(sg, Params) and sg.clahe for sg in self._segments()):
+                final = final[:3] + (3,)
+        if out is not None and not (_is_cuda_tensor(out) and out.dtype == frames.dtype and tuple(out.shape) == final
+                                    and out.device == frames.device and out.is_contiguous()):
+            raise ValueError(f"out must be a contiguous CUDA tensor of shape {final} and the input's dtype and device")
         if not self.enabled or not self.ops:
             return frames if out is None else out.copy_(frames)
         if self._gate()[0]:
@@ -243,7 +294,17 @@ class PreprocessPipeline:
         stream = torch.cuda.current_stream(frames.device).cuda_stream
         cur = frames
         for idx, sg in enumerate(segs):
-            dst = out if (idx == len(segs) - 1 and out is not None) else torch.empty_like(frames)
+            c = cur.shape[3]
+            oc = 3 if sg.clahe else c
+            last = idx == len(segs) - 1 and out is not None
+            if c != 3:
+                dst = out if last else torch.empty((b, h, w, oc), dtype=frames.dtype, device=frames.device)
+                if stream == 0:
+                    torch.cuda.current_stream(frames.device).synchronize()
+                ctx.chain_ex_device(cur.data_ptr(), dst.data_ptr(), b, h, w, sg, 16 if wide else 8, c, stream=stream or None)
+                cur = dst
+                continue
+            dst = out if last else torch.empty_like(cur)
             if wide:
                 if stream == 0:
                     torch.cuda.current_stream(frames.device).synchronize()
