@@ -22,11 +22,14 @@
  *   rv_chain_ex        rv_chain_u8 / rv_chain_u16 for 1-, 3- and 4-channel frames (gray; BGR; BGRA / BGRx) at either depth, as
  *                      cv2 treats the arrays the reference hands it unchanged
  *   rv_gray_span_ex    rv_gray_span / rv_gray_span_u16 for 3- and 4-channel frames
+ *   rv_yuv420_to_bgr   (new) cv2.cvtColor(COLOR_YUV2BGR_NV12 / COLOR_YUV2BGR_I420), the host-side step a user of the reference runs on a
+ *                      decoder's 4:2:0 output before pipeline(frame)
  *   rv_submit/rv_wait  (new) batched multi-frame entry fed from pinned host buffers; no reference
  *                      counterpart (the reference loop is one frame in flight, main_preview.py:88-142)
  *   rv_submit_io       (new) the same with every end of the job placed independently: what src/io_video/capture.py:18-21
  *                      captured on the host goes in, the processed frames and / or the detector's input tensor
  *                      (main_preview.py:99 -> src/detect/yolo_ultralytics.py:28-35) come out on the host or stay on the GPU
+ *   rv_submit_io_yuv   (new) rv_submit_io on NV12 / I420 frames: the YUV bytes cross PCIe and are converted to BGR on the GPU
  *
  * Conventions: plain C types only; every function returns 0 on success or a negative rv_status;
  * rv_last_error(ctx) gives the message.  A context is bound to one CUDA device, owns its streams and
@@ -264,6 +267,23 @@ int rv_chain_ex(rv_ctx *ctx, const void *in, void *out, int n, int h, int w, siz
                 const rv_params *p, int mem_kind, int32_t *processed, void *stream);
 /* span: n ints = max(gray) - min(gray) per 3- or 4-channel frame (synchronous; one channel -> RV_ERR_ARG) */
 int rv_gray_span_ex(rv_ctx *ctx, const void *in, int n, int h, int w, size_t pitch, int bits, int channels, int32_t *span, int mem_kind);
+
+/* ---- YUV 4:2:0 frames (NV12 from hardware decoders: NVDEC, V4L2 M2M, VA-API, GStreamer `appsink format=NV12`; I420 from libavcodec
+ * yuv420p), converted to BGR exactly as cv2.cvtColor(COLOR_YUV2BGR_NV12 / COLOR_YUV2BGR_I420) does (arithmetic in csrc/rv_yuv.cu).
+ * A frame is cv2's single array of 3h/2 rows of `in_pitch` bytes: h rows of Y, then
+ *   RV_YUV_NV12  h/2 rows of interleaved U, V bytes (U first), at the same pitch;
+ *   RV_YUV_I420  w*h/4 bytes of U, then w*h/4 bytes of V, packed (in_pitch must equal w).
+ * Frame f starts at f * in_pitch * h * 3 / 2.  h and w are the BGR frame's, even and >= 2.  RV_ERR_ARG also for a bad layout,
+ * in_pitch < w, out_pitch < 3*w and overlapping buffers. */
+enum rv_yuv { RV_YUV_NV12 = 1, RV_YUV_I420 = 2 };
+/* The conversion alone into n BGR frames at out_pitch.  Host memory goes group by group and is synchronous; RV_MEM_DEVICE with a
+ * `stream` is asynchronous on that stream, without one synchronous on the context's stream. */
+int rv_yuv420_to_bgr(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h, int w, size_t in_pitch, size_t out_pitch, int layout,
+                     int mem_kind, void *stream);
+/* rv_submit_io with 4:2:0 frames in io->in (host or device): each chunk's YUV bytes are uploaded (or read in place on the device),
+ * converted into the BGR workspace, and the chain, gate, letterbox and result copies run exactly as for BGR input.  Results equal
+ * rv_submit_io on the frames rv_yuv420_to_bgr gives. */
+int rv_submit_io_yuv(rv_ctx *ctx, const rv_io *io, int layout, int n, int h, int w, const rv_params *p);
 
 #ifdef __cplusplus
 }

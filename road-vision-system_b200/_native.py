@@ -14,6 +14,7 @@ _SO = os.path.join(_CSRC, "librv_b200.so")
 
 SPACE_YCRCB, SPACE_LAB = 0, 1
 MEM_HOST, MEM_PINNED, MEM_DEVICE = 0, 1, 2
+YUV_LAYOUTS = {"NV12": 1, "I420": 2}        # enum rv_yuv
 
 
 class RvError(RuntimeError):
@@ -212,6 +213,9 @@ EXPORTS = {
     "rv_chain_ex": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_int, C.c_int,
                               C.POINTER(Params), C.c_int, _i32p, C.c_void_p]),
     "rv_gray_span_ex": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_int, C.c_int, C.c_void_p, C.c_int]),
+    "rv_yuv420_to_bgr": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_int, C.c_int,
+                                   C.c_void_p]),
+    "rv_submit_io_yuv": (C.c_int, [C.c_void_p, C.POINTER(IO), C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(Params)]),
 }
 
 
@@ -234,6 +238,10 @@ def load_library():
     return _lib
 
 
+def _is_torch(x):
+    return type(x).__module__.startswith("torch")
+
+
 _U8 = (np.dtype(np.uint8),)
 _U8_U16 = (np.dtype(np.uint8), np.dtype(np.uint16))
 CHANNELS = (1, 3, 4)        # gray, BGR, BGRA / BGRx
@@ -250,6 +258,29 @@ def _check_frames(frames, dtypes=_U8, channels=(3,)):
         raise ValueError(f"(N,H,W,{want}) {frames.dtype} expected, got shape {frames.shape}")
     if frames.shape[1] < 1 or frames.shape[2] < 1:
         raise ValueError("empty frame")
+
+
+def check_yuv_frames(shape, is_uint8, yuv):
+    """A batch of YUV 4:2:0 frames in cv2's single-array form, (B, 3H/2, W) uint8, as cv2.cvtColor(COLOR_YUV2BGR_NV12 / _I420) takes
+    them: returns (layout, B, H, W) of the BGR frames they convert to.  Raises ValueError for an unknown `yuv`, a wrong shape or dtype,
+    rows not divisible by 3 (H must be even), an odd W (cv2 raises for it) and empty frames."""
+    if yuv not in YUV_LAYOUTS:
+        raise ValueError(f"yuv must be None, 'NV12' or 'I420', got {yuv!r}")
+    shape = tuple(int(v) for v in shape)
+    if len(shape) == 4:
+        raise ValueError(f"yuv={yuv!r} takes (B,3H/2,W) frames, not (B,H,W,C) ones (got shape {shape})")
+    if len(shape) != 3:
+        raise ValueError(f"yuv={yuv!r} takes (B,3H/2,W) uint8 frames, got shape {shape}")
+    if not is_uint8:
+        raise ValueError(f"yuv={yuv!r} takes uint8 frames")
+    b, rows, w = shape
+    if rows == 0 or w == 0:
+        raise ValueError(f"empty {yuv} frames (shape {shape})")
+    if rows % 3:
+        raise ValueError(f"{yuv} frames have 3H/2 rows with an even H: {rows} rows is not a multiple of 3")
+    if w % 2:
+        raise ValueError(f"{yuv} frames need an even width, got {w}")
+    return YUV_LAYOUTS[yuv], b, rows // 3 * 2, w
 
 
 U16_MAX_GRID = 64
@@ -479,6 +510,38 @@ class Context:
                                      in_pitch or 3 * w, out_pitch or 3 * w, C.byref(params), MEM_DEVICE,
                                      C.c_void_p(stream) if stream else None))
 
+    def yuv420_to_bgr(self, frames, yuv, out=None):
+        """cv2.cvtColor(COLOR_YUV2BGR_NV12 / _I420) of every frame of a (B,3H/2,W) uint8 batch -> (B,H,W,3) BGR, on the GPU.
+        `frames`: a numpy array (pageable or pinned; synchronous) or a contiguous torch CUDA tensor (asynchronous on torch's current
+        stream; the result is a tensor).  `out` (optional): an array / tensor of the result's shape to write into."""
+        if _is_torch(frames):
+            import torch
+            layout, b, h, w = check_yuv_frames(frames.shape, frames.dtype == torch.uint8, yuv)
+            if not (frames.is_cuda and frames.is_contiguous()):
+                raise ValueError("device frames must be a contiguous CUDA tensor")
+            if out is None:
+                out = torch.empty((b, h, w, 3), dtype=torch.uint8, device=frames.device)
+            elif not (_is_torch(out) and out.dtype == torch.uint8 and tuple(out.shape) == (b, h, w, 3) and out.device == frames.device
+                      and out.is_contiguous()):
+                raise ValueError(f"out must be a contiguous uint8 CUDA tensor of shape {(b, h, w, 3)} on the input's device")
+            stream = torch.cuda.current_stream(frames.device).cuda_stream
+            if stream == 0:             # legacy default stream: run on the context's stream, synchronously
+                torch.cuda.current_stream(frames.device).synchronize()
+            self._ck(self._lib.rv_yuv420_to_bgr(self._h, C.c_void_p(frames.data_ptr()), C.c_void_p(out.data_ptr()), b, h, w, w, 3 * w,
+                                                layout, MEM_DEVICE, C.c_void_p(stream) if stream else None))
+            return out
+        if not isinstance(frames, np.ndarray):
+            raise ValueError("frames must be a numpy array or a torch CUDA tensor")
+        layout, b, h, w = check_yuv_frames(frames.shape, frames.dtype == np.uint8, yuv)
+        frames = np.ascontiguousarray(frames)
+        if out is None:
+            out = np.empty((b, h, w, 3), np.uint8)
+        elif not (isinstance(out, np.ndarray) and out.shape == (b, h, w, 3) and out.dtype == np.uint8 and out.flags.c_contiguous):
+            raise ValueError(f"out must be a C-contiguous uint8 array of shape {(b, h, w, 3)}")
+        kind = MEM_PINNED if (self.mem_kind(frames) == MEM_PINNED and self.mem_kind(out) == MEM_PINNED) else MEM_HOST
+        self._ck(self._lib.rv_yuv420_to_bgr(self._h, frames.ctypes.data, out.ctypes.data, b, h, w, w, 3 * w, layout, kind, None))
+        return out
+
     def kernel_times(self, reset=False):
         """{name: (total_ms, launches)} for the hot-path kernels (needs set_option('kernel_timing', 1))."""
         res = {}
@@ -526,27 +589,40 @@ class Context:
         tensor[:, :, top + nh:, :] = v
         return tensor
 
-    def submit_io(self, frames, params, shape=None, out=None, tensor=None, size=640, pad_value=114, processed=None, padding_present=False):
+    def submit_io(self, frames, params, shape=None, out=None, tensor=None, size=640, pad_value=114, processed=None, padding_present=False,
+                  yuv=None):
         """rv_submit_io: asynchronous job whose ends live independently on the host or on the GPU; call wait() afterwards.
 
         frames: (N,H,W,3) uint8 numpy array (pinned or pageable) or a device object / pointer (then pass shape=(N,H,W)).
         out:    frames result, numpy or device (DeviceArray / anything with __cuda_array_interface__ / int pointer), or None.
-        tensor: (N,3,size,size) float16 detector input, numpy or device, or None."""
-        if isinstance(frames, np.ndarray):
+        tensor: (N,3,size,size) float16 detector input, numpy or device, or None.
+        yuv:    "NV12" / "I420": `frames` are (N,3H/2,W) 4:2:0 frames (rv_submit_io_yuv; `shape` is still (N,H,W)), converted to BGR on
+                the GPU, so only their 1.5 bytes per pixel cross PCIe."""
+        layout = 0
+        if yuv is not None:
+            if isinstance(frames, np.ndarray):
+                layout, n, h, w = check_yuv_frames(frames.shape, frames.dtype == np.uint8, yuv)
+            else:
+                layout = check_yuv_frames((shape[0], shape[1] * 3 // 2, shape[2]), True, yuv)[0]
+                n, h, w = shape
+        elif isinstance(frames, np.ndarray):
             _check_frames(frames)
             n, h, w, _ = frames.shape
         else:
             n, h, w = shape
         io = IO()
         io.in_, io.in_kind = self._end(frames)
-        io.in_pitch = 3 * w
+        io.in_pitch = w if layout else 3 * w
         io.out, io.out_kind = self._end(out)
         io.out_pitch = 3 * w
         io.tensor, io.tensor_kind = self._end(tensor)
         io.tensor_size, io.pad_value = int(size), int(pad_value)
         io.tensor_flags = 1 if padding_present else 0
         io.processed = processed.ctypes.data if processed is not None else None
-        self._ck(self._lib.rv_submit_io(self._h, C.byref(io), n, h, w, C.byref(params)))
+        if layout:
+            self._ck(self._lib.rv_submit_io_yuv(self._h, C.byref(io), layout, n, h, w, C.byref(params)))
+        else:
+            self._ck(self._lib.rv_submit_io(self._h, C.byref(io), n, h, w, C.byref(params)))
 
     # -- stage-level entry points (parity tests) ---------------------------------------------
     def luma_hist(self, frames, space, grid, want_luma=True, want_gray=False):

@@ -158,6 +158,7 @@ struct rv_ctx {
     Buf hist[NWS], quads[NWS], lut[NWS], flags[NWS], mm[NWS];
     Buf din[NWS], dout[NWS];
     Buf dlb[NPIPE];                         // detector tensors of the host pipeline's chunks
+    Buf dyuv[NPIPE];                        // 4:2:0 input chunks of the host pipeline (rv_submit_io_yuv), before the conversion
     WsSync wsync[NWS];
     cudaStream_t fstream = nullptr;         // single-frame path (per-frame plugin contract): its own stream, workspace set and graphs
     std::vector<struct FrameGraph> fgraphs;
@@ -899,6 +900,7 @@ int launch_letterbox(rv_ctx *ctx, const uint8_t *src, size_t pitch, size_t fstri
 // H2D, a device output / tensor skips its D2H (results that the next stage consumes on the same GPU never cross PCIe).
 struct PipeJob {
     const uint8_t *in = nullptr; int in_kind = RV_MEM_HOST; size_t ipitch = 0;
+    int yuv = 0;                            // RV_YUV_NV12 / RV_YUV_I420: 4:2:0 frames in, converted into the BGR workspace first; 0 = BGR
     uint8_t *out = nullptr; int out_kind = RV_MEM_HOST; size_t opitch = 0;      // full-resolution result; nullptr = not wanted
     uint16_t *lb = nullptr; int lb_kind = RV_MEM_HOST; int S = 0, pad = 114;     // detector tensor; nullptr = none
     bool lb_rows_only = false;              // host tensor whose padding rows the caller already holds: copy back the image rows only
@@ -934,8 +936,11 @@ int chain_pipe(rv_ctx *ctx, const PipeJob &j, int n, int h, int w, const rv_para
     }
     const bool fused = j.lb && lg.scale > 0;
     const bool need_dfull = (j.out && !out_dev) || (j.lb && !fused && !(j.out && out_dev));   // a device staging copy of the full result
+    // 4:2:0 chunks are uploaded at a pitch that k_yuv420_to_bgr's vector path can read (I420 planes stay packed)
+    const size_t ypitch = j.yuv == RV_YUV_NV12 ? ((size_t)w + 7) & ~(size_t)7 : (size_t)w, yfs = ypitch * h * 3 / 2;
     for (int i = 0; i < NPIPE; ++i) {
-        if (!in_dev) RV_TRY(ensure(ctx, ctx->din[i], dfs * C));
+        if (!in_dev || j.yuv) RV_TRY(ensure(ctx, ctx->din[i], dfs * C));
+        if (j.yuv && !in_dev) RV_TRY(ensure(ctx, ctx->dyuv[i], yfs * C));
         if (need_dfull) RV_TRY(ensure(ctx, ctx->dout[i], dfs * C));
         if (j.lb && !lb_dev) RV_TRY(ensure(ctx, ctx->dlb[i], lbf * 2 * C));
     }
@@ -953,7 +958,20 @@ int chain_pipe(rv_ctx *ctx, const PipeJob &j, int n, int h, int w, const rv_para
         // input
         const uint8_t *di;
         size_t dip, difs;
-        if (in_dev) {
+        if (j.yuv) {
+            const uint8_t *src = j.in + (size_t)f0 * j.ipitch * h * 3 / 2;
+            size_t sp = j.ipitch;
+            if (!in_dev) {
+                uint8_t *y = (uint8_t *)ctx->dyuv[s].p;
+                if (j.ipitch == ypitch)
+                    CK(cudaMemcpyAsync(y, src, yfs * g, cudaMemcpyHostToDevice, st));
+                else
+                    CK(cudaMemcpy2DAsync(y, ypitch, src, j.ipitch, w, (size_t)h * 3 / 2 * g, cudaMemcpyHostToDevice, st));
+                src = y; sp = ypitch;
+            }
+            RV_TRY(launch_yuv420(ctx, j.yuv, src, sp, (uint8_t *)ctx->din[s].p, dpitch, dfs, g, h, w, st));
+            di = (const uint8_t *)ctx->din[s].p; dip = dpitch; difs = dfs;
+        } else if (in_dev) {
             di = j.in + (size_t)f0 * j.ipitch * h; dip = j.ipitch; difs = j.ipitch * h;
         } else {
             uint8_t *d = (uint8_t *)ctx->din[s].p;
@@ -1250,6 +1268,8 @@ void rv_destroy(rv_ctx *ctx)
             if (set[i].p) cudaFree(set[i].p);
     for (Buf &b : ctx->dlb)
         if (b.p) cudaFree(b.p);
+    for (Buf &b : ctx->dyuv)
+        if (b.p) cudaFree(b.p);
     for (Buf *b : {&ctx->u16.lut, &ctx->u16.mid, &ctx->u16.din, &ctx->u16.dout, &ctx->u16.mm, &ctx->u16.flags})
         if (b->p) cudaFree(b->p);
     if (ctx->u16.hflags) cudaFreeHost(ctx->u16.hflags);
@@ -1435,15 +1455,18 @@ int rv_submit(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h, int w,
     return chain_pipe(ctx, j, n, h, w, p);
 }
 
-int rv_submit_io(rv_ctx *ctx, const rv_io *io, int n, int h, int w, const rv_params *p)
+namespace {
+// rv_submit_io (BGR frames in) and rv_submit_io_yuv (yuv: 4:2:0 frames of `layout` in)
+int submit_io(rv_ctx *ctx, const rv_io *io, bool yuv, int layout, int n, int h, int w, const rv_params *p)
 {
-    if (!ctx) return RV_ERR_ARG;
     if (!io) return fail(ctx, RV_ERR_ARG, "null rv_io");
     if (!io->in) return fail(ctx, RV_ERR_ARG, "null frame pointer");
     if (!io->out && !io->tensor) return fail(ctx, RV_ERR_ARG, "neither a frame output nor a tensor output was given");
     RV_TRY(check_kind(ctx, io->in_kind));
-    // with no frame output the input stands in for it in the shape / pitch checks
-    RV_TRY(check_frames(ctx, io->in, io->out ? io->out : io->in, n, h, w, io->in_pitch, io->out ? io->out_pitch : io->in_pitch, 3));
+    if (yuv)
+        RV_TRY(check_yuv(ctx, io->in, io->out, n, h, w, io->in_pitch, io->out_pitch, layout));
+    else    // with no frame output the input stands in for it in the shape / pitch checks
+        RV_TRY(check_frames(ctx, io->in, io->out ? io->out : io->in, n, h, w, io->in_pitch, io->out ? io->out_pitch : io->in_pitch, 3));
     RV_TRY(check_params_u8(ctx, p));
     if (!p->clahe && p->ksize == 0) return fail(ctx, RV_ERR_ARG, "nothing to do (no CLAHE, no median)");
     if (io->out) {
@@ -1463,7 +1486,21 @@ int rv_submit_io(rv_ctx *ctx, const rv_io *io, int n, int h, int w, const rv_par
     j.lb = io->tensor; j.lb_kind = io->tensor_kind; j.S = io->tensor_size; j.pad = io->pad_value;
     j.lb_rows_only = (io->tensor_flags & RV_TENSOR_PADDING_PRESENT) != 0;
     j.processed = io->processed;
+    j.yuv = yuv ? layout : 0;
     return chain_pipe(ctx, j, n, h, w, p);
+}
+}  // namespace
+
+int rv_submit_io(rv_ctx *ctx, const rv_io *io, int n, int h, int w, const rv_params *p)
+{
+    if (!ctx) return RV_ERR_ARG;
+    return submit_io(ctx, io, false, 0, n, h, w, p);
+}
+
+int rv_submit_io_yuv(rv_ctx *ctx, const rv_io *io, int layout, int n, int h, int w, const rv_params *p)
+{
+    if (!ctx) return RV_ERR_ARG;
+    return submit_io(ctx, io, true, layout, n, h, w, p);
 }
 
 int rv_wait(rv_ctx *ctx) { return rv_sync(ctx); }

@@ -1,6 +1,6 @@
 /*
  * rv_internal.h -- the host toolkit shared by the translation units of librv_b200.so (rv_b200.cu, rv_fog.cu, rv_u16.cu,
- * rv_channels.cu): error
+ * rv_channels.cu, rv_yuv.cu): error
  * recording, device buffers, workspace ordering between streams, and the argument rules and CLAHE geometry that every entry must
  * apply alike.  What is not defined here is defined once, in rv_b200.cu, which owns the context.  Not part of the C ABI
  * (include/rv_b200.h).
@@ -37,7 +37,8 @@ struct U16Ws {
     bool attr_set = false;                      // k_u16_hist_lut's dynamic shared-memory limit is raised
 };
 
-// Workspaces of the 1- and 4-channel path (rv_channels.cu) of one context, used on whichever stream a call runs on.
+// Workspaces of the 1- and 4-channel path (rv_channels.cu) and of rv_yuv420_to_bgr's host path (rv_yuv.cu, din / dout) of one
+// context, used on whichever stream a call runs on.
 struct ChWs {
     Buf pack, din, dout, mm, flags;             // pack: BGR without alpha, the input of the 3-channel chains
     int32_t *hflags = nullptr;                  // page-locked copy of the gate decisions / gray min-max pairs
@@ -113,6 +114,12 @@ int chain_device(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h, int
 long group_frames_u16(const rv_params *p, int h, int w);
 int run_group_u16(rv_ctx *ctx, U16Ws &s, const uint16_t *din, size_t ip, size_t ifs, uint16_t *dout, size_t op, size_t ofs, int n,
                   int h, int w, const rv_params *p, cudaStream_t st, const int32_t **flags_out, bool copy_skipped = true);
+
+// rv_yuv.cu: the argument rules of 4:2:0 frames (in: 3h/2 rows of ipitch bytes per frame; out: BGR, nullptr = none), and the
+// conversion of n such frames at pitch sp into BGR frames at pitch dp, frame stride dfs, on `st`.
+int check_yuv(rv_ctx *ctx, const void *in, const void *out, int n, int h, int w, size_t ipitch, size_t opitch, int layout);
+int launch_yuv420(rv_ctx *ctx, int layout, const uint8_t *src, size_t sp, uint8_t *dst, size_t dp, size_t dfs, int n, int h, int w,
+                  cudaStream_t st);
 
 }  // namespace rv
 

@@ -10,7 +10,7 @@ from typing import Any, Dict
 
 import numpy as np
 
-from .._native import DeviceArray, Params, check_frame_params, check_u16_params, default_context
+from .._native import DeviceArray, Params, check_frame_params, check_u16_params, check_yuv_frames, default_context
 from .base import as_bgr_frame, as_frame
 from .ops import CLAHEDehaze, MedianDerain
 from .ops import clahe_dehaze as _clahe
@@ -149,9 +149,13 @@ class PreprocessPipeline:
         return out
 
     # -- new: batched multi-frame entry --------------------------------------------------
-    def process_batch(self, frames: np.ndarray, out: np.ndarray = None) -> np.ndarray:
+    def process_batch(self, frames: np.ndarray, out: np.ndarray = None, yuv: str = None) -> np.ndarray:
         """(B,H,W,3) uint8 -> (B,H,W,3) uint8; equals B per-frame calls bit for bit.  uint16 frames give uint16 results (cv2's
         16-bit chain: YCrCb only, median k 3 / 5, tile_grid <= 64).
+
+        `yuv="NV12"` / `"I420"`: `frames` are a decoder's (B,3H/2,W) uint8 4:2:0 frames; the result is exactly that of this call on
+        their cv2.cvtColor(COLOR_YUV2BGR_NV12 / _I420) conversion, (B,H,W,3) BGR.  The conversion runs on the GPU; with the stock
+        chain (one fused pass, with or without the gate) only the YUV bytes cross PCIe.
 
         `frames` / `out` may be pinned arrays from `Context.pinned_empty` (fastest: H2D, kernels
         and D2H of consecutive chunks overlap).  Frames the low-contrast gate skips are copied
@@ -159,6 +163,8 @@ class PreprocessPipeline:
         `__cuda_array_interface__`): nothing is copied back, which is what a detector on the same GPU wants
         (main_preview.py:99).
         """
+        if yuv is not None:
+            return self._process_batch_yuv(frames, out, yuv)
         if _is_cuda_tensor(frames):
             return self._process_batch_device(frames, out)
         if isinstance(out, str):
@@ -207,6 +213,56 @@ class PreprocessPipeline:
                     np.copyto(out, cur)
                     cur = out
         return cur
+
+    def _fused_segment(self):
+        """The single fused GPU pass the chain folds to (the stock config), or None."""
+        segs = self._segments() if (self.enabled and self.ops) else []
+        return segs[0] if len(segs) == 1 and isinstance(segs[0], Params) else None
+
+    def _device_ctx(self, frames):
+        return self._context if (self._context is not None and self._context.device == frames.device.index) \
+            else default_context(frames.device.index)
+
+    def _process_batch_yuv(self, frames, out, yuv):
+        """process_batch on (B,3H/2,W) 4:2:0 frames.  One fused pass: host frames go through rv_submit_io_yuv (the YUV bytes are
+        uploaded and converted in the pipeline's BGR workspace).  Anything else converts on the GPU first and takes the BGR path."""
+        if _is_cuda_tensor(frames):
+            import torch
+            _, b, h, w = check_yuv_frames(frames.shape, frames.dtype == torch.uint8, yuv)
+            if not frames.is_contiguous():
+                raise ValueError("frames must be a contiguous CUDA tensor")
+            # everything the device path would refuse is refused before the conversion is enqueued
+            self._check_device_chain()
+            if out is not None and not (_is_cuda_tensor(out) and out.dtype == torch.uint8 and tuple(out.shape) == (b, h, w, 3)
+                                        and out.device == frames.device and out.is_contiguous()):
+                raise ValueError(f"out must be a contiguous uint8 CUDA tensor of shape {(b, h, w, 3)} on the input's device")
+            return self._process_batch_device(self._device_ctx(frames).yuv420_to_bgr(frames, yuv), out)
+        if isinstance(out, str) and out != "device":
+            raise ValueError('out must be an array, None or "device"')
+        if not isinstance(frames, np.ndarray):
+            raise ValueError(f"yuv={yuv!r} takes a (B,3H/2,W) uint8 numpy array or torch CUDA tensor")
+        _, b, h, w = check_yuv_frames(frames.shape, frames.dtype == np.uint8, yuv)
+        shape = (b, h, w, 3)
+        if out is not None and not isinstance(out, str) and not (isinstance(out, np.ndarray) and out.shape == shape and
+                                                                 out.dtype == np.uint8 and out.flags.c_contiguous):
+            raise ValueError(f"out must be a C-contiguous uint8 array of shape {shape}")
+        ctx = self._ctx()
+        seg = self._fused_segment()
+        if seg is None:
+            bgr = ctx.yuv420_to_bgr(frames, yuv)
+            return self._process_batch_keep(bgr) if isinstance(out, str) else self.process_batch(bgr, out)
+        gate, thresh = self._gate()
+        if gate:
+            seg.gate_enable, seg.gate_thresh = 1, thresh
+        if isinstance(out, str):
+            res = DeviceArray(ctx, shape)
+        elif out is not None:
+            res = out
+        else:
+            res = ctx._pooled_pinned(shape) if b * h * w * 3 <= (64 << 20) else np.empty(shape, np.uint8)
+        ctx.submit_io(np.ascontiguousarray(frames), seg, out=res, yuv=yuv)
+        ctx.wait()
+        return res
 
     def _check_batch_channels(self, segs, dtype, channels):
         """_check_channels for a batch, which must have one result shape: with the gate, a CLAHE pass on BGRA frames would give
@@ -262,6 +318,16 @@ class PreprocessPipeline:
             cur = dst
         return cur
 
+    def _check_device_chain(self):
+        """What device-resident batches do not support -- the gate, foreign operators -- raises ValueError.  A disabled or empty
+        pipeline passes (its result is its input)."""
+        if not self.enabled or not self.ops:
+            return
+        if self._gate()[0]:
+            raise ValueError("the low-contrast gate is not supported for device-resident batches; use numpy frames")
+        if not all(isinstance(sg, Params) for sg in self._segments()):
+            raise ValueError("device-resident batches support only CLAHEDehaze / MedianDerain chains")
+
     def _process_batch_device(self, frames, out=None):
         """Device-resident batch: a contiguous torch CUDA uint8 / uint16 tensor (B,H,W,C), C = 1, 3 or 4, in, a tensor of the same
         kind out (3 channels after a CLAHE pass).  Work is enqueued on torch's current stream (no host synchronisation): use the
@@ -283,14 +349,10 @@ class PreprocessPipeline:
             raise ValueError(f"out must be a contiguous CUDA tensor of shape {final} and the input's dtype and device")
         if not self.enabled or not self.ops:
             return frames if out is None else out.copy_(frames)
-        if self._gate()[0]:
-            raise ValueError("the low-contrast gate is not supported for device-resident batches; use numpy frames")
-        ctx = self._context if (self._context is not None and self._context.device == frames.device.index) \
-            else default_context(frames.device.index)
+        self._check_device_chain()
+        ctx = self._device_ctx(frames)
         b, h, w, _ = frames.shape
         segs = self._segments()
-        if not all(isinstance(sg, Params) for sg in segs):
-            raise ValueError("device-resident batches support only CLAHEDehaze / MedianDerain chains")
         stream = torch.cuda.current_stream(frames.device).cuda_stream
         cur = frames
         for idx, sg in enumerate(segs):
@@ -319,7 +381,7 @@ class PreprocessPipeline:
 
     # -- new: chain fused with the detector-input stage (SURVEY.md 8f-1) ------------------------
     def process_batch_to_tensor(self, frames: np.ndarray, size: int = 640, pad_value: int = 114, want_frames: bool = False,
-                                out=None, padding_present: bool = False):
+                                out=None, padding_present: bool = False, yuv: str = None):
         """(B,H,W,3) uint8 -> ((B,3,size,size) float16 network input, processed frames or None).
 
         `out`: optional (B,3,size,size) float16 array for the tensor (pinned, from `Context.pinned_empty(shape, np.float16)`, for
@@ -332,7 +394,11 @@ class PreprocessPipeline:
         yolo_ultralytics.py:28-35: letterbox, BGR->RGB, HWC->CHW, /255, half).  When the chain is the stock
         CLAHEDehaze -> MedianDerain pair and the down-scale is an exact integer (1080p -> 640), the resize happens inside
         the chain kernel and the full-resolution frames are only written if `want_frames` is set.
+
+        `yuv="NV12"` / `"I420"`: `frames` are (B,3H/2,W) uint8 4:2:0 frames, as in process_batch; the processed frames are BGR.
         """
+        if yuv is not None:
+            return self._to_tensor_yuv(frames, size, pad_value, want_frames, out, padding_present, yuv)
         if isinstance(frames, np.ndarray) and frames.dtype == np.uint16:
             raise ValueError("process_batch_to_tensor takes uint8 frames: the detector input is built from 8-bit frames "
                              "(run process_batch on uint16 frames and convert them to 8 bits first)")
@@ -367,3 +433,30 @@ class PreprocessPipeline:
             return dev, full
         return ctx.chain_letterbox(frames, segs[0], size, pad_value, want_full=want_frames, out=out,
                                    padding_present=bool(padding_present and out is not None))
+
+    def _to_tensor_yuv(self, frames, size, pad_value, want_frames, out, padding_present, yuv):
+        """process_batch_to_tensor on (B,3H/2,W) 4:2:0 host frames: where the BGR call takes its fused path (one pass, no gate) the
+        frames go through rv_submit_io_yuv; otherwise they are converted on the GPU and take the BGR call."""
+        if not isinstance(frames, np.ndarray):
+            raise ValueError(f"yuv={yuv!r} takes a (B,3H/2,W) uint8 numpy array")
+        _, b, h, w = check_yuv_frames(frames.shape, frames.dtype == np.uint8, yuv)
+        keep = isinstance(out, str)
+        if keep and out != "device":
+            raise ValueError('out must be an array, None or "device"')
+        if out is not None and not keep and (out.shape != (b, 3, size, size) or out.dtype != np.float16 or not out.flags.c_contiguous):
+            raise ValueError("out must be a C-contiguous (B,3,size,size) float16 array")
+        ctx = self._ctx()
+        seg = self._fused_segment()
+        if seg is None or self._gate()[0]:
+            return self.process_batch_to_tensor(ctx.yuv420_to_bgr(frames, yuv), size, pad_value, want_frames, out, padding_present)
+        if keep:
+            t = DeviceArray(ctx, (b, 3, size, size), np.float16)
+        else:
+            t = np.empty((b, 3, size, size), np.float16) if out is None else out
+        full = None
+        if want_frames:
+            full = ctx._pooled_pinned((b, h, w, 3)) if b * h * w * 3 <= (64 << 20) else np.empty((b, h, w, 3), np.uint8)
+        ctx.submit_io(np.ascontiguousarray(frames), seg, out=full, tensor=t, size=size, pad_value=pad_value,
+                      padding_present=bool(padding_present and out is not None and not keep), yuv=yuv)
+        ctx.wait()
+        return t, full
