@@ -30,6 +30,10 @@
  *                      captured on the host goes in, the processed frames and / or the detector's input tensor
  *                      (main_preview.py:99 -> src/detect/yolo_ultralytics.py:28-35) come out on the host or stay on the GPU
  *   rv_submit_io_yuv   (new) rv_submit_io on NV12 / I420 frames: the YUV bytes cross PCIe and are converted to BGR on the GPU
+ *   rv_bgr_to_yuv420   (new) cv2.cvtColor(COLOR_BGR2YUV_I420) (NV12: its chroma planes interleaved), the host-side step a user runs on
+ *                      processed frames before handing them to a video encoder
+ *   rv_submit_io_fmt   (new) rv_submit_io with the input and the frame output each BGR, NV12 or I420: 4:2:0 results are converted on
+ *                      the GPU, so only their bytes cross PCIe on the way back
  *
  * Conventions: plain C types only; every function returns 0 on success or a negative rv_status;
  * rv_last_error(ctx) gives the message.  A context is bound to one CUDA device, owns its streams and
@@ -284,6 +288,22 @@ int rv_yuv420_to_bgr(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h,
  * converted into the BGR workspace, and the chain, gate, letterbox and result copies run exactly as for BGR input.  Results equal
  * rv_submit_io on the frames rv_yuv420_to_bgr gives. */
 int rv_submit_io_yuv(rv_ctx *ctx, const rv_io *io, int layout, int n, int h, int w, const rv_params *p);
+
+/* ---- BGR to YUV 4:2:0 for a video encoder (NVENC and GStreamer encoders take NV12; libavcodec / x264 `yuv420p` is I420), exactly as
+ * cv2.cvtColor(COLOR_BGR2YUV_I420) computes it: BT.601 video range, chroma from the top-left pixel of each 2 x 2 block.  NV12 is that
+ * result with its U and V planes interleaved (U first) in h/2 rows at the Y pitch.  Frame f of the output starts at
+ * f * out_pitch * h * 3 / 2.  RV_ERR_ARG for odd h or w, a bad layout, in_pitch < 3*w, out_pitch < w (I420: out_pitch != w), a null
+ * buffer and overlapping buffers.
+ * The conversion alone: host memory goes group by group and is synchronous; RV_MEM_DEVICE with a `stream` is asynchronous on that
+ * stream, without one synchronous on the context's stream. */
+int rv_bgr_to_yuv420(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h, int w, size_t in_pitch, size_t out_pitch, int layout,
+                     int mem_kind, void *stream);
+/* rv_submit_io with a layout for each side: in_layout / out_layout 0 (BGR), RV_YUV_NV12 or RV_YUV_I420.  A 4:2:0 io->in is read as
+ * rv_submit_io_yuv reads it; with a 4:2:0 out_layout io->out receives 4:2:0 frames and io->out_pitch is their row pitch: each
+ * chunk's BGR result is converted on the GPU (into a staging buffer that then goes D2H, or straight into a device io->out).  The
+ * gate, the tensor and the chunk schedule are those of the BGR job, and results equal rv_bgr_to_yuv420 of its frames.
+ * rv_submit_io is rv_submit_io_fmt(.., 0, 0, ..) and rv_submit_io_yuv rv_submit_io_fmt(.., layout, 0, ..). */
+int rv_submit_io_fmt(rv_ctx *ctx, const rv_io *io, int in_layout, int out_layout, int n, int h, int w, const rv_params *p);
 
 #ifdef __cplusplus
 }

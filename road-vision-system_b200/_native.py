@@ -216,6 +216,9 @@ EXPORTS = {
     "rv_yuv420_to_bgr": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_int, C.c_int,
                                    C.c_void_p]),
     "rv_submit_io_yuv": (C.c_int, [C.c_void_p, C.POINTER(IO), C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(Params)]),
+    "rv_bgr_to_yuv420": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_int, C.c_int,
+                                   C.c_void_p]),
+    "rv_submit_io_fmt": (C.c_int, [C.c_void_p, C.POINTER(IO), C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(Params)]),
 }
 
 
@@ -281,6 +284,31 @@ def check_yuv_frames(shape, is_uint8, yuv):
     if w % 2:
         raise ValueError(f"{yuv} frames need an even width, got {w}")
     return YUV_LAYOUTS[yuv], b, rows // 3 * 2, w
+
+
+def check_out_yuv(out_yuv):
+    """The enum rv_yuv value of a 4:2:0 output layout; ValueError for an unknown one."""
+    if out_yuv not in YUV_LAYOUTS:
+        raise ValueError(f"out_yuv must be None, 'NV12' or 'I420', got {out_yuv!r}")
+    return YUV_LAYOUTS[out_yuv]
+
+
+def check_bgr_for_yuv(shape, is_uint8, out_yuv):
+    """A (B,H,W,3) uint8 BGR batch to be returned as 4:2:0 frames (cv2.cvtColor(COLOR_BGR2YUV_I420) takes 8-bit BGR only): returns
+    (layout, B, H, W).  Raises ValueError for an unknown `out_yuv`, another rank, channel count or dtype, empty frames, and an odd H
+    or W (cv2 raises for both)."""
+    layout = check_out_yuv(out_yuv)
+    shape = tuple(int(v) for v in shape)
+    if len(shape) != 4 or shape[3] != 3:
+        raise ValueError(f"out_yuv={out_yuv!r} takes (B,H,W,3) BGR frames (no gray or BGRA ones), got shape {shape}")
+    if not is_uint8:
+        raise ValueError(f"out_yuv={out_yuv!r} takes uint8 frames (no 4:2:0 output of 16-bit frames)")
+    b, h, w, _ = shape
+    if h == 0 or w == 0:
+        raise ValueError(f"empty frames (shape {shape})")
+    if h % 2 or w % 2:
+        raise ValueError(f"4:2:0 output needs an even height and width, got {h}x{w}")
+    return layout, b, h, w
 
 
 U16_MAX_GRID = 64
@@ -542,6 +570,41 @@ class Context:
         self._ck(self._lib.rv_yuv420_to_bgr(self._h, frames.ctypes.data, out.ctypes.data, b, h, w, w, 3 * w, layout, kind, None))
         return out
 
+    def bgr_to_yuv420(self, frames, yuv, out=None):
+        """cv2.cvtColor(COLOR_BGR2YUV_I420) of every frame of a (B,H,W,3) uint8 batch -> (B,3H/2,W) 4:2:0 frames, on the GPU; with
+        yuv="NV12" the U and V planes come interleaved (U first) in H/2 rows, the layout video encoders take.  `frames`: a numpy array
+        (pageable or pinned; synchronous) or a contiguous torch CUDA tensor (asynchronous on torch's current stream; the result is a
+        tensor).  `out` (optional): an array / tensor of the result's shape to write into."""
+        if _is_torch(frames):
+            import torch
+            layout, b, h, w = check_bgr_for_yuv(frames.shape, frames.dtype == torch.uint8, yuv)
+            if not (frames.is_cuda and frames.is_contiguous()):
+                raise ValueError("device frames must be a contiguous CUDA tensor")
+            shape = (b, h * 3 // 2, w)
+            if out is None:
+                out = torch.empty(shape, dtype=torch.uint8, device=frames.device)
+            elif not (_is_torch(out) and out.dtype == torch.uint8 and tuple(out.shape) == shape and out.device == frames.device
+                      and out.is_contiguous()):
+                raise ValueError(f"out must be a contiguous uint8 CUDA tensor of shape {shape} on the input's device")
+            stream = torch.cuda.current_stream(frames.device).cuda_stream
+            if stream == 0:             # legacy default stream: run on the context's stream, synchronously
+                torch.cuda.current_stream(frames.device).synchronize()
+            self._ck(self._lib.rv_bgr_to_yuv420(self._h, C.c_void_p(frames.data_ptr()), C.c_void_p(out.data_ptr()), b, h, w, 3 * w, w,
+                                                layout, MEM_DEVICE, C.c_void_p(stream) if stream else None))
+            return out
+        if not isinstance(frames, np.ndarray):
+            raise ValueError("frames must be a numpy array or a torch CUDA tensor")
+        layout, b, h, w = check_bgr_for_yuv(frames.shape, frames.dtype == np.uint8, yuv)
+        frames = np.ascontiguousarray(frames)
+        shape = (b, h * 3 // 2, w)
+        if out is None:
+            out = np.empty(shape, np.uint8)
+        elif not (isinstance(out, np.ndarray) and out.shape == shape and out.dtype == np.uint8 and out.flags.c_contiguous):
+            raise ValueError(f"out must be a C-contiguous uint8 array of shape {shape}")
+        kind = MEM_PINNED if (self.mem_kind(frames) == MEM_PINNED and self.mem_kind(out) == MEM_PINNED) else MEM_HOST
+        self._ck(self._lib.rv_bgr_to_yuv420(self._h, frames.ctypes.data, out.ctypes.data, b, h, w, 3 * w, w, layout, kind, None))
+        return out
+
     def kernel_times(self, reset=False):
         """{name: (total_ms, launches)} for the hot-path kernels (needs set_option('kernel_timing', 1))."""
         res = {}
@@ -590,15 +653,20 @@ class Context:
         return tensor
 
     def submit_io(self, frames, params, shape=None, out=None, tensor=None, size=640, pad_value=114, processed=None, padding_present=False,
-                  yuv=None):
+                  yuv=None, out_yuv=None):
         """rv_submit_io: asynchronous job whose ends live independently on the host or on the GPU; call wait() afterwards.
 
         frames: (N,H,W,3) uint8 numpy array (pinned or pageable) or a device object / pointer (then pass shape=(N,H,W)).
         out:    frames result, numpy or device (DeviceArray / anything with __cuda_array_interface__ / int pointer), or None.
         tensor: (N,3,size,size) float16 detector input, numpy or device, or None.
         yuv:    "NV12" / "I420": `frames` are (N,3H/2,W) 4:2:0 frames (rv_submit_io_yuv; `shape` is still (N,H,W)), converted to BGR on
-                the GPU, so only their 1.5 bytes per pixel cross PCIe."""
+                the GPU, so only their 1.5 bytes per pixel cross PCIe.
+        out_yuv: "NV12" / "I420": `out` receives (N,3H/2,W) 4:2:0 frames (rv_submit_io_fmt), converted from the BGR result on the GPU,
+                so only their 1.5 bytes per pixel cross PCIe on the way back."""
         layout = 0
+        out_layout = check_out_yuv(out_yuv) if out_yuv is not None else 0
+        if out_layout and yuv is None and isinstance(frames, np.ndarray):
+            check_bgr_for_yuv(frames.shape, frames.dtype == np.uint8, out_yuv)
         if yuv is not None:
             if isinstance(frames, np.ndarray):
                 layout, n, h, w = check_yuv_frames(frames.shape, frames.dtype == np.uint8, yuv)
@@ -614,15 +682,12 @@ class Context:
         io.in_, io.in_kind = self._end(frames)
         io.in_pitch = w if layout else 3 * w
         io.out, io.out_kind = self._end(out)
-        io.out_pitch = 3 * w
+        io.out_pitch = w if out_layout else 3 * w
         io.tensor, io.tensor_kind = self._end(tensor)
         io.tensor_size, io.pad_value = int(size), int(pad_value)
         io.tensor_flags = 1 if padding_present else 0
         io.processed = processed.ctypes.data if processed is not None else None
-        if layout:
-            self._ck(self._lib.rv_submit_io_yuv(self._h, C.byref(io), layout, n, h, w, C.byref(params)))
-        else:
-            self._ck(self._lib.rv_submit_io(self._h, C.byref(io), n, h, w, C.byref(params)))
+        self._ck(self._lib.rv_submit_io_fmt(self._h, C.byref(io), layout, out_layout, n, h, w, C.byref(params)))
 
     # -- stage-level entry points (parity tests) ---------------------------------------------
     def luma_hist(self, frames, space, grid, want_luma=True, want_gray=False):

@@ -158,7 +158,8 @@ struct rv_ctx {
     Buf hist[NWS], quads[NWS], lut[NWS], flags[NWS], mm[NWS];
     Buf din[NWS], dout[NWS];
     Buf dlb[NPIPE];                         // detector tensors of the host pipeline's chunks
-    Buf dyuv[NPIPE];                        // 4:2:0 input chunks of the host pipeline (rv_submit_io_yuv), before the conversion
+    Buf dyuv[NPIPE];                        // 4:2:0 chunks of the host pipeline (rv_submit_io_fmt): input before its conversion,
+                                            // output after it (see chain_pipe)
     WsSync wsync[NWS];
     cudaStream_t fstream = nullptr;         // single-frame path (per-frame plugin contract): its own stream, workspace set and graphs
     std::vector<struct FrameGraph> fgraphs;
@@ -902,6 +903,7 @@ struct PipeJob {
     const uint8_t *in = nullptr; int in_kind = RV_MEM_HOST; size_t ipitch = 0;
     int yuv = 0;                            // RV_YUV_NV12 / RV_YUV_I420: 4:2:0 frames in, converted into the BGR workspace first; 0 = BGR
     uint8_t *out = nullptr; int out_kind = RV_MEM_HOST; size_t opitch = 0;      // full-resolution result; nullptr = not wanted
+    int yuv_out = 0;                        // RV_YUV_NV12 / RV_YUV_I420: `out` gets 4:2:0 frames, converted from the BGR result; 0 = BGR
     uint16_t *lb = nullptr; int lb_kind = RV_MEM_HOST; int S = 0, pad = 114;     // detector tensor; nullptr = none
     bool lb_rows_only = false;              // host tensor whose padding rows the caller already holds: copy back the image rows only
     int32_t *processed = nullptr;                                               // host, optional
@@ -935,12 +937,17 @@ int chain_pipe(rv_ctx *ctx, const PipeJob &j, int n, int h, int w, const rv_para
         lbf = (size_t)3 * j.S * j.S;
     }
     const bool fused = j.lb && lg.scale > 0;
-    const bool need_dfull = (j.out && !out_dev) || (j.lb && !fused && !(j.out && out_dev));   // a device staging copy of the full result
-    // 4:2:0 chunks are uploaded at a pitch that k_yuv420_to_bgr's vector path can read (I420 planes stay packed)
-    const size_t ypitch = j.yuv == RV_YUV_NV12 ? ((size_t)w + 7) & ~(size_t)7 : (size_t)w, yfs = ypitch * h * 3 / 2;
+    const bool out_direct = j.out && out_dev && !j.yuv_out;            // the chain writes the caller's device frames itself
+    const bool need_dfull = (j.out && !out_direct) || (j.lb && !fused && !out_direct);       // a device staging copy of the full result
+    // 4:2:0 chunks are staged at a pitch that the conversions' vector paths can use.  One dyuv[s] serves a chunk's input and its
+    // output: on stream s the input conversion reads it before the chain runs, the output conversion writes it after, and the next
+    // chunk on s uploads into it only after this chunk's D2H.
+    const size_t ypitch = yuv_stage_pitch(j.yuv, w), yfs = ypitch * h * 3 / 2;
+    const size_t opy = yuv_stage_pitch(j.yuv_out, w), ofy = opy * h * 3 / 2;
+    const size_t ystage = std::max(j.yuv && !in_dev ? yfs : 0, j.yuv_out && !out_dev ? ofy : 0);
     for (int i = 0; i < NPIPE; ++i) {
         if (!in_dev || j.yuv) RV_TRY(ensure(ctx, ctx->din[i], dfs * C));
-        if (j.yuv && !in_dev) RV_TRY(ensure(ctx, ctx->dyuv[i], yfs * C));
+        if (ystage) RV_TRY(ensure(ctx, ctx->dyuv[i], ystage * C));
         if (need_dfull) RV_TRY(ensure(ctx, ctx->dout[i], dfs * C));
         if (j.lb && !lb_dev) RV_TRY(ensure(ctx, ctx->dlb[i], lbf * 2 * C));
     }
@@ -984,7 +991,7 @@ int chain_pipe(rv_ctx *ctx, const PipeJob &j, int n, int h, int w, const rv_para
         // where the kernels write
         uint8_t *dfull = nullptr;
         size_t dop = dpitch, dofs = dfs;
-        if (j.out && out_dev) { dfull = j.out + (size_t)f0 * j.opitch * h; dop = j.opitch; dofs = j.opitch * h; }
+        if (out_direct) { dfull = j.out + (size_t)f0 * j.opitch * h; dop = j.opitch; dofs = j.opitch * h; }
         else if (need_dfull) dfull = (uint8_t *)ctx->dout[s].p;
         uint16_t *dl = nullptr;
         if (j.lb) dl = lb_dev ? j.lb + (size_t)f0 * lbf : (uint16_t *)ctx->dlb[s].p;
@@ -999,7 +1006,17 @@ int chain_pipe(rv_ctx *ctx, const PipeJob &j, int n, int h, int w, const rv_para
             if (j.lb) RV_TRY(launch_letterbox(ctx, dfull, dop, dofs, g, h, w, lg, j.pad, false, dl, st));
         }
         // results
-        if (j.out && !out_dev) {
+        if (j.yuv_out) {
+            uint8_t *dy = out_dev ? j.out + (size_t)f0 * j.opitch * h * 3 / 2 : (uint8_t *)ctx->dyuv[s].p;
+            RV_TRY(launch_bgr420(ctx, j.yuv_out, dfull, dpitch, dy, out_dev ? j.opitch : opy, g, h, w, st));
+            if (!out_dev) {
+                uint8_t *dst = j.out + (size_t)f0 * j.opitch * h * 3 / 2;
+                if (j.opitch == opy)
+                    CK(cudaMemcpyAsync(dst, dy, ofy * g, cudaMemcpyDeviceToHost, st));
+                else
+                    CK(cudaMemcpy2DAsync(dst, j.opitch, dy, opy, w, (size_t)h * 3 / 2 * g, cudaMemcpyDeviceToHost, st));
+            }
+        } else if (j.out && !out_dev) {
             if (j.opitch == dpitch)
                 CK(cudaMemcpyAsync(j.out + (size_t)f0 * j.opitch * h, dfull, dfs * g, cudaMemcpyDeviceToHost, st));
             else
@@ -1455,16 +1472,15 @@ int rv_submit(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h, int w,
     return chain_pipe(ctx, j, n, h, w, p);
 }
 
-namespace {
-// rv_submit_io (BGR frames in) and rv_submit_io_yuv (yuv: 4:2:0 frames of `layout` in)
-int submit_io(rv_ctx *ctx, const rv_io *io, bool yuv, int layout, int n, int h, int w, const rv_params *p)
+int rv_submit_io_fmt(rv_ctx *ctx, const rv_io *io, int in_layout, int out_layout, int n, int h, int w, const rv_params *p)
 {
+    if (!ctx) return RV_ERR_ARG;
     if (!io) return fail(ctx, RV_ERR_ARG, "null rv_io");
     if (!io->in) return fail(ctx, RV_ERR_ARG, "null frame pointer");
     if (!io->out && !io->tensor) return fail(ctx, RV_ERR_ARG, "neither a frame output nor a tensor output was given");
     RV_TRY(check_kind(ctx, io->in_kind));
-    if (yuv)
-        RV_TRY(check_yuv(ctx, io->in, io->out, n, h, w, io->in_pitch, io->out_pitch, layout));
+    if (in_layout || out_layout)
+        RV_TRY(check_yuv(ctx, io->in, io->out, n, h, w, io->in_pitch, io->out_pitch, in_layout, out_layout));
     else    // with no frame output the input stands in for it in the shape / pitch checks
         RV_TRY(check_frames(ctx, io->in, io->out ? io->out : io->in, n, h, w, io->in_pitch, io->out ? io->out_pitch : io->in_pitch, 3));
     RV_TRY(check_params_u8(ctx, p));
@@ -1486,21 +1502,21 @@ int submit_io(rv_ctx *ctx, const rv_io *io, bool yuv, int layout, int n, int h, 
     j.lb = io->tensor; j.lb_kind = io->tensor_kind; j.S = io->tensor_size; j.pad = io->pad_value;
     j.lb_rows_only = (io->tensor_flags & RV_TENSOR_PADDING_PRESENT) != 0;
     j.processed = io->processed;
-    j.yuv = yuv ? layout : 0;
+    j.yuv = in_layout;
+    j.yuv_out = io->out ? out_layout : 0;
     return chain_pipe(ctx, j, n, h, w, p);
 }
-}  // namespace
 
 int rv_submit_io(rv_ctx *ctx, const rv_io *io, int n, int h, int w, const rv_params *p)
 {
-    if (!ctx) return RV_ERR_ARG;
-    return submit_io(ctx, io, false, 0, n, h, w, p);
+    return rv_submit_io_fmt(ctx, io, 0, 0, n, h, w, p);
 }
 
 int rv_submit_io_yuv(rv_ctx *ctx, const rv_io *io, int layout, int n, int h, int w, const rv_params *p)
 {
     if (!ctx) return RV_ERR_ARG;
-    return submit_io(ctx, io, true, layout, n, h, w, p);
+    if (!layout) return fail(ctx, RV_ERR_ARG, "bad YUV layout 0");       // 0 would mean BGR frames to rv_submit_io_fmt
+    return rv_submit_io_fmt(ctx, io, layout, 0, n, h, w, p);
 }
 
 int rv_wait(rv_ctx *ctx) { return rv_sync(ctx); }

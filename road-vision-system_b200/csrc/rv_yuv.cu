@@ -137,17 +137,25 @@ constexpr size_t GROUP_BYTES = (size_t)1 << 30;     // BGR bytes of one frame gr
 
 }  // namespace
 
-int rv::check_yuv(rv_ctx *ctx, const void *in, const void *out, int n, int h, int w, size_t ipitch, size_t opitch, int layout)
+int rv::check_yuv(rv_ctx *ctx, const void *in, const void *out, int n, int h, int w, size_t ipitch, size_t opitch, int in_layout,
+                  int out_layout)
 {
     if (!ctx) return RV_ERR_ARG;
-    if (layout != RV_YUV_NV12 && layout != RV_YUV_I420) return fail(ctx, RV_ERR_ARG, "bad YUV layout %d", layout);
+    for (int layout : {in_layout, out_layout})
+        if (layout != 0 && layout != RV_YUV_NV12 && layout != RV_YUV_I420) return fail(ctx, RV_ERR_ARG, "bad YUV layout %d", layout);
+    if (!in_layout && !out_layout) return fail(ctx, RV_ERR_ARG, "bad YUV layout 0");
+    const int ib = in_layout ? 1 : 3, ob = out_layout ? 1 : 3;
     // without a frame output (a tensor-only job) the input stands in for it
-    RV_TRY(check_frames(ctx, in, out ? out : in, n, h, w, ipitch, out ? opitch : (size_t)3 * w, 1, 3, 1));
+    RV_TRY(check_frames(ctx, in, out ? out : in, n, h, w, ipitch, out ? opitch : (size_t)ob * w, ib, ob, 1));
     if (h < 2 || w < 2 || ((h | w) & 1))
         return fail(ctx, RV_ERR_ARG, "4:2:0 frames need an even height and width of at least 2, got %dx%d", w, h);
-    if (layout == RV_YUV_I420 && ipitch != (size_t)w) return fail(ctx, RV_ERR_ARG, "I420 frames need in_pitch == w (packed planes)");
+    if (in_layout == RV_YUV_I420 && ipitch != (size_t)w) return fail(ctx, RV_ERR_ARG, "I420 frames need in_pitch == w (packed planes)");
+    if (out && out_layout == RV_YUV_I420 && opitch != (size_t)w)
+        return fail(ctx, RV_ERR_ARG, "I420 frames need out_pitch == w (packed planes)");
     if (out && n > 0) {
-        const uintptr_t a0 = (uintptr_t)in, a1 = a0 + (size_t)n * ipitch * h * 3 / 2, b0 = (uintptr_t)out, b1 = b0 + (size_t)n * h * opitch;
+        // 4:2:0 frames are 3h/2 rows
+        const uintptr_t a0 = (uintptr_t)in, a1 = a0 + (size_t)n * ipitch * h * (in_layout ? 3 : 2) / 2;
+        const uintptr_t b0 = (uintptr_t)out, b1 = b0 + (size_t)n * opitch * h * (out_layout ? 3 : 2) / 2;
         if (a0 < b1 && b0 < a1) return fail(ctx, RV_ERR_ARG, "input and output ranges overlap");
     }
     return RV_OK;
@@ -178,7 +186,7 @@ int rv_yuv420_to_bgr(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h,
 {
     if (!ctx) return RV_ERR_ARG;
     if (!out) return fail(ctx, RV_ERR_ARG, "null frame pointer");      // check_yuv takes a null `out` for a tensor-only job
-    RV_TRY(check_yuv(ctx, in, out, n, h, w, in_pitch, out_pitch, layout));
+    RV_TRY(check_yuv(ctx, in, out, n, h, w, in_pitch, out_pitch, layout, 0));
     RV_TRY(check_kind(ctx, mem_kind));
     if (n == 0) return RV_OK;
     CK(cudaSetDevice(rv_internal_device(ctx)));
@@ -192,7 +200,7 @@ int rv_yuv420_to_bgr(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h,
     ChWs &c = rv_internal_ch(ctx);
     cudaStream_t st = (cudaStream_t)rv_internal_stream(ctx);
     RV_TRY(ws_acquire(ctx, c.sync, st));
-    const size_t yp = layout == RV_YUV_NV12 ? ((size_t)w + 7) & ~(size_t)7 : (size_t)w, yfs = yp * h * 3 / 2;
+    const size_t yp = yuv_stage_pitch(layout, w), yfs = yp * h * 3 / 2;
     const size_t rowb = (size_t)3 * w, bp = (rowb + 15) & ~(size_t)15, bfs = bp * h;
     const int G = (int)std::max<size_t>(1, std::min<size_t>(256, GROUP_BYTES / bfs));
     for (int f0 = 0; f0 < n; f0 += G) {

@@ -10,7 +10,8 @@ from typing import Any, Dict
 
 import numpy as np
 
-from .._native import DeviceArray, Params, check_frame_params, check_u16_params, check_yuv_frames, default_context
+from .._native import (MEM_DEVICE, DeviceArray, Params, check_bgr_for_yuv, check_frame_params, check_out_yuv, check_u16_params,
+                       check_yuv_frames, default_context)
 from .base import as_bgr_frame, as_frame
 from .ops import CLAHEDehaze, MedianDerain
 from .ops import clahe_dehaze as _clahe
@@ -149,7 +150,7 @@ class PreprocessPipeline:
         return out
 
     # -- new: batched multi-frame entry --------------------------------------------------
-    def process_batch(self, frames: np.ndarray, out: np.ndarray = None, yuv: str = None) -> np.ndarray:
+    def process_batch(self, frames: np.ndarray, out: np.ndarray = None, yuv: str = None, out_yuv: str = None) -> np.ndarray:
         """(B,H,W,3) uint8 -> (B,H,W,3) uint8; equals B per-frame calls bit for bit.  uint16 frames give uint16 results (cv2's
         16-bit chain: YCrCb only, median k 3 / 5, tile_grid <= 64).
 
@@ -157,12 +158,19 @@ class PreprocessPipeline:
         their cv2.cvtColor(COLOR_YUV2BGR_NV12 / _I420) conversion, (B,H,W,3) BGR.  The conversion runs on the GPU; with the stock
         chain (one fused pass, with or without the gate) only the YUV bytes cross PCIe.
 
+        `out_yuv="NV12"` / `"I420"` (8-bit BGR or `yuv=` frames): the result comes back as (B,3H/2,W) uint8 4:2:0 frames for a video
+        encoder, exactly cv2.cvtColor(COLOR_BGR2YUV_I420) of the BGR result this call returns without it (NV12: its U and V planes
+        interleaved, U first) -- frames the gate skips included, so a 4:2:0 frame that is not processed comes back re-encoded, not as
+        its input bytes.  The conversion runs on the GPU; with the stock chain only the 4:2:0 bytes cross PCIe on the way back.
+
         `frames` / `out` may be pinned arrays from `Context.pinned_empty` (fastest: H2D, kernels
         and D2H of consecutive chunks overlap).  Frames the low-contrast gate skips are copied
         through unchanged.  `out="device"` keeps the result on the GPU (a `DeviceArray`, usable from torch / cupy through
         `__cuda_array_interface__`): nothing is copied back, which is what a detector on the same GPU wants
         (main_preview.py:99).
         """
+        if out_yuv is not None:
+            return self._process_batch_yuv_out(frames, out, yuv, out_yuv)
         if yuv is not None:
             return self._process_batch_yuv(frames, out, yuv)
         if _is_cuda_tensor(frames):
@@ -261,6 +269,61 @@ class PreprocessPipeline:
         else:
             res = ctx._pooled_pinned(shape) if b * h * w * 3 <= (64 << 20) else np.empty(shape, np.uint8)
         ctx.submit_io(np.ascontiguousarray(frames), seg, out=res, yuv=yuv)
+        ctx.wait()
+        return res
+
+    def _process_batch_yuv_out(self, frames, out, yuv, out_yuv):
+        """process_batch with 4:2:0 results.  Host frames with the stock chain (one fused pass) go through rv_submit_io_fmt: each
+        chunk's BGR result is converted on the GPU and only the 4:2:0 bytes are copied back.  Anything else computes the BGR result as
+        process_batch does and converts it on the GPU.  Every refusal comes before a context is made or work is enqueued."""
+        check_out_yuv(out_yuv)
+        tensor = _is_cuda_tensor(frames)
+        if not tensor and not isinstance(frames, np.ndarray):
+            raise ValueError("frames must be a numpy array or a torch CUDA tensor")
+        if tensor:
+            import torch
+            u8 = frames.dtype == torch.uint8
+        else:
+            u8 = frames.dtype == np.uint8
+        if yuv is not None:
+            _, b, h, w = check_yuv_frames(frames.shape, u8, yuv)
+        else:
+            _, b, h, w = check_bgr_for_yuv(frames.shape, u8, out_yuv)
+        shape = (b, h * 3 // 2, w)
+        if tensor:
+            if not frames.is_contiguous():
+                raise ValueError("frames must be a contiguous CUDA tensor")
+            if out is not None and not (_is_cuda_tensor(out) and out.dtype == torch.uint8 and tuple(out.shape) == shape
+                                        and out.device == frames.device and out.is_contiguous()):
+                raise ValueError(f"out must be a contiguous uint8 CUDA tensor of shape {shape} on the input's device")
+            self._check_device_chain()
+            ctx = self._device_ctx(frames)
+            bgr = ctx.yuv420_to_bgr(frames, yuv) if yuv is not None else frames
+            return ctx.bgr_to_yuv420(self._process_batch_device(bgr), out_yuv, out=out)
+        if isinstance(out, str) and out != "device":
+            raise ValueError('out must be an array, None or "device"')
+        if out is not None and not isinstance(out, str) and not (isinstance(out, np.ndarray) and out.shape == shape and
+                                                                 out.dtype == np.uint8 and out.flags.c_contiguous):
+            raise ValueError(f"out must be a C-contiguous uint8 array of shape {shape}")
+        ctx = self._ctx()
+        seg = self._fused_segment()
+        if seg is None:
+            if isinstance(out, str):
+                bgr = self.process_batch(frames, out="device", yuv=yuv)
+                res = DeviceArray(ctx, shape)
+                ctx._ck(ctx._lib.rv_bgr_to_yuv420(ctx._h, bgr.ptr, res.ptr, b, h, w, 3 * w, w, check_out_yuv(out_yuv), MEM_DEVICE, None))
+                return res
+            return ctx.bgr_to_yuv420(self.process_batch(frames, yuv=yuv), out_yuv, out=out)
+        gate, thresh = self._gate()
+        if gate:
+            seg.gate_enable, seg.gate_thresh = 1, thresh
+        if isinstance(out, str):
+            res = DeviceArray(ctx, shape)
+        elif out is not None:
+            res = out
+        else:
+            res = ctx._pooled_pinned(shape) if b * h * w * 3 // 2 <= (64 << 20) else np.empty(shape, np.uint8)
+        ctx.submit_io(np.ascontiguousarray(frames), seg, out=res, yuv=yuv, out_yuv=out_yuv)
         ctx.wait()
         return res
 
