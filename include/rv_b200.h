@@ -34,6 +34,10 @@
  *                      processed frames before handing them to a video encoder
  *   rv_submit_io_fmt   (new) rv_submit_io with the input and the frame output each BGR, NV12 or I420: 4:2:0 results are converted on
  *                      the GPU, so only their bytes cross PCIe on the way back
+ *   rv_yuv422_to_bgr   (new) cv2.cvtColor(COLOR_YUV2BGR_YUY2 / COLOR_YUV2BGR_UYVY), the host-side step a user of the reference runs on
+ *                      a camera's packed 4:2:2 frames before pipeline(frame) (a UVC camera's YUYV, VideoSource(source=0),
+ *                      src/io_video/capture.py:11-16; UYVY from GMSL / FPD-Link serializers and SDI capture cards); rv_submit_io_fmt
+ *                      takes such frames as in_layout, so only their 2 bytes per pixel cross PCIe
  *
  * Conventions: plain C types only; every function returns 0 on success or a negative rv_status;
  * rv_last_error(ctx) gives the message.  A context is bound to one CUDA device, owns its streams and
@@ -298,12 +302,30 @@ int rv_submit_io_yuv(rv_ctx *ctx, const rv_io *io, int layout, int n, int h, int
  * stream, without one synchronous on the context's stream. */
 int rv_bgr_to_yuv420(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h, int w, size_t in_pitch, size_t out_pitch, int layout,
                      int mem_kind, void *stream);
-/* rv_submit_io with a layout for each side: in_layout / out_layout 0 (BGR), RV_YUV_NV12 or RV_YUV_I420.  A 4:2:0 io->in is read as
- * rv_submit_io_yuv reads it; with a 4:2:0 out_layout io->out receives 4:2:0 frames and io->out_pitch is their row pitch: each
- * chunk's BGR result is converted on the GPU (into a staging buffer that then goes D2H, or straight into a device io->out).  The
+/* rv_submit_io with a layout for each side: in_layout / out_layout 0 (BGR), RV_YUV_NV12 or RV_YUV_I420 (in_layout also RV_YUV_YUY2 /
+ * RV_YUV_UYVY, below).  A 4:2:0 io->in is read as rv_submit_io_yuv reads it; with a 4:2:0 out_layout io->out receives 4:2:0 frames
+ * and io->out_pitch is their row pitch: each chunk's BGR result is converted on the GPU (into a staging buffer that then goes D2H, or straight into a device io->out).  The
  * gate, the tensor and the chunk schedule are those of the BGR job, and results equal rv_bgr_to_yuv420 of its frames.
  * rv_submit_io is rv_submit_io_fmt(.., 0, 0, ..) and rv_submit_io_yuv rv_submit_io_fmt(.., layout, 0, ..). */
 int rv_submit_io_fmt(rv_ctx *ctx, const rv_io *io, int in_layout, int out_layout, int n, int h, int w, const rv_params *p);
+
+/* ---- packed YUV 4:2:2 camera frames (YUY2, which V4L2 calls YUYV: UVC / USB cameras; UYVY: GMSL / FPD-Link serializers, SDI capture
+ * cards), converted to BGR exactly as cv2.cvtColor(COLOR_YUV2BGR_YUY2 / COLOR_YUV2BGR_UYVY) does: the arithmetic of the 4:2:0
+ * conversion with one (U, V) pair per horizontal pixel pair (arithmetic in csrc/rv_yuv422.cu).  A frame is cv2's (h, w, 2) array:
+ * h rows of `in_pitch` bytes, each holding w/2 groups of 4 bytes, one per pixel pair:
+ *   RV_YUV_YUY2  Y0 U Y1 V
+ *   RV_YUV_UYVY  U Y0 V Y1
+ * Frame f starts at f * in_pitch * h.  w is even (cv2 raises for an odd one), h any.  A separate range from enum rv_yuv: the 4:2:0
+ * entries (rv_yuv420_to_bgr, rv_submit_io_yuv) refuse these values. */
+enum rv_yuv422 { RV_YUV_YUY2 = 16, RV_YUV_UYVY = 17 };
+/* The conversion alone into n BGR frames at out_pitch.  RV_ERR_ARG for odd or zero w, zero h, in_pitch < 2*w, out_pitch < 3*w, a null
+ * buffer, overlapping buffers and a layout that is not RV_YUV_YUY2 / RV_YUV_UYVY.  Host memory goes group by group and is synchronous;
+ * RV_MEM_DEVICE with a `stream` is asynchronous on that stream, without one synchronous on the context's stream.
+ * rv_submit_io_fmt also takes RV_YUV_YUY2 / RV_YUV_UYVY as in_layout, with any out_layout (a 4:2:0 out_layout still needs an even h):
+ * each chunk is uploaded as it is (or read in place on the device), converted into the BGR workspace, and the job goes on as a BGR
+ * job; results equal rv_submit_io_fmt on the frames rv_yuv422_to_bgr gives. */
+int rv_yuv422_to_bgr(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h, int w, size_t in_pitch, size_t out_pitch, int layout,
+                     int mem_kind, void *stream);
 
 #ifdef __cplusplus
 }

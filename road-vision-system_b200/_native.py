@@ -15,6 +15,7 @@ _SO = os.path.join(_CSRC, "librv_b200.so")
 SPACE_YCRCB, SPACE_LAB = 0, 1
 MEM_HOST, MEM_PINNED, MEM_DEVICE = 0, 1, 2
 YUV_LAYOUTS = {"NV12": 1, "I420": 2}        # enum rv_yuv
+YUV422_LAYOUTS = {"YUY2": 16, "UYVY": 17}   # enum rv_yuv422
 
 
 class RvError(RuntimeError):
@@ -219,6 +220,8 @@ EXPORTS = {
     "rv_bgr_to_yuv420": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_int, C.c_int,
                                    C.c_void_p]),
     "rv_submit_io_fmt": (C.c_int, [C.c_void_p, C.POINTER(IO), C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(Params)]),
+    "rv_yuv422_to_bgr": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_int, C.c_int,
+                                   C.c_void_p]),
 }
 
 
@@ -266,9 +269,12 @@ def _check_frames(frames, dtypes=_U8, channels=(3,)):
 def check_yuv_frames(shape, is_uint8, yuv):
     """A batch of YUV 4:2:0 frames in cv2's single-array form, (B, 3H/2, W) uint8, as cv2.cvtColor(COLOR_YUV2BGR_NV12 / _I420) takes
     them: returns (layout, B, H, W) of the BGR frames they convert to.  Raises ValueError for an unknown `yuv`, a wrong shape or dtype,
-    rows not divisible by 3 (H must be even), an odd W (cv2 raises for it) and empty frames."""
+    rows not divisible by 3 (H must be even), an odd W (cv2 raises for it) and empty frames.  A 4:2:2 `yuv` ("YUY2", "UYVY") takes
+    the rule of check_yuv422_frames instead, so that every entry with a `yuv=` argument checks its frames here."""
+    if yuv in YUV422_LAYOUTS:
+        return check_yuv422_frames(shape, is_uint8, yuv)
     if yuv not in YUV_LAYOUTS:
-        raise ValueError(f"yuv must be None, 'NV12' or 'I420', got {yuv!r}")
+        raise ValueError(f"yuv must be None, 'NV12', 'I420', 'YUY2' or 'UYVY', got {yuv!r}")
     shape = tuple(int(v) for v in shape)
     if len(shape) == 4:
         raise ValueError(f"yuv={yuv!r} takes (B,3H/2,W) frames, not (B,H,W,C) ones (got shape {shape})")
@@ -284,6 +290,28 @@ def check_yuv_frames(shape, is_uint8, yuv):
     if w % 2:
         raise ValueError(f"{yuv} frames need an even width, got {w}")
     return YUV_LAYOUTS[yuv], b, rows // 3 * 2, w
+
+
+def check_yuv422_frames(shape, is_uint8, yuv):
+    """A batch of packed YUV 4:2:2 camera frames, (B, H, W, 2) uint8, as cv2.cvtColor(COLOR_YUV2BGR_YUY2 / _UYVY) takes them (each row
+    holds W/2 groups of 4 bytes, one per pixel pair: YUY2 Y0 U Y1 V, UYVY U Y0 V Y1): returns (layout, B, H, W) of the BGR frames they
+    convert to.  Raises ValueError for a wrong shape, channel count or dtype, an odd W (cv2 raises for it) and empty frames."""
+    shape = tuple(int(v) for v in shape)
+    if len(shape) != 4 or shape[3] != 2:
+        raise ValueError(f"yuv={yuv!r} takes (B,H,W,2) uint8 frames, got shape {shape}")
+    if not is_uint8:
+        raise ValueError(f"yuv={yuv!r} takes uint8 frames")
+    b, h, w, _ = shape
+    if h == 0 or w == 0:
+        raise ValueError(f"empty {yuv} frames (shape {shape})")
+    if w % 2:
+        raise ValueError(f"{yuv} frames need an even width (one (U, V) pair per pixel pair), got {w}")
+    return YUV422_LAYOUTS[yuv], b, h, w
+
+
+def yuv_pitch(layout, w):
+    """Row pitch in bytes of contiguous YUV frames of `layout` (enum rv_yuv / rv_yuv422) and width w."""
+    return 2 * w if layout in YUV422_LAYOUTS.values() else w
 
 
 def check_out_yuv(out_yuv):
@@ -542,6 +570,21 @@ class Context:
         """cv2.cvtColor(COLOR_YUV2BGR_NV12 / _I420) of every frame of a (B,3H/2,W) uint8 batch -> (B,H,W,3) BGR, on the GPU.
         `frames`: a numpy array (pageable or pinned; synchronous) or a contiguous torch CUDA tensor (asynchronous on torch's current
         stream; the result is a tensor).  `out` (optional): an array / tensor of the result's shape to write into."""
+        if yuv in YUV422_LAYOUTS:
+            raise ValueError(f"yuv420_to_bgr takes 'NV12' or 'I420' frames; {yuv!r} frames go to yuv422_to_bgr")
+        return self._yuv_to_bgr(frames, yuv, out)
+
+    def yuv422_to_bgr(self, frames, yuv, out=None):
+        """cv2.cvtColor(COLOR_YUV2BGR_YUY2 / _UYVY) of every frame of a (B,H,W,2) uint8 batch of packed 4:2:2 camera frames ->
+        (B,H,W,3) BGR, on the GPU.  `frames`: a numpy array (pageable or pinned; synchronous) or a contiguous torch CUDA tensor
+        (asynchronous on torch's current stream; the result is a tensor).  `out` (optional): an array / tensor of the result's shape to
+        write into."""
+        if yuv not in YUV422_LAYOUTS:
+            raise ValueError(f"yuv422_to_bgr takes 'YUY2' or 'UYVY' frames, got {yuv!r}")
+        return self._yuv_to_bgr(frames, yuv, out)
+
+    def _yuv_to_bgr(self, frames, yuv, out=None):
+        """yuv420_to_bgr or yuv422_to_bgr, whichever `yuv` names (rv_yuv420_to_bgr / rv_yuv422_to_bgr)."""
         if _is_torch(frames):
             import torch
             layout, b, h, w = check_yuv_frames(frames.shape, frames.dtype == torch.uint8, yuv)
@@ -555,8 +598,8 @@ class Context:
             stream = torch.cuda.current_stream(frames.device).cuda_stream
             if stream == 0:             # legacy default stream: run on the context's stream, synchronously
                 torch.cuda.current_stream(frames.device).synchronize()
-            self._ck(self._lib.rv_yuv420_to_bgr(self._h, C.c_void_p(frames.data_ptr()), C.c_void_p(out.data_ptr()), b, h, w, w, 3 * w,
-                                                layout, MEM_DEVICE, C.c_void_p(stream) if stream else None))
+            self._ck(self._convert_fn(layout)(self._h, C.c_void_p(frames.data_ptr()), C.c_void_p(out.data_ptr()), b, h, w,
+                                              yuv_pitch(layout, w), 3 * w, layout, MEM_DEVICE, C.c_void_p(stream) if stream else None))
             return out
         if not isinstance(frames, np.ndarray):
             raise ValueError("frames must be a numpy array or a torch CUDA tensor")
@@ -567,8 +610,12 @@ class Context:
         elif not (isinstance(out, np.ndarray) and out.shape == (b, h, w, 3) and out.dtype == np.uint8 and out.flags.c_contiguous):
             raise ValueError(f"out must be a C-contiguous uint8 array of shape {(b, h, w, 3)}")
         kind = MEM_PINNED if (self.mem_kind(frames) == MEM_PINNED and self.mem_kind(out) == MEM_PINNED) else MEM_HOST
-        self._ck(self._lib.rv_yuv420_to_bgr(self._h, frames.ctypes.data, out.ctypes.data, b, h, w, w, 3 * w, layout, kind, None))
+        self._ck(self._convert_fn(layout)(self._h, frames.ctypes.data, out.ctypes.data, b, h, w, yuv_pitch(layout, w), 3 * w, layout,
+                                          kind, None))
         return out
+
+    def _convert_fn(self, layout):
+        return self._lib.rv_yuv422_to_bgr if layout in YUV422_LAYOUTS.values() else self._lib.rv_yuv420_to_bgr
 
     def bgr_to_yuv420(self, frames, yuv, out=None):
         """cv2.cvtColor(COLOR_BGR2YUV_I420) of every frame of a (B,H,W,3) uint8 batch -> (B,3H/2,W) 4:2:0 frames, on the GPU; with
@@ -660,7 +707,8 @@ class Context:
         out:    frames result, numpy or device (DeviceArray / anything with __cuda_array_interface__ / int pointer), or None.
         tensor: (N,3,size,size) float16 detector input, numpy or device, or None.
         yuv:    "NV12" / "I420": `frames` are (N,3H/2,W) 4:2:0 frames (rv_submit_io_yuv; `shape` is still (N,H,W)), converted to BGR on
-                the GPU, so only their 1.5 bytes per pixel cross PCIe.
+                the GPU, so only their 1.5 bytes per pixel cross PCIe.  "YUY2" / "UYVY": `frames` are (N,H,W,2) packed 4:2:2 frames
+                (rv_submit_io_fmt), so only their 2 bytes per pixel cross PCIe.
         out_yuv: "NV12" / "I420": `out` receives (N,3H/2,W) 4:2:0 frames (rv_submit_io_fmt), converted from the BGR result on the GPU,
                 so only their 1.5 bytes per pixel cross PCIe on the way back."""
         layout = 0
@@ -671,8 +719,8 @@ class Context:
             if isinstance(frames, np.ndarray):
                 layout, n, h, w = check_yuv_frames(frames.shape, frames.dtype == np.uint8, yuv)
             else:
-                layout = check_yuv_frames((shape[0], shape[1] * 3 // 2, shape[2]), True, yuv)[0]
                 n, h, w = shape
+                layout = check_yuv_frames((n, h, w, 2) if yuv in YUV422_LAYOUTS else (n, h * 3 // 2, w), True, yuv)[0]
         elif isinstance(frames, np.ndarray):
             _check_frames(frames)
             n, h, w, _ = frames.shape
@@ -680,7 +728,7 @@ class Context:
             n, h, w = shape
         io = IO()
         io.in_, io.in_kind = self._end(frames)
-        io.in_pitch = w if layout else 3 * w
+        io.in_pitch = yuv_pitch(layout, w) if layout else 3 * w
         io.out, io.out_kind = self._end(out)
         io.out_pitch = w if out_layout else 3 * w
         io.tensor, io.tensor_kind = self._end(tensor)

@@ -158,7 +158,7 @@ struct rv_ctx {
     Buf hist[NWS], quads[NWS], lut[NWS], flags[NWS], mm[NWS];
     Buf din[NWS], dout[NWS];
     Buf dlb[NPIPE];                         // detector tensors of the host pipeline's chunks
-    Buf dyuv[NPIPE];                        // 4:2:0 chunks of the host pipeline (rv_submit_io_fmt): input before its conversion,
+    Buf dyuv[NPIPE];                        // YUV chunks of the host pipeline (rv_submit_io_fmt): input before its conversion,
                                             // output after it (see chain_pipe)
     WsSync wsync[NWS];
     cudaStream_t fstream = nullptr;         // single-frame path (per-frame plugin contract): its own stream, workspace set and graphs
@@ -901,7 +901,8 @@ int launch_letterbox(rv_ctx *ctx, const uint8_t *src, size_t pitch, size_t fstri
 // H2D, a device output / tensor skips its D2H (results that the next stage consumes on the same GPU never cross PCIe).
 struct PipeJob {
     const uint8_t *in = nullptr; int in_kind = RV_MEM_HOST; size_t ipitch = 0;
-    int yuv = 0;                            // RV_YUV_NV12 / RV_YUV_I420: 4:2:0 frames in, converted into the BGR workspace first; 0 = BGR
+    int yuv = 0;                            // RV_YUV_NV12 / RV_YUV_I420 / RV_YUV_YUY2 / RV_YUV_UYVY: 4:2:0 or 4:2:2 frames in, converted
+                                            // into the BGR workspace first; 0 = BGR
     uint8_t *out = nullptr; int out_kind = RV_MEM_HOST; size_t opitch = 0;      // full-resolution result; nullptr = not wanted
     int yuv_out = 0;                        // RV_YUV_NV12 / RV_YUV_I420: `out` gets 4:2:0 frames, converted from the BGR result; 0 = BGR
     uint16_t *lb = nullptr; int lb_kind = RV_MEM_HOST; int S = 0, pad = 114;     // detector tensor; nullptr = none
@@ -939,10 +940,10 @@ int chain_pipe(rv_ctx *ctx, const PipeJob &j, int n, int h, int w, const rv_para
     const bool fused = j.lb && lg.scale > 0;
     const bool out_direct = j.out && out_dev && !j.yuv_out;            // the chain writes the caller's device frames itself
     const bool need_dfull = (j.out && !out_direct) || (j.lb && !fused && !out_direct);       // a device staging copy of the full result
-    // 4:2:0 chunks are staged at a pitch that the conversions' vector paths can use.  One dyuv[s] serves a chunk's input and its
+    // YUV chunks are staged at a pitch that the conversions' vector paths can use.  One dyuv[s] serves a chunk's input and its
     // output: on stream s the input conversion reads it before the chain runs, the output conversion writes it after, and the next
     // chunk on s uploads into it only after this chunk's D2H.
-    const size_t ypitch = yuv_stage_pitch(j.yuv, w), yfs = ypitch * h * 3 / 2;
+    const size_t yrows = frame_rows(j.yuv, h), ypitch = yuv_stage_pitch(j.yuv, w), yfs = ypitch * yrows;
     const size_t opy = yuv_stage_pitch(j.yuv_out, w), ofy = opy * h * 3 / 2;
     const size_t ystage = std::max(j.yuv && !in_dev ? yfs : 0, j.yuv_out && !out_dev ? ofy : 0);
     for (int i = 0; i < NPIPE; ++i) {
@@ -966,17 +967,18 @@ int chain_pipe(rv_ctx *ctx, const PipeJob &j, int n, int h, int w, const rv_para
         const uint8_t *di;
         size_t dip, difs;
         if (j.yuv) {
-            const uint8_t *src = j.in + (size_t)f0 * j.ipitch * h * 3 / 2;
+            const uint8_t *src = j.in + (size_t)f0 * j.ipitch * yrows;
             size_t sp = j.ipitch;
             if (!in_dev) {
                 uint8_t *y = (uint8_t *)ctx->dyuv[s].p;
                 if (j.ipitch == ypitch)
                     CK(cudaMemcpyAsync(y, src, yfs * g, cudaMemcpyHostToDevice, st));
                 else
-                    CK(cudaMemcpy2DAsync(y, ypitch, src, j.ipitch, w, (size_t)h * 3 / 2 * g, cudaMemcpyHostToDevice, st));
+                    CK(cudaMemcpy2DAsync(y, ypitch, src, j.ipitch, yuv_row_bytes(j.yuv, w), yrows * g, cudaMemcpyHostToDevice, st));
                 src = y; sp = ypitch;
             }
-            RV_TRY(launch_yuv420(ctx, j.yuv, src, sp, (uint8_t *)ctx->din[s].p, dpitch, dfs, g, h, w, st));
+            if (is_yuv422(j.yuv)) RV_TRY(launch_yuv422(ctx, j.yuv, src, sp, (uint8_t *)ctx->din[s].p, dpitch, dfs, g, h, w, st));
+            else RV_TRY(launch_yuv420(ctx, j.yuv, src, sp, (uint8_t *)ctx->din[s].p, dpitch, dfs, g, h, w, st));
             di = (const uint8_t *)ctx->din[s].p; dip = dpitch; difs = dfs;
         } else if (in_dev) {
             di = j.in + (size_t)f0 * j.ipitch * h; dip = j.ipitch; difs = j.ipitch * h;
@@ -1515,7 +1517,8 @@ int rv_submit_io(rv_ctx *ctx, const rv_io *io, int n, int h, int w, const rv_par
 int rv_submit_io_yuv(rv_ctx *ctx, const rv_io *io, int layout, int n, int h, int w, const rv_params *p)
 {
     if (!ctx) return RV_ERR_ARG;
-    if (!layout) return fail(ctx, RV_ERR_ARG, "bad YUV layout 0");       // 0 would mean BGR frames to rv_submit_io_fmt
+    // 0 would mean BGR frames to rv_submit_io_fmt; 4:2:2 frames are not this entry's
+    if (!is_yuv420(layout)) return fail(ctx, RV_ERR_ARG, "bad YUV layout %d", layout);
     return rv_submit_io_fmt(ctx, io, layout, 0, n, h, w, p);
 }
 

@@ -1,6 +1,6 @@
 /*
  * rv_internal.h -- the host toolkit shared by the translation units of librv_b200.so (rv_b200.cu, rv_fog.cu, rv_u16.cu,
- * rv_channels.cu, rv_yuv.cu, rv_yuv_out.cu): error
+ * rv_channels.cu, rv_yuv.cu, rv_yuv422.cu, rv_yuv_out.cu): error
  * recording, device buffers, workspace ordering between streams, and the argument rules and CLAHE geometry that every entry must
  * apply alike.  What is not defined here is defined once, in rv_b200.cu, which owns the context.  Not part of the C ABI
  * (include/rv_b200.h).
@@ -37,8 +37,9 @@ struct U16Ws {
     bool attr_set = false;                      // k_u16_hist_lut's dynamic shared-memory limit is raised
 };
 
-// Workspaces of the 1- and 4-channel path (rv_channels.cu) and of the host paths of rv_yuv420_to_bgr (rv_yuv.cu) and
-// rv_bgr_to_yuv420 (rv_yuv_out.cu) (din / dout) of one context, used on whichever stream a call runs on.
+// Workspaces of the 1- and 4-channel path (rv_channels.cu) and of the host paths of rv_yuv420_to_bgr (rv_yuv.cu),
+// rv_yuv422_to_bgr (rv_yuv422.cu) and rv_bgr_to_yuv420 (rv_yuv_out.cu) (din / dout) of one context, used on whichever stream a call
+// runs on.
 struct ChWs {
     Buf pack, din, dout, mm, flags;             // pack: BGR without alpha, the input of the 3-channel chains
     int32_t *hflags = nullptr;                  // page-locked copy of the gate decisions / gray min-max pairs
@@ -115,17 +116,30 @@ long group_frames_u16(const rv_params *p, int h, int w);
 int run_group_u16(rv_ctx *ctx, U16Ws &s, const uint16_t *din, size_t ip, size_t ifs, uint16_t *dout, size_t op, size_t ofs, int n,
                   int h, int w, const rv_params *p, cudaStream_t st, const int32_t **flags_out, bool copy_skipped = true);
 
-// rv_yuv.cu: the argument rules of a job with 4:2:0 frames on either side (in_layout / out_layout: RV_YUV_NV12, RV_YUV_I420, or 0
-// for BGR, not both 0; a 4:2:0 frame is 3h/2 rows of its pitch; out: nullptr = none) and the conversion of n 4:2:0 frames at pitch
-// sp into BGR frames at pitch dp, frame stride dfs, on `st`.  rv_yuv_out.cu: the conversion of n BGR frames at pitch sp (frame
-// stride sp * h) into 4:2:0 frames at pitch dp, on `st`.
+inline bool is_yuv420(int layout) { return layout == RV_YUV_NV12 || layout == RV_YUV_I420; }
+inline bool is_yuv422(int layout) { return layout == RV_YUV_YUY2 || layout == RV_YUV_UYVY; }
+
+// rv_yuv.cu: the argument rules of a job with YUV frames on either side (in_layout: RV_YUV_NV12, RV_YUV_I420, RV_YUV_YUY2,
+// RV_YUV_UYVY or 0 for BGR; out_layout: RV_YUV_NV12, RV_YUV_I420 or 0; not both 0; out: nullptr = none) and the conversion of n
+// 4:2:0 frames at pitch sp into BGR frames at pitch dp, frame stride dfs, on `st`.  rv_yuv422.cu: the same conversion of n 4:2:2
+// frames.  rv_yuv_out.cu: the conversion of n BGR frames at pitch sp (frame stride sp * h) into 4:2:0 frames at pitch dp, on `st`.
 int check_yuv(rv_ctx *ctx, const void *in, const void *out, int n, int h, int w, size_t ipitch, size_t opitch, int in_layout,
               int out_layout);
 int launch_yuv420(rv_ctx *ctx, int layout, const uint8_t *src, size_t sp, uint8_t *dst, size_t dp, size_t dfs, int n, int h, int w,
                   cudaStream_t st);
+int launch_yuv422(rv_ctx *ctx, int layout, const uint8_t *src, size_t sp, uint8_t *dst, size_t dp, size_t dfs, int n, int h, int w,
+                  cudaStream_t st);
 int launch_bgr420(rv_ctx *ctx, int layout, const uint8_t *src, size_t sp, uint8_t *dst, size_t dp, int n, int h, int w, cudaStream_t st);
-// the row pitch of 4:2:0 frames staged on the device: one that the conversions' vector paths can use (I420 planes stay packed)
-inline size_t yuv_stage_pitch(int layout, int w) { return layout == RV_YUV_NV12 ? ((size_t)w + 7) & ~(size_t)7 : (size_t)w; }
+// rows of one frame of `layout` (0: BGR): 4:2:0 frames are 3h/2 rows of their pitch, BGR and 4:2:2 frames h rows
+inline size_t frame_rows(int layout, int h) { return is_yuv420(layout) ? (size_t)h * 3 / 2 : (size_t)h; }
+// bytes of one row of a YUV frame of `layout`: w for 4:2:0 planes, 2w for 4:2:2 pixel pairs
+inline size_t yuv_row_bytes(int layout, int w) { return (size_t)(is_yuv422(layout) ? 2 : 1) * w; }
+// the row pitch of YUV frames staged on the device: one that the conversions' vector paths can use (I420 planes stay packed)
+inline size_t yuv_stage_pitch(int layout, int w)
+{
+    if (is_yuv422(layout)) return ((size_t)2 * w + 15) & ~(size_t)15;
+    return layout == RV_YUV_NV12 ? ((size_t)w + 7) & ~(size_t)7 : (size_t)w;
+}
 
 }  // namespace rv
 

@@ -4,7 +4,7 @@
  * produce I420.  Taking those frames as they are halves the bytes a host-fed batch moves over PCIe (1.5 bytes per pixel against 3)
  * and spares the host its own colour conversion.
  *
- * What cv2 computes (ITU-R BT.601 video range, 20-bit fixed point; every term fits in int32):
+ * What cv2 computes (ITU-R BT.601 video range, 20-bit fixed point; every term fits in int32; rv_yuv_px.cuh, shared with rv_yuv422.cu):
  *   u = U - 128, v = V - 128, one (U, V) pair per 2 x 2 block of Y
  *   ruv = 2^19 + CVR v,  guv = 2^19 + CVG v + CUG u,  buv = 2^19 + CUB u,  y = max(0, Y - 16) CY
  *   B, G, R = sat_u8((y + buv) >> 20), sat_u8((y + guv) >> 20), sat_u8((y + ruv) >> 20)
@@ -25,42 +25,14 @@
 #include <algorithm>
 
 #include "rv_internal.h"
+#include "rv_yuv_px.cuh"
 
 using namespace rv;
+using namespace rv::yuv;
 
 namespace {
 
-constexpr int CY = 1220542, CUB = 2116026, CUG = -409993, CVG = -852492, CVR = 1673527, HALF = 1 << 19;
-
-__device__ __forceinline__ uint32_t sat8(int v) { return (uint32_t)min(max(v >> 20, 0), 255); }
-
-// the B, G, R bytes of one pixel from its Y and its block's chroma terms
-__device__ __forceinline__ void bgr_px(int Y, int buv, int guv, int ruv, uint32_t *b)
-{
-    const int y = max(0, Y - 16) * CY;
-    b[0] = sat8(y + buv);
-    b[1] = sat8(y + guv);
-    b[2] = sat8(y + ruv);
-}
-
-__device__ __forceinline__ void chroma_terms(int U, int V, int &buv, int &guv, int &ruv)
-{
-    const int u = U - 128, v = V - 128;
-    buv = HALF + CUB * u;
-    guv = HALF + CVG * v + CUG * u;
-    ruv = HALF + CVR * v;
-}
-
 __device__ __forceinline__ int byte_of(uint2 v, int k) { return (int)(((k < 4 ? v.x : v.y) >> (8 * (k & 3))) & 0xFFu); }
-
-__device__ __forceinline__ void store24(uint8_t *d, const uint32_t (&b)[24])
-{
-    uint32_t o[6];
-    #pragma unroll
-    for (int i = 0; i < 6; ++i) o[i] = b[4 * i] | (b[4 * i + 1] << 8) | (b[4 * i + 2] << 16) | (b[4 * i + 3] << 24);
-    #pragma unroll
-    for (int i = 0; i < 3; ++i) reinterpret_cast<uint2 *>(d)[i] = make_uint2(o[2 * i], o[2 * i + 1]);
-}
 
 // the 2 x 2 block whose left column is x, one byte at a time (da / db: the block's two output rows)
 template <int LAYOUT>
@@ -141,21 +113,21 @@ int rv::check_yuv(rv_ctx *ctx, const void *in, const void *out, int n, int h, in
                   int out_layout)
 {
     if (!ctx) return RV_ERR_ARG;
-    for (int layout : {in_layout, out_layout})
-        if (layout != 0 && layout != RV_YUV_NV12 && layout != RV_YUV_I420) return fail(ctx, RV_ERR_ARG, "bad YUV layout %d", layout);
+    if (in_layout != 0 && !is_yuv420(in_layout) && !is_yuv422(in_layout)) return fail(ctx, RV_ERR_ARG, "bad YUV layout %d", in_layout);
+    if (out_layout != 0 && !is_yuv420(out_layout)) return fail(ctx, RV_ERR_ARG, "bad YUV layout %d", out_layout);
     if (!in_layout && !out_layout) return fail(ctx, RV_ERR_ARG, "bad YUV layout 0");
-    const int ib = in_layout ? 1 : 3, ob = out_layout ? 1 : 3;
+    const int ib = !in_layout ? 3 : is_yuv422(in_layout) ? 2 : 1, ob = out_layout ? 1 : 3;
     // without a frame output (a tensor-only job) the input stands in for it
     RV_TRY(check_frames(ctx, in, out ? out : in, n, h, w, ipitch, out ? opitch : (size_t)ob * w, ib, ob, 1));
-    if (h < 2 || w < 2 || ((h | w) & 1))
+    if ((is_yuv420(in_layout) || out_layout) && (h < 2 || w < 2 || ((h | w) & 1)))
         return fail(ctx, RV_ERR_ARG, "4:2:0 frames need an even height and width of at least 2, got %dx%d", w, h);
+    if (is_yuv422(in_layout) && (w & 1)) return fail(ctx, RV_ERR_ARG, "4:2:2 frames need an even width, got %d", w);
     if (in_layout == RV_YUV_I420 && ipitch != (size_t)w) return fail(ctx, RV_ERR_ARG, "I420 frames need in_pitch == w (packed planes)");
     if (out && out_layout == RV_YUV_I420 && opitch != (size_t)w)
         return fail(ctx, RV_ERR_ARG, "I420 frames need out_pitch == w (packed planes)");
     if (out && n > 0) {
-        // 4:2:0 frames are 3h/2 rows
-        const uintptr_t a0 = (uintptr_t)in, a1 = a0 + (size_t)n * ipitch * h * (in_layout ? 3 : 2) / 2;
-        const uintptr_t b0 = (uintptr_t)out, b1 = b0 + (size_t)n * opitch * h * (out_layout ? 3 : 2) / 2;
+        const uintptr_t a0 = (uintptr_t)in, a1 = a0 + (size_t)n * ipitch * frame_rows(in_layout, h);
+        const uintptr_t b0 = (uintptr_t)out, b1 = b0 + (size_t)n * opitch * frame_rows(out_layout, h);
         if (a0 < b1 && b0 < a1) return fail(ctx, RV_ERR_ARG, "input and output ranges overlap");
     }
     return RV_OK;
@@ -186,6 +158,7 @@ int rv_yuv420_to_bgr(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h,
 {
     if (!ctx) return RV_ERR_ARG;
     if (!out) return fail(ctx, RV_ERR_ARG, "null frame pointer");      // check_yuv takes a null `out` for a tensor-only job
+    if (is_yuv422(layout)) return fail(ctx, RV_ERR_ARG, "bad YUV layout %d (4:2:2 frames: rv_yuv422_to_bgr)", layout);
     RV_TRY(check_yuv(ctx, in, out, n, h, w, in_pitch, out_pitch, layout, 0));
     RV_TRY(check_kind(ctx, mem_kind));
     if (n == 0) return RV_OK;

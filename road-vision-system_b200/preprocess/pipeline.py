@@ -158,6 +158,11 @@ class PreprocessPipeline:
         their cv2.cvtColor(COLOR_YUV2BGR_NV12 / _I420) conversion, (B,H,W,3) BGR.  The conversion runs on the GPU; with the stock
         chain (one fused pass, with or without the gate) only the YUV bytes cross PCIe.
 
+        `yuv="YUY2"` / `"UYVY"`: `frames` are a camera's (B,H,W,2) uint8 packed 4:2:2 frames (the array cv2.cvtColor takes; each row
+        holds W/2 groups of 4 bytes, one per pixel pair: YUY2 Y0 U Y1 V, UYVY U Y0 V Y1); the result is exactly that of this call on
+        their cv2.cvtColor(COLOR_YUV2BGR_YUY2 / _UYVY) conversion.  W must be even, H may be odd.  Routed as the 4:2:0 input is: with
+        the stock chain only their 2 bytes per pixel cross PCIe.
+
         `out_yuv="NV12"` / `"I420"` (8-bit BGR or `yuv=` frames): the result comes back as (B,3H/2,W) uint8 4:2:0 frames for a video
         encoder, exactly cv2.cvtColor(COLOR_BGR2YUV_I420) of the BGR result this call returns without it (NV12: its U and V planes
         interleaved, U first) -- frames the gate skips included, so a 4:2:0 frame that is not processed comes back re-encoded, not as
@@ -232,8 +237,9 @@ class PreprocessPipeline:
             else default_context(frames.device.index)
 
     def _process_batch_yuv(self, frames, out, yuv):
-        """process_batch on (B,3H/2,W) 4:2:0 frames.  One fused pass: host frames go through rv_submit_io_yuv (the YUV bytes are
-        uploaded and converted in the pipeline's BGR workspace).  Anything else converts on the GPU first and takes the BGR path."""
+        """process_batch on (B,3H/2,W) 4:2:0 or (B,H,W,2) 4:2:2 frames.  One fused pass: host frames go through rv_submit_io_fmt (the
+        YUV bytes are uploaded and converted in the pipeline's BGR workspace).  Anything else converts on the GPU first and takes the
+        BGR path."""
         if _is_cuda_tensor(frames):
             import torch
             _, b, h, w = check_yuv_frames(frames.shape, frames.dtype == torch.uint8, yuv)
@@ -244,11 +250,11 @@ class PreprocessPipeline:
             if out is not None and not (_is_cuda_tensor(out) and out.dtype == torch.uint8 and tuple(out.shape) == (b, h, w, 3)
                                         and out.device == frames.device and out.is_contiguous()):
                 raise ValueError(f"out must be a contiguous uint8 CUDA tensor of shape {(b, h, w, 3)} on the input's device")
-            return self._process_batch_device(self._device_ctx(frames).yuv420_to_bgr(frames, yuv), out)
+            return self._process_batch_device(self._device_ctx(frames)._yuv_to_bgr(frames, yuv), out)
         if isinstance(out, str) and out != "device":
             raise ValueError('out must be an array, None or "device"')
         if not isinstance(frames, np.ndarray):
-            raise ValueError(f"yuv={yuv!r} takes a (B,3H/2,W) uint8 numpy array or torch CUDA tensor")
+            raise ValueError(f"yuv={yuv!r} takes a uint8 numpy array or torch CUDA tensor")
         _, b, h, w = check_yuv_frames(frames.shape, frames.dtype == np.uint8, yuv)
         shape = (b, h, w, 3)
         if out is not None and not isinstance(out, str) and not (isinstance(out, np.ndarray) and out.shape == shape and
@@ -257,7 +263,7 @@ class PreprocessPipeline:
         ctx = self._ctx()
         seg = self._fused_segment()
         if seg is None:
-            bgr = ctx.yuv420_to_bgr(frames, yuv)
+            bgr = ctx._yuv_to_bgr(frames, yuv)
             return self._process_batch_keep(bgr) if isinstance(out, str) else self.process_batch(bgr, out)
         gate, thresh = self._gate()
         if gate:
@@ -287,6 +293,8 @@ class PreprocessPipeline:
             u8 = frames.dtype == np.uint8
         if yuv is not None:
             _, b, h, w = check_yuv_frames(frames.shape, u8, yuv)
+            if h % 2:           # (4:2:2 frames may have an odd height)
+                raise ValueError(f"4:2:0 output needs an even height and width, got {h}x{w}")
         else:
             _, b, h, w = check_bgr_for_yuv(frames.shape, u8, out_yuv)
         shape = (b, h * 3 // 2, w)
@@ -298,7 +306,7 @@ class PreprocessPipeline:
                 raise ValueError(f"out must be a contiguous uint8 CUDA tensor of shape {shape} on the input's device")
             self._check_device_chain()
             ctx = self._device_ctx(frames)
-            bgr = ctx.yuv420_to_bgr(frames, yuv) if yuv is not None else frames
+            bgr = ctx._yuv_to_bgr(frames, yuv) if yuv is not None else frames
             return ctx.bgr_to_yuv420(self._process_batch_device(bgr), out_yuv, out=out)
         if isinstance(out, str) and out != "device":
             raise ValueError('out must be an array, None or "device"')
@@ -458,7 +466,8 @@ class PreprocessPipeline:
         CLAHEDehaze -> MedianDerain pair and the down-scale is an exact integer (1080p -> 640), the resize happens inside
         the chain kernel and the full-resolution frames are only written if `want_frames` is set.
 
-        `yuv="NV12"` / `"I420"`: `frames` are (B,3H/2,W) uint8 4:2:0 frames, as in process_batch; the processed frames are BGR.
+        `yuv="NV12"` / `"I420"` / `"YUY2"` / `"UYVY"`: `frames` are (B,3H/2,W) uint8 4:2:0 or (B,H,W,2) uint8 4:2:2 frames, as in
+        process_batch; the processed frames are BGR.
         """
         if yuv is not None:
             return self._to_tensor_yuv(frames, size, pad_value, want_frames, out, padding_present, yuv)
@@ -498,10 +507,10 @@ class PreprocessPipeline:
                                    padding_present=bool(padding_present and out is not None))
 
     def _to_tensor_yuv(self, frames, size, pad_value, want_frames, out, padding_present, yuv):
-        """process_batch_to_tensor on (B,3H/2,W) 4:2:0 host frames: where the BGR call takes its fused path (one pass, no gate) the
-        frames go through rv_submit_io_yuv; otherwise they are converted on the GPU and take the BGR call."""
+        """process_batch_to_tensor on (B,3H/2,W) 4:2:0 or (B,H,W,2) 4:2:2 host frames: where the BGR call takes its fused path (one
+        pass, no gate) the frames go through rv_submit_io_fmt; otherwise they are converted on the GPU and take the BGR call."""
         if not isinstance(frames, np.ndarray):
-            raise ValueError(f"yuv={yuv!r} takes a (B,3H/2,W) uint8 numpy array")
+            raise ValueError(f"yuv={yuv!r} takes a uint8 numpy array")
         _, b, h, w = check_yuv_frames(frames.shape, frames.dtype == np.uint8, yuv)
         keep = isinstance(out, str)
         if keep and out != "device":
@@ -511,7 +520,7 @@ class PreprocessPipeline:
         ctx = self._ctx()
         seg = self._fused_segment()
         if seg is None or self._gate()[0]:
-            return self.process_batch_to_tensor(ctx.yuv420_to_bgr(frames, yuv), size, pad_value, want_frames, out, padding_present)
+            return self.process_batch_to_tensor(ctx._yuv_to_bgr(frames, yuv), size, pad_value, want_frames, out, padding_present)
         if keep:
             t = DeviceArray(ctx, (b, 3, size, size), np.float16)
         else:
