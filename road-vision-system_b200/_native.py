@@ -248,6 +248,23 @@ def _is_torch(x):
     return type(x).__module__.startswith("torch")
 
 
+def _torch_stream(device):
+    """torch's current stream on `device` as a cudaStream_t int for the C entries, or None on the legacy default stream: torch's
+    queued work is then waited for, and the call runs on the context's stream, synchronously."""
+    import torch
+    stream = torch.cuda.current_stream(device)
+    if stream.cuda_stream == 0:
+        stream.synchronize()
+    return stream.cuda_stream or None
+
+
+def _check_torch_out(out, shape, dtype, device, msg):
+    """A caller's `out` tensor (None: none given) must be contiguous, of `shape` and `dtype`, on `device`; ValueError(msg) if not."""
+    if out is not None and not (_is_torch(out) and out.dtype == dtype and tuple(out.shape) == tuple(shape) and out.device == device
+                                and out.is_contiguous()):
+        raise ValueError(msg)
+
+
 _U8 = (np.dtype(np.uint8),)
 _U8_U16 = (np.dtype(np.uint8), np.dtype(np.uint16))
 CHANNELS = (1, 3, 4)        # gray, BGR, BGRA / BGRx
@@ -469,6 +486,10 @@ class Context:
         self._last_lease_addr = blk[0]
         return lease.view(np.ndarray)
 
+    def _host_result(self, shape):
+        """A new uint8 host array for a result: pooled page-locked memory (the D2H copy is a plain DMA) up to 64 MB, pageable above."""
+        return self._pooled_pinned(shape) if int(np.prod(shape)) <= (64 << 20) else np.empty(shape, np.uint8)
+
     def _device_block(self, nbytes):
         """Device memory for a DeviceArray; blocks are recycled per size (cudaMalloc / cudaFree cost milliseconds and
         synchronise the device, which a per-batch allocation must not pay)."""
@@ -572,7 +593,7 @@ class Context:
         stream; the result is a tensor).  `out` (optional): an array / tensor of the result's shape to write into."""
         if yuv in YUV422_LAYOUTS:
             raise ValueError(f"yuv420_to_bgr takes 'NV12' or 'I420' frames; {yuv!r} frames go to yuv422_to_bgr")
-        return self._yuv_to_bgr(frames, yuv, out)
+        return self._convert(frames, yuv, None, out)
 
     def yuv422_to_bgr(self, frames, yuv, out=None):
         """cv2.cvtColor(COLOR_YUV2BGR_YUY2 / _UYVY) of every frame of a (B,H,W,2) uint8 batch of packed 4:2:2 camera frames ->
@@ -581,75 +602,53 @@ class Context:
         write into."""
         if yuv not in YUV422_LAYOUTS:
             raise ValueError(f"yuv422_to_bgr takes 'YUY2' or 'UYVY' frames, got {yuv!r}")
-        return self._yuv_to_bgr(frames, yuv, out)
-
-    def _yuv_to_bgr(self, frames, yuv, out=None):
-        """yuv420_to_bgr or yuv422_to_bgr, whichever `yuv` names (rv_yuv420_to_bgr / rv_yuv422_to_bgr)."""
-        if _is_torch(frames):
-            import torch
-            layout, b, h, w = check_yuv_frames(frames.shape, frames.dtype == torch.uint8, yuv)
-            if not (frames.is_cuda and frames.is_contiguous()):
-                raise ValueError("device frames must be a contiguous CUDA tensor")
-            if out is None:
-                out = torch.empty((b, h, w, 3), dtype=torch.uint8, device=frames.device)
-            elif not (_is_torch(out) and out.dtype == torch.uint8 and tuple(out.shape) == (b, h, w, 3) and out.device == frames.device
-                      and out.is_contiguous()):
-                raise ValueError(f"out must be a contiguous uint8 CUDA tensor of shape {(b, h, w, 3)} on the input's device")
-            stream = torch.cuda.current_stream(frames.device).cuda_stream
-            if stream == 0:             # legacy default stream: run on the context's stream, synchronously
-                torch.cuda.current_stream(frames.device).synchronize()
-            self._ck(self._convert_fn(layout)(self._h, C.c_void_p(frames.data_ptr()), C.c_void_p(out.data_ptr()), b, h, w,
-                                              yuv_pitch(layout, w), 3 * w, layout, MEM_DEVICE, C.c_void_p(stream) if stream else None))
-            return out
-        if not isinstance(frames, np.ndarray):
-            raise ValueError("frames must be a numpy array or a torch CUDA tensor")
-        layout, b, h, w = check_yuv_frames(frames.shape, frames.dtype == np.uint8, yuv)
-        frames = np.ascontiguousarray(frames)
-        if out is None:
-            out = np.empty((b, h, w, 3), np.uint8)
-        elif not (isinstance(out, np.ndarray) and out.shape == (b, h, w, 3) and out.dtype == np.uint8 and out.flags.c_contiguous):
-            raise ValueError(f"out must be a C-contiguous uint8 array of shape {(b, h, w, 3)}")
-        kind = MEM_PINNED if (self.mem_kind(frames) == MEM_PINNED and self.mem_kind(out) == MEM_PINNED) else MEM_HOST
-        self._ck(self._convert_fn(layout)(self._h, frames.ctypes.data, out.ctypes.data, b, h, w, yuv_pitch(layout, w), 3 * w, layout,
-                                          kind, None))
-        return out
-
-    def _convert_fn(self, layout):
-        return self._lib.rv_yuv422_to_bgr if layout in YUV422_LAYOUTS.values() else self._lib.rv_yuv420_to_bgr
+        return self._convert(frames, yuv, None, out)
 
     def bgr_to_yuv420(self, frames, yuv, out=None):
         """cv2.cvtColor(COLOR_BGR2YUV_I420) of every frame of a (B,H,W,3) uint8 batch -> (B,3H/2,W) 4:2:0 frames, on the GPU; with
         yuv="NV12" the U and V planes come interleaved (U first) in H/2 rows, the layout video encoders take.  `frames`: a numpy array
-        (pageable or pinned; synchronous) or a contiguous torch CUDA tensor (asynchronous on torch's current stream; the result is a
-        tensor).  `out` (optional): an array / tensor of the result's shape to write into."""
-        if _is_torch(frames):
+        (pageable or pinned; synchronous), a contiguous torch CUDA tensor (asynchronous on torch's current stream; the result is a
+        tensor) or a DeviceArray (synchronous; the result is a DeviceArray).  `out` (optional): an array / tensor / DeviceArray of the
+        result's shape to write into."""
+        return self._convert(frames, None, yuv, out)
+
+    def _convert(self, frames, in_layout, out_layout, out=None):
+        """The conversion of every frame of a batch from `in_layout` ("NV12", "I420", "YUY2", "UYVY") to BGR, or from BGR to
+        `out_layout` ("NV12", "I420"); the other layout is None.  `frames`: a numpy array (synchronous), a contiguous torch CUDA tensor
+        (asynchronous on torch's current stream) or a DeviceArray (synchronous); the result is of the same kind, `out` if given."""
+        torch_in = _is_torch(frames)
+        if torch_in:
             import torch
-            layout, b, h, w = check_bgr_for_yuv(frames.shape, frames.dtype == torch.uint8, yuv)
+            u8 = frames.dtype == torch.uint8
+        elif isinstance(frames, (np.ndarray, DeviceArray)):
+            u8 = frames.dtype == np.uint8
+        else:
+            raise ValueError("frames must be a numpy array or a torch CUDA tensor")
+        if in_layout is not None:
+            layout, b, h, w = check_yuv_frames(frames.shape, u8, in_layout)
+            shape, pitches = (b, h, w, 3), (yuv_pitch(layout, w), 3 * w)
+            fn = self._lib.rv_yuv422_to_bgr if in_layout in YUV422_LAYOUTS else self._lib.rv_yuv420_to_bgr
+        else:
+            layout, b, h, w = check_bgr_for_yuv(frames.shape, u8, out_layout)
+            shape, pitches, fn = (b, h * 3 // 2, w), (3 * w, w), self._lib.rv_bgr_to_yuv420
+        if torch_in:
             if not (frames.is_cuda and frames.is_contiguous()):
                 raise ValueError("device frames must be a contiguous CUDA tensor")
-            shape = (b, h * 3 // 2, w)
-            if out is None:
-                out = torch.empty(shape, dtype=torch.uint8, device=frames.device)
-            elif not (_is_torch(out) and out.dtype == torch.uint8 and tuple(out.shape) == shape and out.device == frames.device
-                      and out.is_contiguous()):
-                raise ValueError(f"out must be a contiguous uint8 CUDA tensor of shape {shape} on the input's device")
-            stream = torch.cuda.current_stream(frames.device).cuda_stream
-            if stream == 0:             # legacy default stream: run on the context's stream, synchronously
-                torch.cuda.current_stream(frames.device).synchronize()
-            self._ck(self._lib.rv_bgr_to_yuv420(self._h, C.c_void_p(frames.data_ptr()), C.c_void_p(out.data_ptr()), b, h, w, 3 * w, w,
-                                                layout, MEM_DEVICE, C.c_void_p(stream) if stream else None))
+            _check_torch_out(out, shape, torch.uint8, frames.device,
+                             f"out must be a contiguous uint8 CUDA tensor of shape {shape} on the input's device")
+            out = torch.empty(shape, dtype=torch.uint8, device=frames.device) if out is None else out
+            self._ck(fn(self._h, C.c_void_p(frames.data_ptr()), C.c_void_p(out.data_ptr()), b, h, w, *pitches, layout, MEM_DEVICE,
+                        _torch_stream(frames.device)))
             return out
-        if not isinstance(frames, np.ndarray):
-            raise ValueError("frames must be a numpy array or a torch CUDA tensor")
-        layout, b, h, w = check_bgr_for_yuv(frames.shape, frames.dtype == np.uint8, yuv)
-        frames = np.ascontiguousarray(frames)
-        shape = (b, h * 3 // 2, w)
+        dev = isinstance(frames, DeviceArray)
+        frames = frames if dev else np.ascontiguousarray(frames)
         if out is None:
-            out = np.empty(shape, np.uint8)
-        elif not (isinstance(out, np.ndarray) and out.shape == shape and out.dtype == np.uint8 and out.flags.c_contiguous):
+            out = DeviceArray(self, shape) if dev else np.empty(shape, np.uint8)
+        elif not (isinstance(out, DeviceArray if dev else np.ndarray) and out.shape == shape and out.dtype == np.uint8
+                  and (dev or out.flags.c_contiguous)):
             raise ValueError(f"out must be a C-contiguous uint8 array of shape {shape}")
-        kind = MEM_PINNED if (self.mem_kind(frames) == MEM_PINNED and self.mem_kind(out) == MEM_PINNED) else MEM_HOST
-        self._ck(self._lib.rv_bgr_to_yuv420(self._h, frames.ctypes.data, out.ctypes.data, b, h, w, 3 * w, w, layout, kind, None))
+        (src, kind), (dst, out_kind) = self._end(frames), self._end(out)
+        self._ck(fn(self._h, src, dst, b, h, w, *pitches, layout, kind if kind == out_kind else MEM_HOST, None))
         return out
 
     def kernel_times(self, reset=False):
@@ -792,7 +791,7 @@ class Context:
             frames = np.ascontiguousarray(frames)
             full = None
             if want_full:
-                full = self._pooled_pinned(frames.shape) if frames.nbytes <= (64 << 20) else np.empty_like(frames)
+                full = self._host_result(frames.shape)
             self.submit_io(frames, params, out=full, tensor=out, size=size, pad_value=pad_value, padding_present=True)
             self.wait()
             return out, full
@@ -803,7 +802,7 @@ class Context:
             out = np.empty((n, 3, size, size), np.float16)
         full = None
         if want_full:
-            full = self._pooled_pinned(frames.shape) if frames.nbytes <= (64 << 20) else np.empty_like(frames)
+            full = self._host_result(frames.shape)
         kind = MEM_PINNED if (self.mem_kind(frames) == MEM_PINNED and self.mem_kind(out) == MEM_PINNED and
                               (full is None or self.mem_kind(full) == MEM_PINNED)) else MEM_HOST
         self._ck(self._lib.rv_chain_letterbox_f16(self._h, frames.ctypes.data, n, h, w, 3 * w, C.byref(params), out.ctypes.data,

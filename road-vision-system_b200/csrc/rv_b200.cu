@@ -694,8 +694,7 @@ long auto_group(const rv_ctx *ctx, int h, int w)
     if (ctx->group_frames > 0) return ctx->group_frames;
     // The chain is instruction-bound, not DRAM-bound (profiles/), so a group is as large as the
     // workspaces comfortably allow: three launches per batch, no tail effects between small groups.
-    const size_t fb = (size_t)3 * w * h;
-    return std::max<long>(1, std::min<long>(256, (long)(((size_t)1 << 30) / fb)));
+    return group_frames((size_t)3 * w * h);
 }
 
 long auto_chunk(const rv_ctx *ctx, int h, int w)
@@ -927,9 +926,7 @@ long chunk_frames_at(long C, bool taper, long n, int chunk, long left)
 int chain_pipe(rv_ctx *ctx, const PipeJob &j, int n, int h, int w, const rv_params *p)
 {
     const long C = std::min<long>(std::min<long>(auto_chunk(ctx, h, w), std::max(1, n)), 4096);
-    const size_t rowb = (size_t)3 * w;
-    const size_t dpitch = (rowb + 15) & ~(size_t)15;
-    const size_t dfs = dpitch * h;
+    const size_t dpitch = stage_pitch(0, w), dfs = dpitch * h;
     const bool in_dev = j.in_kind == RV_MEM_DEVICE, out_dev = j.out_kind == RV_MEM_DEVICE, lb_dev = j.lb_kind == RV_MEM_DEVICE;
     LbGeo lg = {};
     size_t lbf = 0;                                         // halves per frame of the detector tensor
@@ -943,8 +940,8 @@ int chain_pipe(rv_ctx *ctx, const PipeJob &j, int n, int h, int w, const rv_para
     // YUV chunks are staged at a pitch that the conversions' vector paths can use.  One dyuv[s] serves a chunk's input and its
     // output: on stream s the input conversion reads it before the chain runs, the output conversion writes it after, and the next
     // chunk on s uploads into it only after this chunk's D2H.
-    const size_t yrows = frame_rows(j.yuv, h), ypitch = yuv_stage_pitch(j.yuv, w), yfs = ypitch * yrows;
-    const size_t opy = yuv_stage_pitch(j.yuv_out, w), ofy = opy * h * 3 / 2;
+    const size_t yrows = frame_rows(j.yuv, h), ypitch = stage_pitch(j.yuv, w), yfs = ypitch * yrows;
+    const size_t orows = frame_rows(j.yuv_out, h), opy = stage_pitch(j.yuv_out, w), ofy = opy * orows;
     const size_t ystage = std::max(j.yuv && !in_dev ? yfs : 0, j.yuv_out && !out_dev ? ofy : 0);
     for (int i = 0; i < NPIPE; ++i) {
         if (!in_dev || j.yuv) RV_TRY(ensure(ctx, ctx->din[i], dfs * C));
@@ -971,23 +968,17 @@ int chain_pipe(rv_ctx *ctx, const PipeJob &j, int n, int h, int w, const rv_para
             size_t sp = j.ipitch;
             if (!in_dev) {
                 uint8_t *y = (uint8_t *)ctx->dyuv[s].p;
-                if (j.ipitch == ypitch)
-                    CK(cudaMemcpyAsync(y, src, yfs * g, cudaMemcpyHostToDevice, st));
-                else
-                    CK(cudaMemcpy2DAsync(y, ypitch, src, j.ipitch, yuv_row_bytes(j.yuv, w), yrows * g, cudaMemcpyHostToDevice, st));
+                RV_TRY(copy_rows(ctx, y, ypitch, src, j.ipitch, row_bytes(j.yuv, w), yrows * g, cudaMemcpyHostToDevice, st));
                 src = y; sp = ypitch;
             }
-            if (is_yuv422(j.yuv)) RV_TRY(launch_yuv422(ctx, j.yuv, src, sp, (uint8_t *)ctx->din[s].p, dpitch, dfs, g, h, w, st));
-            else RV_TRY(launch_yuv420(ctx, j.yuv, src, sp, (uint8_t *)ctx->din[s].p, dpitch, dfs, g, h, w, st));
+            RV_TRY(launch_convert(ctx, j.yuv, 0, src, sp, (uint8_t *)ctx->din[s].p, dpitch, g, h, w, st));
             di = (const uint8_t *)ctx->din[s].p; dip = dpitch; difs = dfs;
         } else if (in_dev) {
             di = j.in + (size_t)f0 * j.ipitch * h; dip = j.ipitch; difs = j.ipitch * h;
         } else {
             uint8_t *d = (uint8_t *)ctx->din[s].p;
-            if (j.ipitch == dpitch)
-                CK(cudaMemcpyAsync(d, j.in + (size_t)f0 * j.ipitch * h, dfs * g, cudaMemcpyHostToDevice, st));
-            else
-                CK(cudaMemcpy2DAsync(d, dpitch, j.in + (size_t)f0 * j.ipitch * h, j.ipitch, rowb, (size_t)h * g, cudaMemcpyHostToDevice, st));
+            RV_TRY(copy_rows(ctx, d, dpitch, j.in + (size_t)f0 * j.ipitch * h, j.ipitch, row_bytes(0, w), (size_t)h * g,
+                             cudaMemcpyHostToDevice, st));
             di = d; dip = dpitch; difs = dfs;
         }
         // where the kernels write
@@ -1009,20 +1000,13 @@ int chain_pipe(rv_ctx *ctx, const PipeJob &j, int n, int h, int w, const rv_para
         }
         // results
         if (j.yuv_out) {
-            uint8_t *dy = out_dev ? j.out + (size_t)f0 * j.opitch * h * 3 / 2 : (uint8_t *)ctx->dyuv[s].p;
-            RV_TRY(launch_bgr420(ctx, j.yuv_out, dfull, dpitch, dy, out_dev ? j.opitch : opy, g, h, w, st));
-            if (!out_dev) {
-                uint8_t *dst = j.out + (size_t)f0 * j.opitch * h * 3 / 2;
-                if (j.opitch == opy)
-                    CK(cudaMemcpyAsync(dst, dy, ofy * g, cudaMemcpyDeviceToHost, st));
-                else
-                    CK(cudaMemcpy2DAsync(dst, j.opitch, dy, opy, w, (size_t)h * 3 / 2 * g, cudaMemcpyDeviceToHost, st));
-            }
+            uint8_t *dst = j.out + (size_t)f0 * j.opitch * orows, *dy = out_dev ? dst : (uint8_t *)ctx->dyuv[s].p;
+            RV_TRY(launch_convert(ctx, 0, j.yuv_out, dfull, dpitch, dy, out_dev ? j.opitch : opy, g, h, w, st));
+            if (!out_dev)
+                RV_TRY(copy_rows(ctx, dst, j.opitch, dy, opy, row_bytes(j.yuv_out, w), orows * g, cudaMemcpyDeviceToHost, st));
         } else if (j.out && !out_dev) {
-            if (j.opitch == dpitch)
-                CK(cudaMemcpyAsync(j.out + (size_t)f0 * j.opitch * h, dfull, dfs * g, cudaMemcpyDeviceToHost, st));
-            else
-                CK(cudaMemcpy2DAsync(j.out + (size_t)f0 * j.opitch * h, j.opitch, dfull, dpitch, rowb, (size_t)h * g, cudaMemcpyDeviceToHost, st));
+            RV_TRY(copy_rows(ctx, j.out + (size_t)f0 * j.opitch * h, j.opitch, dfull, dpitch, row_bytes(0, w), (size_t)h * g,
+                             cudaMemcpyDeviceToHost, st));
         }
         if (j.lb && !lb_dev) {
             if (j.lb_rows_only && lg.nh < j.S) {

@@ -62,8 +62,6 @@ using namespace rv;
 
 namespace {
 
-constexpr size_t GROUP_BYTES = (size_t)1 << 30;     // input bytes of one frame group, as the 3-channel paths
-
 template <typename T> struct Word;                  // one 4-sample pixel as one load
 template <> struct Word<uint8_t> { using type = uint32_t; };
 template <> struct Word<uint16_t> { using type = uint2; };
@@ -223,7 +221,7 @@ k_ch_median(const uint8_t *__restrict__ src, size_t spitch, size_t sfstride, uin
 }
 
 // ------------------------------------------------------------------------------------------------ host side
-// Every launch covers one frame group (group_of: at most 256 frames), so frames always fit on gridDim.z in one launch.
+// Every launch covers one frame group (group_frames: at most 256 frames), so frames always fit on gridDim.z in one launch.
 template <typename T>
 int launch_strip(rv_ctx *ctx, const uint8_t *src, size_t sp, size_t sfs, uint8_t *dst, size_t dp, size_t dfs, int n, int h, int w,
                  cudaStream_t st)
@@ -300,8 +298,6 @@ int check_depth(rv_ctx *ctx, int bits, int channels)
     return RV_OK;
 }
 
-long group_of(size_t frame_bytes) { return std::max<long>(1, std::min<long>(256, (long)(GROUP_BYTES / frame_bytes))); }
-
 }  // namespace
 
 extern "C" {
@@ -338,7 +334,7 @@ int rv_chain_ex(rv_ctx *ctx, const void *in, void *out, int n, int h, int w, siz
     if (processed && p->gate_enable) RV_TRY(host_flags(ctx, c, (size_t)n));
     const size_t ib = (size_t)channels * sb * w, ob = (size_t)oc * sb * w;     // packed row bytes of the host path
     const size_t pp = ((size_t)3 * sb * w + 15) & ~(size_t)15;                 // row pitch of the BGR workspace
-    long G = group_of(ib * h);
+    long G = group_frames(ib * h);
     if (u16_clahe) G = std::min(G, group_frames_u16(p, h, w));
     for (int f0 = 0; f0 < n; f0 += (int)G) {
         const int g = (int)std::min<long>(G, n - f0);
@@ -427,7 +423,7 @@ int rv_gray_span_ex(rv_ctx *ctx, const void *in, int n, int h, int w, size_t pit
     RV_TRY(ws_acquire(ctx, c.sync, st));
     RV_TRY(host_flags(ctx, c, 2 * (size_t)n));
     const size_t ib = (size_t)4 * sb * w;
-    const int G = (int)group_of(ib * h);
+    const int G = (int)group_frames(ib * h);
     for (int f0 = 0; f0 < n; f0 += G) {
         const int g = std::min(G, n - f0);
         const uint8_t *gin = (const uint8_t *)in + (size_t)f0 * h * pitch;

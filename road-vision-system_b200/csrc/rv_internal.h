@@ -8,6 +8,8 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include <algorithm>
+
 #include "../../include/rv_b200.h"
 #include "rv_common.cuh"        // Geo
 
@@ -37,9 +39,8 @@ struct U16Ws {
     bool attr_set = false;                      // k_u16_hist_lut's dynamic shared-memory limit is raised
 };
 
-// Workspaces of the 1- and 4-channel path (rv_channels.cu) and of the host paths of rv_yuv420_to_bgr (rv_yuv.cu),
-// rv_yuv422_to_bgr (rv_yuv422.cu) and rv_bgr_to_yuv420 (rv_yuv_out.cu) (din / dout) of one context, used on whichever stream a call
-// runs on.
+// Workspaces of the 1- and 4-channel path (rv_channels.cu) and of the host path of convert_frames (rv_yuv.cu; din / dout) of one
+// context, used on whichever stream a call runs on.
 struct ChWs {
     Buf pack, din, dout, mm, flags;             // pack: BGR without alpha, the input of the 3-channel chains
     int32_t *hflags = nullptr;                  // page-locked copy of the gate decisions / gray min-max pairs
@@ -116,30 +117,51 @@ long group_frames_u16(const rv_params *p, int h, int w);
 int run_group_u16(rv_ctx *ctx, U16Ws &s, const uint16_t *din, size_t ip, size_t ifs, uint16_t *dout, size_t op, size_t ofs, int n,
                   int h, int w, const rv_params *p, cudaStream_t st, const int32_t **flags_out, bool copy_skipped = true);
 
+// Frames per group of a pass that works group by group: as many frames of `frame_bytes` as fit in 1 GiB, at least 1, at most 256.
+inline long group_frames(size_t frame_bytes) { return std::max<long>(1, std::min<long>(256, (long)(((size_t)1 << 30) / frame_bytes))); }
+
+// `rows` rows of `rowb` bytes from src (pitch spitch) to dst (pitch dpitch) on `st`: one linear copy when the pitches are equal,
+// else a 2D copy of the row bytes.
+inline int copy_rows(rv_ctx *ctx, void *dst, size_t dpitch, const void *src, size_t spitch, size_t rowb, size_t rows,
+                     cudaMemcpyKind dir, cudaStream_t st)
+{
+    if (dpitch == spitch) CK(cudaMemcpyAsync(dst, src, spitch * rows, dir, st));
+    else CK(cudaMemcpy2DAsync(dst, dpitch, src, spitch, rowb, rows, dir, st));
+    return RV_OK;
+}
+
+// Frame layouts: 0 is BGR, else enum rv_yuv (4:2:0) or enum rv_yuv422 (4:2:2).
 inline bool is_yuv420(int layout) { return layout == RV_YUV_NV12 || layout == RV_YUV_I420; }
 inline bool is_yuv422(int layout) { return layout == RV_YUV_YUY2 || layout == RV_YUV_UYVY; }
+// rows of one frame: 4:2:0 frames are 3h/2 rows of their pitch, BGR and 4:2:2 frames h rows
+inline size_t frame_rows(int layout, int h) { return is_yuv420(layout) ? (size_t)h * 3 / 2 : (size_t)h; }
+// bytes of one row: 3w for BGR pixels, w for 4:2:0 planes, 2w for 4:2:2 pixel pairs
+inline size_t row_bytes(int layout, int w) { return (size_t)(!layout ? 3 : is_yuv422(layout) ? 2 : 1) * w; }
+// the row pitch of frames staged on the device: one that the chains and the conversions' vector paths can use (16 bytes for BGR
+// and 4:2:2 rows, 8 for NV12; I420 planes stay packed)
+inline size_t stage_pitch(int layout, int w)
+{
+    if (layout == RV_YUV_NV12) return ((size_t)w + 7) & ~(size_t)7;
+    return layout == RV_YUV_I420 ? (size_t)w : (row_bytes(layout, w) + 15) & ~(size_t)15;
+}
 
 // rv_yuv.cu: the argument rules of a job with YUV frames on either side (in_layout: RV_YUV_NV12, RV_YUV_I420, RV_YUV_YUY2,
-// RV_YUV_UYVY or 0 for BGR; out_layout: RV_YUV_NV12, RV_YUV_I420 or 0; not both 0; out: nullptr = none) and the conversion of n
-// 4:2:0 frames at pitch sp into BGR frames at pitch dp, frame stride dfs, on `st`.  rv_yuv422.cu: the same conversion of n 4:2:2
-// frames.  rv_yuv_out.cu: the conversion of n BGR frames at pitch sp (frame stride sp * h) into 4:2:0 frames at pitch dp, on `st`.
+// RV_YUV_UYVY or 0 for BGR; out_layout: RV_YUV_NV12, RV_YUV_I420 or 0; not both 0; out: nullptr = none).
 int check_yuv(rv_ctx *ctx, const void *in, const void *out, int n, int h, int w, size_t ipitch, size_t opitch, int in_layout,
               int out_layout);
-int launch_yuv420(rv_ctx *ctx, int layout, const uint8_t *src, size_t sp, uint8_t *dst, size_t dp, size_t dfs, int n, int h, int w,
-                  cudaStream_t st);
-int launch_yuv422(rv_ctx *ctx, int layout, const uint8_t *src, size_t sp, uint8_t *dst, size_t dp, size_t dfs, int n, int h, int w,
-                  cudaStream_t st);
+// rv_yuv.cu: the conversion of n frames of in_layout at pitch sp into frames of out_layout at pitch dp on `st` (one side BGR; frame
+// f of either side starts at f * pitch * frame_rows).  It takes the launcher of its family: launch_yuv420 (rv_yuv.cu),
+// launch_yuv422 (rv_yuv422.cu) or launch_bgr420 (rv_yuv_out.cu), `layout` being the YUV side's.
+int launch_convert(rv_ctx *ctx, int in_layout, int out_layout, const uint8_t *src, size_t sp, uint8_t *dst, size_t dp, int n, int h,
+                   int w, cudaStream_t st);
+int launch_yuv420(rv_ctx *ctx, int layout, const uint8_t *src, size_t sp, uint8_t *dst, size_t dp, int n, int h, int w, cudaStream_t st);
+int launch_yuv422(rv_ctx *ctx, int layout, const uint8_t *src, size_t sp, uint8_t *dst, size_t dp, int n, int h, int w, cudaStream_t st);
 int launch_bgr420(rv_ctx *ctx, int layout, const uint8_t *src, size_t sp, uint8_t *dst, size_t dp, int n, int h, int w, cudaStream_t st);
-// rows of one frame of `layout` (0: BGR): 4:2:0 frames are 3h/2 rows of their pitch, BGR and 4:2:2 frames h rows
-inline size_t frame_rows(int layout, int h) { return is_yuv420(layout) ? (size_t)h * 3 / 2 : (size_t)h; }
-// bytes of one row of a YUV frame of `layout`: w for 4:2:0 planes, 2w for 4:2:2 pixel pairs
-inline size_t yuv_row_bytes(int layout, int w) { return (size_t)(is_yuv422(layout) ? 2 : 1) * w; }
-// the row pitch of YUV frames staged on the device: one that the conversions' vector paths can use (I420 planes stay packed)
-inline size_t yuv_stage_pitch(int layout, int w)
-{
-    if (is_yuv422(layout)) return ((size_t)2 * w + 15) & ~(size_t)15;
-    return layout == RV_YUV_NV12 ? ((size_t)w + 7) & ~(size_t)7 : (size_t)w;
-}
+// rv_yuv.cu: the checked job of rv_yuv420_to_bgr, rv_yuv422_to_bgr and rv_bgr_to_yuv420 -- check_yuv, check_kind, then device frames
+// converted on `stream` (or, without one, synchronously on the context's stream), host frames group by group through the context's
+// ChWs din / dout at stage_pitch.
+int convert_frames(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h, int w, size_t in_pitch, size_t out_pitch, int in_layout,
+                   int out_layout, int mem_kind, void *stream);
 
 }  // namespace rv
 

@@ -295,8 +295,7 @@ int check_params_u16(rv_ctx *ctx, const rv_params *p)
 
 long group_frames_u16(const rv_params *p, int h, int w)
 {
-    const size_t fb = (size_t)6 * w * h;
-    long g = std::max<long>(1, std::min<long>(256, (long)(((size_t)1 << 30) / fb)));
+    long g = group_frames((size_t)6 * w * h);
     if (p->clahe) {
         const size_t lb = (size_t)p->grid * p->grid * 65536 * 2;
         g = std::min<long>(g, std::max<long>(1, (long)(LUT_GROUP_BYTES / lb)));
@@ -464,7 +463,7 @@ int rv_gray_span_u16(rv_ctx *ctx, const uint16_t *in, int n, int h, int w, size_
     RV_TRY(ws_acquire(ctx, s.sync, st));
     RV_TRY(host_flags(ctx, s, 2 * n));
     const size_t fb = (size_t)6 * w * h;
-    const int G = (int)std::max<long>(1, std::min<long>(256, (long)(((size_t)1 << 30) / fb)));
+    const int G = (int)group_frames(fb);
     for (int f0 = 0; f0 < n; f0 += G) {
         const int g = std::min(G, n - f0);
         const uint16_t *gin = (const uint16_t *)((const uint8_t *)in + (size_t)f0 * h * pitch);

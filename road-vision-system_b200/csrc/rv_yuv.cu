@@ -105,8 +105,6 @@ __global__ void __launch_bounds__(256) k_yuv420_to_bgr(const uint8_t *__restrict
     }
 }
 
-constexpr size_t GROUP_BYTES = (size_t)1 << 30;     // BGR bytes of one frame group of the host path, as the 3-channel paths
-
 }  // namespace
 
 int rv::check_yuv(rv_ctx *ctx, const void *in, const void *out, int n, int h, int w, size_t ipitch, size_t opitch, int in_layout,
@@ -133,10 +131,10 @@ int rv::check_yuv(rv_ctx *ctx, const void *in, const void *out, int n, int h, in
     return RV_OK;
 }
 
-int rv::launch_yuv420(rv_ctx *ctx, int layout, const uint8_t *src, size_t sp, uint8_t *dst, size_t dp, size_t dfs, int n, int h, int w,
+int rv::launch_yuv420(rv_ctx *ctx, int layout, const uint8_t *src, size_t sp, uint8_t *dst, size_t dp, int n, int h, int w,
                       cudaStream_t st)
 {
-    const size_t sfs = sp * h * 3 / 2;
+    const size_t sfs = sp * frame_rows(layout, h), dfs = dp * h;
     const int vec = (((uintptr_t)src | sp | sfs | (uintptr_t)dst | dp | dfs) % 8) == 0;
     const int groups = (w + 7) / 8;
     for (int f0 = 0; f0 < n; f0 += MAX_FRAMES_PER_LAUNCH) {
@@ -151,6 +149,50 @@ int rv::launch_yuv420(rv_ctx *ctx, int layout, const uint8_t *src, size_t sp, ui
     return RV_OK;
 }
 
+int rv::launch_convert(rv_ctx *ctx, int in_layout, int out_layout, const uint8_t *src, size_t sp, uint8_t *dst, size_t dp, int n, int h,
+                       int w, cudaStream_t st)
+{
+    if (is_yuv420(in_layout)) return launch_yuv420(ctx, in_layout, src, sp, dst, dp, n, h, w, st);
+    if (is_yuv422(in_layout)) return launch_yuv422(ctx, in_layout, src, sp, dst, dp, n, h, w, st);
+    return launch_bgr420(ctx, out_layout, src, sp, dst, dp, n, h, w, st);
+}
+
+int rv::convert_frames(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h, int w, size_t in_pitch, size_t out_pitch,
+                       int in_layout, int out_layout, int mem_kind, void *stream)
+{
+    RV_TRY(check_yuv(ctx, in, out, n, h, w, in_pitch, out_pitch, in_layout, out_layout));
+    RV_TRY(check_kind(ctx, mem_kind));
+    if (n == 0) return RV_OK;
+    CK(cudaSetDevice(rv_internal_device(ctx)));
+    if (mem_kind == RV_MEM_DEVICE) {
+        cudaStream_t st = stream ? (cudaStream_t)stream : (cudaStream_t)rv_internal_stream(ctx);
+        RV_TRY(launch_convert(ctx, in_layout, out_layout, in, in_pitch, out, out_pitch, n, h, w, st));
+        if (!stream) CK(cudaStreamSynchronize(st));
+        return RV_OK;
+    }
+    // host frames, group by group: H2D at a pitch the vector paths can read, conversion into a pitch they can write, D2H at the
+    // caller's pitch
+    ChWs &c = rv_internal_ch(ctx);
+    cudaStream_t st = (cudaStream_t)rv_internal_stream(ctx);
+    RV_TRY(ws_acquire(ctx, c.sync, st));
+    const size_t irows = frame_rows(in_layout, h), ip = stage_pitch(in_layout, w);
+    const size_t orows = frame_rows(out_layout, h), op = stage_pitch(out_layout, w);
+    const int G = (int)group_frames(stage_pitch(0, w) * h);
+    for (int f0 = 0; f0 < n; f0 += G) {
+        const int g = std::min(G, n - f0);
+        RV_TRY(ensure(ctx, c.din, ip * irows * g));
+        RV_TRY(ensure(ctx, c.dout, op * orows * g));
+        RV_TRY(copy_rows(ctx, c.din.p, ip, in + (size_t)f0 * in_pitch * irows, in_pitch, row_bytes(in_layout, w), irows * g,
+                         cudaMemcpyHostToDevice, st));
+        RV_TRY(launch_convert(ctx, in_layout, out_layout, (const uint8_t *)c.din.p, ip, (uint8_t *)c.dout.p, op, g, h, w, st));
+        RV_TRY(copy_rows(ctx, out + (size_t)f0 * out_pitch * orows, out_pitch, c.dout.p, op, row_bytes(out_layout, w), orows * g,
+                         cudaMemcpyDeviceToHost, st));
+    }
+    RV_TRY(ws_release(ctx, c.sync, st));
+    CK(cudaStreamSynchronize(st));
+    return RV_OK;
+}
+
 extern "C" {
 
 int rv_yuv420_to_bgr(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h, int w, size_t in_pitch, size_t out_pitch, int layout,
@@ -159,36 +201,7 @@ int rv_yuv420_to_bgr(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h,
     if (!ctx) return RV_ERR_ARG;
     if (!out) return fail(ctx, RV_ERR_ARG, "null frame pointer");      // check_yuv takes a null `out` for a tensor-only job
     if (is_yuv422(layout)) return fail(ctx, RV_ERR_ARG, "bad YUV layout %d (4:2:2 frames: rv_yuv422_to_bgr)", layout);
-    RV_TRY(check_yuv(ctx, in, out, n, h, w, in_pitch, out_pitch, layout, 0));
-    RV_TRY(check_kind(ctx, mem_kind));
-    if (n == 0) return RV_OK;
-    CK(cudaSetDevice(rv_internal_device(ctx)));
-    if (mem_kind == RV_MEM_DEVICE) {
-        cudaStream_t st = stream ? (cudaStream_t)stream : (cudaStream_t)rv_internal_stream(ctx);
-        RV_TRY(launch_yuv420(ctx, layout, in, in_pitch, out, out_pitch, out_pitch * h, n, h, w, st));
-        if (!stream) CK(cudaStreamSynchronize(st));
-        return RV_OK;
-    }
-    // host frames, group by group: H2D at a pitch the vector path can read, conversion, D2H at the caller's pitch
-    ChWs &c = rv_internal_ch(ctx);
-    cudaStream_t st = (cudaStream_t)rv_internal_stream(ctx);
-    RV_TRY(ws_acquire(ctx, c.sync, st));
-    const size_t yp = yuv_stage_pitch(layout, w), yfs = yp * h * 3 / 2;
-    const size_t rowb = (size_t)3 * w, bp = (rowb + 15) & ~(size_t)15, bfs = bp * h;
-    const int G = (int)std::max<size_t>(1, std::min<size_t>(256, GROUP_BYTES / bfs));
-    for (int f0 = 0; f0 < n; f0 += G) {
-        const int g = std::min(G, n - f0);
-        RV_TRY(ensure(ctx, c.din, yfs * g));
-        RV_TRY(ensure(ctx, c.dout, bfs * g));
-        const uint8_t *src = in + (size_t)f0 * in_pitch * h * 3 / 2;
-        if (in_pitch == yp) CK(cudaMemcpyAsync(c.din.p, src, yfs * g, cudaMemcpyHostToDevice, st));
-        else CK(cudaMemcpy2DAsync(c.din.p, yp, src, in_pitch, w, (size_t)h * 3 / 2 * g, cudaMemcpyHostToDevice, st));
-        RV_TRY(launch_yuv420(ctx, layout, (const uint8_t *)c.din.p, yp, (uint8_t *)c.dout.p, bp, bfs, g, h, w, st));
-        CK(cudaMemcpy2DAsync(out + (size_t)f0 * h * out_pitch, out_pitch, c.dout.p, bp, rowb, (size_t)h * g, cudaMemcpyDeviceToHost, st));
-    }
-    RV_TRY(ws_release(ctx, c.sync, st));
-    CK(cudaStreamSynchronize(st));
-    return RV_OK;
+    return convert_frames(ctx, in, out, n, h, w, in_pitch, out_pitch, layout, 0, mem_kind, stream);
 }
 
 }  // extern "C"

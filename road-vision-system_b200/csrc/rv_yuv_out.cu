@@ -109,14 +109,12 @@ __global__ void __launch_bounds__(256) k_bgr_to_yuv420(const uint8_t *__restrict
     }
 }
 
-constexpr size_t GROUP_BYTES = (size_t)1 << 30;     // BGR bytes of one frame group of the host path, as the 3-channel paths
-
 }  // namespace
 
 int rv::launch_bgr420(rv_ctx *ctx, int layout, const uint8_t *src, size_t sp, uint8_t *dst, size_t dp, int n, int h, int w,
                       cudaStream_t st)
 {
-    const size_t sfs = sp * h, dfs = dp * h * 3 / 2;
+    const size_t sfs = sp * h, dfs = dp * frame_rows(layout, h);
     const int vec = (((uintptr_t)src | sp | (uintptr_t)dst | dp) % 8) == 0;       // (then both frame strides are multiples of 8)
     const int groups = (w + 7) / 8;
     for (int f0 = 0; f0 < n; f0 += MAX_FRAMES_PER_LAUNCH) {
@@ -138,38 +136,7 @@ int rv_bgr_to_yuv420(rv_ctx *ctx, const uint8_t *in, uint8_t *out, int n, int h,
 {
     if (!ctx) return RV_ERR_ARG;
     if (!out) return fail(ctx, RV_ERR_ARG, "null frame pointer");      // check_yuv takes a null `out` for a tensor-only job
-    RV_TRY(check_yuv(ctx, in, out, n, h, w, in_pitch, out_pitch, 0, layout));
-    RV_TRY(check_kind(ctx, mem_kind));
-    if (n == 0) return RV_OK;
-    CK(cudaSetDevice(rv_internal_device(ctx)));
-    if (mem_kind == RV_MEM_DEVICE) {
-        cudaStream_t st = stream ? (cudaStream_t)stream : (cudaStream_t)rv_internal_stream(ctx);
-        RV_TRY(launch_bgr420(ctx, layout, in, in_pitch, out, out_pitch, n, h, w, st));
-        if (!stream) CK(cudaStreamSynchronize(st));
-        return RV_OK;
-    }
-    // host frames, group by group: H2D at a 16-byte pitch, conversion at a pitch the vector path can write, D2H at the caller's pitch
-    ChWs &c = rv_internal_ch(ctx);
-    cudaStream_t st = (cudaStream_t)rv_internal_stream(ctx);
-    RV_TRY(ws_acquire(ctx, c.sync, st));
-    const size_t yp = yuv_stage_pitch(layout, w), yfs = yp * h * 3 / 2;
-    const size_t rowb = (size_t)3 * w, bp = (rowb + 15) & ~(size_t)15, bfs = bp * h;
-    const int G = (int)std::max<size_t>(1, std::min<size_t>(256, GROUP_BYTES / bfs));
-    for (int f0 = 0; f0 < n; f0 += G) {
-        const int g = std::min(G, n - f0);
-        RV_TRY(ensure(ctx, c.din, bfs * g));
-        RV_TRY(ensure(ctx, c.dout, yfs * g));
-        const uint8_t *src = in + (size_t)f0 * in_pitch * h;
-        if (in_pitch == bp) CK(cudaMemcpyAsync(c.din.p, src, bfs * g, cudaMemcpyHostToDevice, st));
-        else CK(cudaMemcpy2DAsync(c.din.p, bp, src, in_pitch, rowb, (size_t)h * g, cudaMemcpyHostToDevice, st));
-        RV_TRY(launch_bgr420(ctx, layout, (const uint8_t *)c.din.p, bp, (uint8_t *)c.dout.p, yp, g, h, w, st));
-        uint8_t *dst = out + (size_t)f0 * out_pitch * h * 3 / 2;
-        if (out_pitch == yp) CK(cudaMemcpyAsync(dst, c.dout.p, yfs * g, cudaMemcpyDeviceToHost, st));
-        else CK(cudaMemcpy2DAsync(dst, out_pitch, c.dout.p, yp, w, (size_t)h * 3 / 2 * g, cudaMemcpyDeviceToHost, st));
-    }
-    RV_TRY(ws_release(ctx, c.sync, st));
-    CK(cudaStreamSynchronize(st));
-    return RV_OK;
+    return convert_frames(ctx, in, out, n, h, w, in_pitch, out_pitch, 0, layout, mem_kind, stream);
 }
 
 }  // extern "C"

@@ -10,8 +10,8 @@ from typing import Any, Dict
 
 import numpy as np
 
-from .._native import (MEM_DEVICE, DeviceArray, Params, check_bgr_for_yuv, check_frame_params, check_out_yuv, check_u16_params,
-                       check_yuv_frames, default_context)
+from .._native import (DeviceArray, Params, _check_torch_out, _torch_stream, check_bgr_for_yuv, check_frame_params, check_out_yuv,
+                       check_u16_params, check_yuv_frames, default_context)
 from .base import as_bgr_frame, as_frame
 from .ops import CLAHEDehaze, MedianDerain
 from .ops import clahe_dehaze as _clahe
@@ -247,10 +247,9 @@ class PreprocessPipeline:
                 raise ValueError("frames must be a contiguous CUDA tensor")
             # everything the device path would refuse is refused before the conversion is enqueued
             self._check_device_chain()
-            if out is not None and not (_is_cuda_tensor(out) and out.dtype == torch.uint8 and tuple(out.shape) == (b, h, w, 3)
-                                        and out.device == frames.device and out.is_contiguous()):
-                raise ValueError(f"out must be a contiguous uint8 CUDA tensor of shape {(b, h, w, 3)} on the input's device")
-            return self._process_batch_device(self._device_ctx(frames)._yuv_to_bgr(frames, yuv), out)
+            _check_torch_out(out, (b, h, w, 3), torch.uint8, frames.device,
+                             f"out must be a contiguous uint8 CUDA tensor of shape {(b, h, w, 3)} on the input's device")
+            return self._process_batch_device(self._device_ctx(frames)._convert(frames, yuv, None), out)
         if isinstance(out, str) and out != "device":
             raise ValueError('out must be an array, None or "device"')
         if not isinstance(frames, np.ndarray):
@@ -263,7 +262,7 @@ class PreprocessPipeline:
         ctx = self._ctx()
         seg = self._fused_segment()
         if seg is None:
-            bgr = ctx._yuv_to_bgr(frames, yuv)
+            bgr = ctx._convert(frames, yuv, None)
             return self._process_batch_keep(bgr) if isinstance(out, str) else self.process_batch(bgr, out)
         gate, thresh = self._gate()
         if gate:
@@ -273,7 +272,7 @@ class PreprocessPipeline:
         elif out is not None:
             res = out
         else:
-            res = ctx._pooled_pinned(shape) if b * h * w * 3 <= (64 << 20) else np.empty(shape, np.uint8)
+            res = ctx._host_result(shape)
         ctx.submit_io(np.ascontiguousarray(frames), seg, out=res, yuv=yuv)
         ctx.wait()
         return res
@@ -301,12 +300,11 @@ class PreprocessPipeline:
         if tensor:
             if not frames.is_contiguous():
                 raise ValueError("frames must be a contiguous CUDA tensor")
-            if out is not None and not (_is_cuda_tensor(out) and out.dtype == torch.uint8 and tuple(out.shape) == shape
-                                        and out.device == frames.device and out.is_contiguous()):
-                raise ValueError(f"out must be a contiguous uint8 CUDA tensor of shape {shape} on the input's device")
+            _check_torch_out(out, shape, torch.uint8, frames.device,
+                             f"out must be a contiguous uint8 CUDA tensor of shape {shape} on the input's device")
             self._check_device_chain()
             ctx = self._device_ctx(frames)
-            bgr = ctx._yuv_to_bgr(frames, yuv) if yuv is not None else frames
+            bgr = ctx._convert(frames, yuv, None) if yuv is not None else frames
             return ctx.bgr_to_yuv420(self._process_batch_device(bgr), out_yuv, out=out)
         if isinstance(out, str) and out != "device":
             raise ValueError('out must be an array, None or "device"')
@@ -317,10 +315,7 @@ class PreprocessPipeline:
         seg = self._fused_segment()
         if seg is None:
             if isinstance(out, str):
-                bgr = self.process_batch(frames, out="device", yuv=yuv)
-                res = DeviceArray(ctx, shape)
-                ctx._ck(ctx._lib.rv_bgr_to_yuv420(ctx._h, bgr.ptr, res.ptr, b, h, w, 3 * w, w, check_out_yuv(out_yuv), MEM_DEVICE, None))
-                return res
+                return ctx.bgr_to_yuv420(self.process_batch(frames, out="device", yuv=yuv), out_yuv)
             return ctx.bgr_to_yuv420(self.process_batch(frames, yuv=yuv), out_yuv, out=out)
         gate, thresh = self._gate()
         if gate:
@@ -330,7 +325,7 @@ class PreprocessPipeline:
         elif out is not None:
             res = out
         else:
-            res = ctx._pooled_pinned(shape) if b * h * w * 3 // 2 <= (64 << 20) else np.empty(shape, np.uint8)
+            res = ctx._host_result(shape)
         ctx.submit_io(np.ascontiguousarray(frames), seg, out=res, yuv=yuv, out_yuv=out_yuv)
         ctx.wait()
         return res
@@ -415,16 +410,14 @@ class PreprocessPipeline:
             self._check_batch_channels(self._segments(), np.uint16 if wide else np.uint8, frames.shape[3])
             if any(isinstance(sg, Params) and sg.clahe for sg in self._segments()):
                 final = final[:3] + (3,)
-        if out is not None and not (_is_cuda_tensor(out) and out.dtype == frames.dtype and tuple(out.shape) == final
-                                    and out.device == frames.device and out.is_contiguous()):
-            raise ValueError(f"out must be a contiguous CUDA tensor of shape {final} and the input's dtype and device")
+        _check_torch_out(out, final, frames.dtype, frames.device,
+                         f"out must be a contiguous CUDA tensor of shape {final} and the input's dtype and device")
         if not self.enabled or not self.ops:
             return frames if out is None else out.copy_(frames)
         self._check_device_chain()
         ctx = self._device_ctx(frames)
         b, h, w, _ = frames.shape
         segs = self._segments()
-        stream = torch.cuda.current_stream(frames.device).cuda_stream
         cur = frames
         for idx, sg in enumerate(segs):
             c = cur.shape[3]
@@ -432,18 +425,14 @@ class PreprocessPipeline:
             last = idx == len(segs) - 1 and out is not None
             if c != 3:
                 dst = out if last else torch.empty((b, h, w, oc), dtype=frames.dtype, device=frames.device)
-                if stream == 0:
-                    torch.cuda.current_stream(frames.device).synchronize()
-                ctx.chain_ex_device(cur.data_ptr(), dst.data_ptr(), b, h, w, sg, 16 if wide else 8, c, stream=stream or None)
+                ctx.chain_ex_device(cur.data_ptr(), dst.data_ptr(), b, h, w, sg, 16 if wide else 8, c, stream=_torch_stream(frames.device))
                 cur = dst
                 continue
             dst = out if last else torch.empty_like(cur)
+            stream = _torch_stream(frames.device)
             if wide:
-                if stream == 0:
-                    torch.cuda.current_stream(frames.device).synchronize()
-                ctx.chain_u16_device(cur.data_ptr(), dst.data_ptr(), b, h, w, sg, stream=stream or None)
-            elif stream == 0:        # legacy default stream: run on the context's stream, synchronously
-                torch.cuda.current_stream(frames.device).synchronize()
+                ctx.chain_u16_device(cur.data_ptr(), dst.data_ptr(), b, h, w, sg, stream=stream)
+            elif stream is None:        # legacy default stream: run on the context's stream, synchronously
                 ctx.chain_device(cur.data_ptr(), dst.data_ptr(), b, h, w, sg)
             else:
                 ctx.submit_device(cur.data_ptr(), dst.data_ptr(), b, h, w, sg, stream=stream)
@@ -498,8 +487,7 @@ class PreprocessPipeline:
         if keep:
             frames = np.ascontiguousarray(frames)
             dev = DeviceArray(ctx, (frames.shape[0], 3, size, size), np.float16)
-            full = ctx._pooled_pinned(frames.shape) if (want_frames and frames.nbytes <= (64 << 20)) else \
-                (np.empty_like(frames) if want_frames else None)
+            full = ctx._host_result(frames.shape) if want_frames else None
             ctx.submit_io(frames, segs[0], out=full, tensor=dev, size=size, pad_value=pad_value)
             ctx.wait()
             return dev, full
@@ -520,14 +508,12 @@ class PreprocessPipeline:
         ctx = self._ctx()
         seg = self._fused_segment()
         if seg is None or self._gate()[0]:
-            return self.process_batch_to_tensor(ctx._yuv_to_bgr(frames, yuv), size, pad_value, want_frames, out, padding_present)
+            return self.process_batch_to_tensor(ctx._convert(frames, yuv, None), size, pad_value, want_frames, out, padding_present)
         if keep:
             t = DeviceArray(ctx, (b, 3, size, size), np.float16)
         else:
             t = np.empty((b, 3, size, size), np.float16) if out is None else out
-        full = None
-        if want_frames:
-            full = ctx._pooled_pinned((b, h, w, 3)) if b * h * w * 3 <= (64 << 20) else np.empty((b, h, w, 3), np.uint8)
+        full = ctx._host_result((b, h, w, 3)) if want_frames else None
         ctx.submit_io(np.ascontiguousarray(frames), seg, out=full, tensor=t, size=size, pad_value=pad_value,
                       padding_present=bool(padding_present and out is not None and not keep), yuv=yuv)
         ctx.wait()
